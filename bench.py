@@ -5,6 +5,7 @@ target-assign + loss + NMS, SSD300 / 8732 priors) -- one JSON line on stdout.
     python bench.py --gpus 1 --steps 20 --warmup 5
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference          # the reference's own CPU code on the host cores
+    python bench.py --dump-outputs DIR        # also save the last timed step's results as DIR/*.npy
 
 A step is one pass of the chain over one synthetic batch per GPU (weak scaling: the per-GPU batch is fixed;
 ``--scaling strong --global-batch G`` fixes the total instead).  ``value`` is measured with the inputs resident in HBM,
@@ -71,7 +72,15 @@ def parse():
                          "over all ranks' batches (exact-global, staged all-reduces)")
     ap.add_argument("--exchange", default="ssdg", choices=["ssdg", "torch"],
                     help="data-parallel exchange through the library's own ssdg_comm_* (NCCL) or torch.distributed")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returns to its caller (loss result block, kept lists, counts; "
+                         "rank 0's shard) as DIR/<name>.npy, so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -565,6 +574,27 @@ def profile_json(name):
         return None
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(path, outputs):
+    """Save the last timed step's results as float64 (loss result block) and float32 (kept prior indices, -1 padded,
+    and counts: exact below 2**24).  Kept lists and counts are per image; if together they would pass
+    DUMP_LIMIT_BYTES, a fixed seeded sample of images is written instead, its indices in images.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {"loss_result": outputs["loss_result"].astype(np.float64), "kept": outputs["kept"].astype(np.float32),
+              "count": outputs["count"].astype(np.float32)}
+    batch = arrays["count"].shape[0]
+    per_image = (arrays["kept"].nbytes + arrays["count"].nbytes) // batch + 8        # + its index in images.npy
+    room = (DUMP_LIMIT_BYTES - arrays["loss_result"].nbytes - 4 * 4096) // per_image     # (.npy headers)
+    if room < batch:
+        images = np.sort(np.random.default_rng(0).choice(batch, room, replace=False))
+        arrays["kept"], arrays["count"] = arrays["kept"][images], arrays["count"][images]
+        arrays["images"] = images.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_ours(args):
     from ssdgeom import _native as N, device as D, synth
     R = Ranks()
@@ -595,6 +625,8 @@ def run_ours(args):
         return
     line = report(args, R, comm, b, M, detail_cfg)
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, M["outputs"])
     if comm is not None:
         comm.close()
     R.close()
@@ -621,6 +653,9 @@ def headline(R, args, comm, sampler, b):
     value = b * world * 1e3 / ms_step
     hp.use_set((args.steps - 1) % n_sets)
     res = hp.loss["result"].to_host()
+    # the buffers HotPath.download reads hold the last timed step's results until the next step runs
+    outputs = {"loss_result": res, "kept": hp.det["kept"].to_host(), "count": hp.det["count"].to_host()} \
+        if args.dump_outputs else None
     clocks = sampler.summary(t0, t1, t_load0, time.perf_counter())
     # the same steps as closed units (each joined before the next starts): the latency of one step
     depth, closed_ms = hp.depth, ms_step
@@ -760,7 +795,7 @@ def headline(R, args, comm, sampler, b):
                 kernel_ms=kernel_ms, tiles_evaluated=tiles_evaluated, ce_alone_ms=ce_alone_ms,
                 filter_alone_ms=filter_alone_ms, grad_ms=grad_ms, e2e=e2e, launches=hp.kernel_launches_per_step,
                 memsets=hp.memsets_per_step, fused=bool(hp.fused), logits_mb=hp.pred_cls.nbytes / 1e6,
-                gt_rows=float(np.diff(off).sum()))
+                gt_rows=float(np.diff(off).sum()), outputs=outputs)
 
 
 def report(args, R, comm, b, M, detail_cfg):
