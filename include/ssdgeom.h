@@ -345,6 +345,65 @@ SSDG_API int ssdg_nms(const float* probs, const float* boxes, int64_t batch, int
              int32_t* out_kept, int32_t* out_count, float* out_kept_score, void* workspace,
              size_t workspace_bytes, void* stream);
 
+/* ---- A11: detection evaluation ---------------------------------------------------------------------------
+ * The reference has no evaluation code.  COCO's AP (pycocotools COCOeval.evaluateImg + accumulate, iouType "bbox",
+ * area range "all", no crowd / ignore flags) over the kept lists of ssdg_detect, accumulated on the device over
+ * batches and data-parallel ranks (spec: tests/coco_eval_oracle.py; PARITY UNPINNED against pycocotools on pixel
+ * boxes, bit-exact against that restatement).
+ *   detections of (image, class c): the first min(count, max_dets) entries of the kept list (already in score desc,
+ *     prior asc order); ground truth of (image, c): the image's CSR rows whose class (gt_cls truncated to int32, as
+ *     ssdg_match_encode) is c, in row order.
+ *   IoU in float64 from the exactly promoted float32 cxcywh boxes: x0 = cx - 0.5w, x1 = cx + 0.5w (y alike),
+ *     iw = min(x1) - max(x0), ih alike, 0 unless iw > 0 and ih > 0, else inter / ((wd*hd + wg*hg) - inter).
+ *   matching at threshold t: visit the detections in order; best = min(t, 1 - 1e-10); over the unmatched ground
+ *     truth rows in order, skip iou < best, else best = iou and m = row (the last of equal IoUs wins); m >= 0 is a TP.
+ * Each image has a GLOBAL index image_base + i, unique over batches and ranks, that orders equal scores.
+ *
+ * State (caller-owned device memory, 256-byte aligned, ssdg_eval_state_bytes bytes; K = n_classes - 1,
+ * M = max_images, D = max_dets):
+ *   int32 header[64]  [0] GT rows with a class outside [0, K)  [1] images with more GT rows than max_gt
+ *                     [2] slots written more than once (set by finalize)  [3] kept prior indices outside [0, A)
+ *   uint32 flags[K][M][D]  bits 0..15: TP at threshold k, bit 16: present
+ *   int32 n_gt[K][M]       ground-truth rows per (class, image)
+ *   int64 keys[K][M][D]    score_bits << 32 | (0xFFFFFFFF - (image << 10 | rank)); 0 = empty
+ * One fixed slot per (class, global image, rank) with exactly one writer: no global atomics on the slots,
+ * deterministic, and re-adding a batch with the same image_base overwrites it.  12 bytes per slot: COCO val
+ * (5 000 images, 80 classes, 100 detections) takes 480 MB.
+ * Limits: max_images < 2^22, max_dets <= 1024 and <= top_k, K*M*D < 2^31, n_thresholds <= 16, max_gt <= 2048,
+ * n_recall <= 256.
+ *
+ * Data parallel: every slot is written by one rank and zero on the others, so summing the two buffers of
+ * ssdg_eval_exchange over the ranks (ssdg_comm_allreduce_sum: which 0 as SSDG_I64, which 1 as SSDG_I32) is an
+ * all-gather.  A slot written by two ranks carries its present bit into bit 17: finalize reports it (header[2]).
+ *
+ * Finalize (once per evaluation, leaves the state unchanged): records of class c in (score desc, global image asc,
+ * rank asc) order; tp / fp cumulative sums as integers; rc = tp / n_gt, pr = tp / ((fp + tp) + 2^-52), pr made
+ * non-increasing from the right; precision[t][r][c] = pr[searchsorted_left(rc, recall_thresholds[r])], 0 past the
+ * last detection; recall[t][c] = rc[-1] (0 without detections); classes without ground truth: -1 in both.
+ * Outputs: precision f64[T][R][K], recall f64[T][K], n_gt i64[K], n_det i64[K] (device).
+ * Workspace: ssdg_eval_finalize_workspace_bytes (the sorted copy of the slots plus the sort's temporary storage;
+ * the size query needs a CUDA device).
+ */
+SSDG_API size_t ssdg_eval_state_bytes(int32_t n_classes, int64_t max_images, int32_t max_dets,
+                                      int32_t n_thresholds);   /* 0: arguments out of range */
+SSDG_API int ssdg_eval_reset(void* state, size_t state_bytes, void* stream);
+SSDG_API int ssdg_eval_accumulate(const int32_t* kept, const int32_t* count, const float* kept_score, int32_t top_k,
+                         const float* boxes /* [B,A,4], 16-byte aligned */, int32_t batch, int32_t n_priors,
+                         int32_t n_classes, const float* gt_boxes, const float* gt_cls, const int32_t* gt_offsets,
+                         int32_t max_gt, const double* iou_thresholds /* host */, int32_t n_thresholds,
+                         int32_t max_dets, int64_t image_base, int64_t max_images, void* state, size_t state_bytes,
+                         void* stream);
+SSDG_API int ssdg_eval_exchange(void* state, int32_t n_classes, int64_t max_images, int32_t max_dets, int32_t which,
+                       void** out_ptr, int64_t* out_count);
+/* Synchronous: status bits of the state (1: GT class out of range, 2: an image with more GT rows than max_gt,
+ * 4: a slot written by more than one rank -- known after ssdg_eval_finalize, 8: a kept prior index out of range). */
+SSDG_API int ssdg_eval_status(const void* state, int32_t* status, void* stream);
+SSDG_API size_t ssdg_eval_finalize_workspace_bytes(int32_t n_classes, int64_t max_images, int32_t max_dets);
+SSDG_API int ssdg_eval_finalize(void* state, size_t state_bytes, int32_t n_classes, int64_t max_images,
+                       int32_t max_dets, int32_t n_thresholds, const double* recall_thresholds /* host */,
+                       int32_t n_recall, double* out_precision, double* out_recall, int64_t* out_n_gt,
+                       int64_t* out_n_det, void* workspace, size_t workspace_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -32,6 +32,7 @@ UNITS = {
     "loss.cu": [],
     "detect.cu": [],
     "comm.cu": [],
+    "eval.cu": ["-fmad=false"],
 }
 
 

@@ -79,6 +79,15 @@ PROTOTYPES = {
     "ssdg_multibox_loss_fused": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp,
                                            _vp, _vp, _vp, _sz, _vp]),
     "ssdg_nms": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _i32, _f32, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ssdg_eval_state_bytes": (_sz, [_i32, _i64, _i32, _i32]),
+    "ssdg_eval_reset": (C.c_int, [_vp, _sz, _vp]),
+    "ssdg_eval_accumulate": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _pf64, _i32,
+                                       _i32, _i64, _i64, _vp, _sz, _vp]),
+    "ssdg_eval_exchange": (C.c_int, [_vp, _i32, _i64, _i32, _i32, C.POINTER(C.c_void_p), C.POINTER(C.c_int64)]),
+    "ssdg_eval_status": (C.c_int, [_vp, _pi32, _vp]),
+    "ssdg_eval_finalize_workspace_bytes": (_sz, [_i32, _i64, _i32]),
+    "ssdg_eval_finalize": (C.c_int, [_vp, _sz, _i32, _i64, _i32, _i32, _pf64, _i32, _vp, _vp, _vp, _vp, _vp, _sz,
+                                     _vp]),
     "ssdg_comm_available": (C.c_int, [C.POINTER(C.c_int)]),
     "ssdg_comm_unique_id": (C.c_int, [_vp]),
     "ssdg_comm_init_rank": (C.c_int, [C.POINTER(_vp), _vp, _i32, _i32]),

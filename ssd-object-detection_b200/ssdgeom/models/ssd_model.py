@@ -130,3 +130,20 @@ class SSDBoxGeometry:
 
     def visualize_scores(self, pred_conf, thresh=0.5):
         return score_head(pred_conf, thresh)
+
+
+def evaluate_detections(kept, count, kept_score, boxes, gt_boxes, gt_cls, gt_offsets, max_dets=100,
+                        iou_thresholds=None, recall_thresholds=None) -> dict:
+    """COCO-style AP of one set of host detections (``detect(..., return_aux=True)``: kept, count, kept_score and
+    the decoded boxes) against CSR ground truth (relative cxcywh, class ids as float32), evaluated on the device.
+    Returns {"AP", "AP50", "AP75", "AR", "per_class_AP", "precision", "recall", "n_gt", "n_det"}."""
+    from ..evaluate import DetectionEvaluator
+    kept = np.ascontiguousarray(kept, np.int32)
+    b, k, _ = kept.shape
+    ev = DetectionEvaluator(n_classes=k + 1, max_images=b, max_dets=max_dets, iou_thresholds=iou_thresholds,
+                            recall_thresholds=recall_thresholds)
+    det = {"kept": kept, "count": np.ascontiguousarray(count, np.int32),
+           "kept_score": np.ascontiguousarray(kept_score, np.float32), "boxes": np.ascontiguousarray(boxes, np.float32)}
+    ev.add(det, np.ascontiguousarray(gt_boxes, np.float32), np.ascontiguousarray(gt_cls, np.float32),
+           np.ascontiguousarray(gt_offsets, np.int32), image_base=0)
+    return ev.summarize()

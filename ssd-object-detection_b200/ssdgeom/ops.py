@@ -466,3 +466,93 @@ def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores
                          D.stream_handle(stream)), "nms")
     out["_keep"] = (probs, boxes, ws)
     return out
+
+
+# ---- A11 ------------------------------------------------------------------------------------------------
+EVAL_STATUS_BAD_CLASS, EVAL_STATUS_TOO_MANY_GT, EVAL_STATUS_DUPLICATE, EVAL_STATUS_BAD_PRIOR = 1, 2, 4, 8
+
+
+class EvalState(D.DeviceArray):
+    """The device accumulator of the detection evaluation (include/ssdgeom.h, A11) with the sizes it was made for."""
+
+    def __init__(self, n_classes: int, max_images: int, max_dets: int, n_thresholds: int):
+        nbytes = int(N.lib().ssdg_eval_state_bytes(int(n_classes), int(max_images), int(max_dets), int(n_thresholds)))
+        if nbytes == 0:
+            raise ValueError("evaluation state out of range: n_classes >= 2, 0 < max_images < 2^22, "
+                             "0 < max_dets <= 1024, 0 < n_thresholds <= 16, (n_classes-1)*max_images*max_dets < 2^31")
+        super().__init__((nbytes,), np.uint8)
+        self.n_classes, self.max_images = int(n_classes), int(max_images)
+        self.max_dets, self.n_thresholds = int(max_dets), int(n_thresholds)
+
+
+def eval_state(n_classes: int, max_images: int, max_dets: int = 100, n_thresholds: int = 10, stream=None) -> EvalState:
+    st = EvalState(n_classes, max_images, max_dets, n_thresholds)
+    eval_reset(st, stream)
+    return st
+
+
+def eval_reset(state: EvalState, stream=None):
+    N.check(N.lib().ssdg_eval_reset(state.ptr, state.nbytes, D.stream_handle(stream)), "eval_reset")
+
+
+def eval_accumulate(det: dict, gt_boxes, gt_cls, gt_offsets, state: EvalState, iou_thresholds, image_base: int,
+                    max_gt: int, stream=None):
+    """Match one batch of ``detect`` outputs (``kept``, ``count``, ``kept_score``, ``boxes``) to its ground truth
+    (CSR, as ``match_encode``) and write the slots of global images ``image_base ..`` (ssdg_eval_accumulate)."""
+    kept, count = D.as_device(det["kept"], np.int32, stream), D.as_device(det["count"], np.int32, stream)
+    kept_score = D.as_device(det["kept_score"], np.float32, stream)
+    boxes = D.as_device(det["boxes"], np.float32, stream)
+    gt_boxes, gt_cls = D.as_device(gt_boxes, np.float32, stream), D.as_device(gt_cls, np.float32, stream)
+    gt_offsets = D.as_device(gt_offsets, np.int32, stream)
+    if len(kept.shape) != 3 or len(boxes.shape) != 3:
+        raise AssertionError("kept must be [B,C-1,top_k] and boxes [B,A,4]")
+    b, k, top_k = kept.shape
+    if k + 1 != state.n_classes or count.size != b * k or kept_score.size != kept.size or boxes.shape[0] != b \
+            or gt_offsets.size != b + 1:
+        raise AssertionError("detections, ground truth and evaluation state disagree in shape")
+    thr = np.ascontiguousarray(iou_thresholds, np.float64)
+    if thr.size != state.n_thresholds:
+        raise ValueError("the state was made for %d IoU thresholds" % state.n_thresholds)
+    N.check(N.lib().ssdg_eval_accumulate(
+        kept.ptr, count.ptr, kept_score.ptr, top_k, boxes.ptr, b, boxes.shape[1], state.n_classes, gt_boxes.ptr,
+        gt_cls.ptr, gt_offsets.ptr, int(max_gt), thr.ctypes.data_as(C.POINTER(C.c_double)), thr.size, state.max_dets,
+        int(image_base), state.max_images, state.ptr, state.nbytes, D.stream_handle(stream)), "eval_accumulate")
+    return (kept, count, kept_score, boxes, gt_boxes, gt_cls, gt_offsets)     # keep-alives until the stream passes
+
+
+def eval_exchange(state: EvalState) -> list:
+    """The buffers a data-parallel caller sums over the ranks, in place: [int64 keys, int32 header/flags/GT counts]."""
+    out = []
+    for which, dt in ((0, np.int64), (1, np.int32)):
+        ptr, cnt = C.c_void_p(), C.c_int64()
+        N.check(N.lib().ssdg_eval_exchange(state.ptr, state.n_classes, state.max_images, state.max_dets, which,
+                                           C.byref(ptr), C.byref(cnt)), "eval_exchange")
+        out.append(D.DeviceArray((int(cnt.value),), dt, ptr=ptr.value, owner=state))
+    return out
+
+
+def eval_status(state: EvalState, stream=None) -> int:
+    """Status bits of the state (synchronises): EVAL_STATUS_*."""
+    st = C.c_int32(0)
+    N.check(N.lib().ssdg_eval_status(state.ptr, C.byref(st), D.stream_handle(stream)), "eval_status")
+    return st.value
+
+
+def eval_finalize(state: EvalState, recall_thresholds, stream=None, pool=None) -> dict:
+    """COCOeval.accumulate over everything accumulated: device precision f64[T,R,K], recall f64[T,K],
+    n_gt i64[K], n_det i64[K].  The state is left unchanged."""
+    rec = np.ascontiguousarray(recall_thresholds, np.float64)
+    k, t, r = state.n_classes - 1, state.n_thresholds, rec.size
+    out = {"precision": D.empty((t, r, k), np.float64), "recall": D.empty((t, k), np.float64),
+           "n_gt": D.empty((k,), np.int64), "n_det": D.empty((k,), np.int64)}
+    lib = N.lib()
+    nbytes = int(lib.ssdg_eval_finalize_workspace_bytes(state.n_classes, state.max_images, state.max_dets))
+    if nbytes == 0:
+        raise N.SsdgeomError("eval_finalize: the workspace size query failed (no CUDA device?)")
+    ws = (pool or POOL).get("eval_finalize", nbytes)
+    N.check(lib.ssdg_eval_finalize(state.ptr, state.nbytes, state.n_classes, state.max_images, state.max_dets, t,
+                                   rec.ctypes.data_as(C.POINTER(C.c_double)), r, out["precision"].ptr,
+                                   out["recall"].ptr, out["n_gt"].ptr, out["n_det"].ptr, ws.ptr, ws.nbytes,
+                                   D.stream_handle(stream)), "eval_finalize")
+    out["_keep"] = (state, ws)
+    return out

@@ -19,7 +19,7 @@ INPUT_NAMES = ("gt_boxes", "gt_cls", "gt_off", "pred_cls", "pred_box")
 class HotPath:
     def __init__(self, table=None, batch=256, max_gt=100, classes=81, thresh=0.5, neg_ratio=3,
                  score_thresh=0.01, top_k=200, iou_thresh=0.45, total_gt=None, mining="shard", global_priors=None,
-                 allreduce=None, comm=None, depth=1):
+                 allreduce=None, comm=None, depth=1, evaluator=None):
         """depth: steps in flight.  1 -- ``step()`` joins both branches on ``s_main`` before it returns the stream to
         the caller (a step is a closed unit).  2 -- every per-step buffer (targets, row statistics, candidate lists,
         workspaces, results) exists twice and consecutive steps use them in turn: step k+1 starts as soon as its
@@ -34,7 +34,10 @@ class HotPath:
 
         Data-parallel exchange: ``comm`` (ssdgeom.comm.Comm, the library's own NCCL entry points) sums the additive
         loss words -- or the mining histograms -- over the processes; alternatively ``allreduce(buf, stream)`` /
-        ``loss_exchange(stream)`` callables (a torch.distributed or gloo stand-in) do."""
+        ``loss_exchange(stream)`` callables (a torch.distributed or gloo stand-in) do.
+
+        evaluator: an ``evaluate.DetectionEvaluator``; every step then also matches its kept lists to its ground truth
+        (``step(image_base)``) after the NMS, on the NMS stream.  None (the default) changes nothing."""
         table = SSD300 if table is None else table
         self.batch, self.max_gt, self.classes = int(batch), int(max_gt), int(classes)
         self.thresh, self.neg_ratio = float(thresh), int(neg_ratio)
@@ -49,12 +52,18 @@ class HotPath:
         self._bind(self._sets[0])
         self.depth = 1 if mining == "global" else max(1, int(depth))
         self._n_steps = 0
+        self.evaluator = evaluator
+        if evaluator is not None and (evaluator.n_classes != c or evaluator.max_dets > self.top_k):
+            raise ValueError("the evaluator needs n_classes == classes and max_dets <= top_k")
 
         def make_slot():   # everything a step writes
+            det = {"kept": D.empty((b, c - 1, self.top_k), np.int32), "count": D.empty((b, c - 1), np.int32)}
+            if evaluator is not None:   # the filter then writes the decoded boxes here instead of into its workspace
+                det.update(kept_score=D.empty((b, c - 1, self.top_k), np.float32), boxes=D.empty((b, a, 4), np.float32))
             return {"tgt": {"cls": D.empty((b, a), np.int32), "loc": D.empty((b, a, 4), np.float32),
                             "mask": D.empty((b, a), np.uint8)},
                     "loss": {"result": D.empty((N.LOSS_RESULT_LEN,), np.float64)},
-                    "det": {"kept": D.empty((b, c - 1, self.top_k), np.int32), "count": D.empty((b, c - 1), np.int32)},
+                    "det": det,
                     "det_stats": {"row_ml": D.empty((b, a, 2), np.float32), "row_negbg": D.empty((b, a), np.float32)},
                     "pool": ops.WorkspacePool(), "ev_a": D.Event(), "ev_d": D.Event(), "ev_x": D.Event(),
                     "x_pending": False, "used": False, "loss_exchange": None}
@@ -113,7 +122,7 @@ class HotPath:
             self.staged = ops.StagedLoss(self.tgt["cls"], self.tgt["loc"], self.tgt["mask"], self.pred_box, self.pred_cls,
                                          int(global_priors), self.neg_ratio, out=self.loss)
         # search, match | lossprep (or ce), select x2, final | filter, nms per slice of the post-processing
-        self.kernel_launches_per_step = 6 + 2 * self.detect_parts
+        self.kernel_launches_per_step = 6 + 2 * self.detect_parts + (1 if evaluator is not None else 0)
         # matcher head + loss histograms (cudaMemsetAsync), + the lead node of small batches
         self.memsets_per_step = 2 + (1 if self.lead_assign else 0)
         self.h2d_bytes = sum(self._sets[0][k].nbytes for k in INPUT_NAMES)
@@ -206,8 +215,12 @@ class HotPath:
                    self.iou_thresh, out={k: rows(v) for k, v in out.items()}, stream=stream, stage=stage,
                    want_row_stats=stats, ws_key="detect%d" % part, pool=self.pool)
 
-    def step(self):
-        """One pass of the chain over the resident batch; work is ordered on ``s_main``.
+    def evaluate_stage(self, stream, image_base=None):
+        self.evaluator.add(self.det, self.gt_boxes, self.gt_cls, self.gt_off, image_base, stream, max_gt=self.max_gt)
+
+    def step(self, image_base=None):
+        """One pass of the chain over the resident batch; work is ordered on ``s_main``.  With an evaluator the batch's
+        images get the global indices ``image_base ..`` (None: after the highest added so far).
 
         Four streams so that kernels bound by different resources share the SMs:
           phase A   the filter pass (HBM-bound, s_d, high priority)     with  the matcher (latency-bound, s_a, high)
@@ -244,6 +257,8 @@ class HotPath:
             for part in range(parts):
                 D.stream_wait_event(self.s_n, self.ev_parts[part])
                 self.detect_stage(self.s_n, stage=1, stats=fused, part=part if parts > 1 else None)
+            if self.evaluator is not None:      # before ev_d: the waits on ev_d cover its reads of GT and lists
+                self.evaluate_stage(self.s_n, image_base)
             D.stream_wait_event(self.s_l, self.ev_m)
             if fused:
                 D.stream_wait_event(self.s_l, self.ev_mid)
@@ -263,6 +278,8 @@ class HotPath:
             self.ev_d.record(self.s_n)
         else:
             self.detect_stage(self.s_d)
+            if self.evaluator is not None:
+                self.evaluate_stage(self.s_d, image_base)
             self.assign(self.s_a)
             self.loss_stage(self.s_a)
             if loss_exchange is not None:

@@ -73,3 +73,22 @@ def make_predictions(seed: int, batch: int, num_anchors: int, num_classes: int =
     pred_cls[..., -1] += np.float32(bg_bias)
     pred_box = rng.standard_normal(size=(batch, num_anchors, 4), dtype=np.float32) * np.float32(0.5)
     return pred_cls, pred_box
+
+
+def make_trained_predictions(seed: int, tgt_cls, tgt_loc, tgt_mask, num_classes: int = 81, bg_bias: float = 7.0,
+                             max_noise: float = 0.25, boost=(3.0, 12.0)):
+    """Predictions of a partly trained detector, built from the matcher's targets (cls i32[B,A], loc f32[B,A,4], mask
+    [B,A]) so that AP is meaningful: every positive prior gets its encoded target plus N(0, s^2) noise with s ~
+    U(0, max_noise) per prior (IoUs spread over all COCO thresholds) and its ground-truth logit raised by U(boost);
+    everything else is ``make_predictions``."""
+    tgt_cls, tgt_loc = np.asarray(tgt_cls), np.asarray(tgt_loc, np.float32)
+    pos = np.asarray(tgt_mask).astype(bool)
+    b, a = pos.shape
+    pred_cls, pred_box = make_predictions(seed, b, a, num_classes, bg_bias)
+    rng = np.random.default_rng(seed + 104729)
+    n = int(pos.sum())
+    sigma = rng.uniform(0.0, max_noise, size=(n, 1))
+    pred_box[pos] = (tgt_loc[pos] + rng.standard_normal(size=(n, 4)) * sigma).astype(np.float32)
+    bi, ai = np.nonzero(pos)
+    pred_cls[bi, ai, tgt_cls[pos]] += rng.uniform(boost[0], boost[1], size=n).astype(np.float32)
+    return pred_cls, pred_box
