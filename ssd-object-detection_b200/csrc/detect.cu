@@ -235,9 +235,14 @@ __device__ __forceinline__ void filter_tile(const DetectParams& P, int b, int j,
         // every e_c carries the common factor 2^d, d = ref*log2e + kexp (the rounding of kexp; exact in one FMA):
         // it cancels in e/sum, the logarithm takes it out explicitly
         const float d = fmaf(ref, SSDG_LOG2E, kexp);
-        const float lg = fmaf(-d, 0.693147180559945f, logf(s0 + s1));
+        const float s = s0 + s1;
+        const float lg = fmaf(-d, 0.693147180559945f, logf(s));
         P.row_ml[n] = make_float2(ref, lg);
-        P.row_negbg[n] = lg - (xbg - ref);
+        // With the background as the reference its own term e_bg = 2^d (the same exp2 of the same argument) opens the
+        // sum, and the background CE log(s / e_bg) is >= 0: exactly 0 when the rest of the sum is lost in rounding
+        // (s == e_bg; the max-shifted formula of the standalone CE pass has log 1 there), else lg, whose rounding of
+        // d (either sign, ~1e-7) is held at +0.
+        P.row_negbg[n] = xbg != ref ? lg - (xbg - ref) : (s != exp2_ftz(d) && lg > 0.f ? lg : 0.f);
       }
     } else {
       const int lim = min(nfg, 96);

@@ -516,16 +516,44 @@ def test_detect_other_parameters(priors300):
         _check_detect(pred_cls, pred_box, priors300, **kw)
 
 
-def test_detect_many_classes_and_odd_shapes():
-    """C > 97 (classes beyond the register bit-sets), prior counts that are not multiples of 4 or 32
-    (the non-TMA tile path), tiny images."""
+# Foreground class counts at every boundary of the filter's class words: <= 32, <= 64, (64, 80] (two lanes share a
+# class of the third word), (80, 96), exactly 96 (the last streaming case) and 97 (the two-pass variant), with prior
+# counts that are not multiples of 4 or 32 (the non-TMA tile path).
+FILTER_WORD_CASES = [(2, 203, nfg + 1, 2.0) for nfg in (1, 16, 31, 32, 33, 63, 64, 65, 79, 80, 81, 90, 95, 96, 97)]
+# SSD300-sized rows (8 732 priors): the COCO label space of torchvision's SSD (91) and each side of the two-pass switch
+FILTER_SSD300_CLASSES = (91, 97, 98)
+
+
+def _rand_detect_inputs(rng, b, a, c, bias):
+    pri = np.concatenate([rng.uniform(0.1, 0.9, (a, 2)), rng.uniform(0.05, 0.4, (a, 2))], 1)
+    pred_cls = rng.normal(size=(b, a, c)).astype(np.float32)
+    pred_cls[..., -1] += bias
+    pred_box = (rng.normal(size=(b, a, 4)) * 0.3).astype(np.float32)
+    return pred_cls, pred_box, pri
+
+
+def test_detect_many_classes_and_odd_shapes(priors300):
+    """C > 97 (classes beyond the register bit-sets), every class-word boundary of the filter, prior counts that are
+    not multiples of 4 or 32 (the non-TMA tile path), tiny images."""
     rng = np.random.default_rng(12)
-    for (b, a, c, bias) in [(2, 333, 130, 3.0), (3, 64, 21, 2.0), (1, 37, 5, 0.0), (2, 1000, 200, 4.0)]:
-        pri = np.concatenate([rng.uniform(0.1, 0.9, (a, 2)), rng.uniform(0.05, 0.4, (a, 2))], 1)
-        pred_cls = rng.normal(size=(b, a, c)).astype(np.float32)
-        pred_cls[..., -1] += bias
-        pred_box = (rng.normal(size=(b, a, 4)) * 0.3).astype(np.float32)
+    for (b, a, c, bias) in [(2, 333, 130, 3.0), (3, 64, 21, 2.0), (1, 37, 5, 0.0), (2, 1000, 200, 4.0)] + FILTER_WORD_CASES:
+        pred_cls, pred_box, pri = _rand_detect_inputs(rng, b, a, c, bias)
         _check_detect(pred_cls, pred_box, pri, score_thresh=0.01, top_k=100, iou_thresh=0.45)
+    for c in FILTER_SSD300_CLASSES:
+        pred_cls, pred_box = synth.make_predictions(90 + c, 1, 8732, c, bg_bias=4.0)
+        _check_detect(pred_cls, pred_box, priors300, score_thresh=0.01, top_k=100, iou_thresh=0.45)
+
+
+@pytest.mark.parametrize("b,a,c,bias", FILTER_WORD_CASES + [(1, 8732, c, 4.0) for c in FILTER_SSD300_CLASSES])
+def test_detect_streaming_filter_word_boundaries(b, a, c, bias, priors300):
+    """The streaming variant (background logit as the exponent reference, row statistics for the loss) at the same
+    class counts: kept scores, row_ml and row_negbg against the float64 oracle, the lists end to end."""
+    rng = np.random.default_rng(1000 + c)
+    pred_cls, pred_box, pri = _rand_detect_inputs(rng, b, a, c, bias)
+    if a == 8732:
+        pri = priors300
+    eq, lists = _check_detect_streaming(pred_cls, pred_box, pri, score_thresh=0.01, top_k=100, iou_thresh=0.45)
+    assert eq >= lists - 2, "end-to-end kept lists equal to the float64 oracle: %d of %d" % (eq, lists)
 
 
 def test_nms_on_oracle_inputs_bit_exact(priors300):
