@@ -93,6 +93,42 @@ struct CeAcc {
   int npos;
 };
 
+// Positive prior n adds ce_of(its ground-truth class), its L1 box distance and 1 to the thread's sums.
+template <typename CeOf>
+__device__ __forceinline__ void add_positive(const LossParams& P, long long n, CeOf ce_of, CeAcc& acc) {
+  int lab = P.gt_cls[n];
+  if (lab < 0 || lab >= P.C) {   // TensorFlow raises here (models/ssd_model.py:357): flagged through the status word
+    atomicAdd(&P.ws->nparts[1], 1u);
+    lab = lab < 0 ? 0 : P.C - 1;
+  }
+  acc.pos_ce += ce_of(lab);
+  const float4 pb = __ldg(reinterpret_cast<const float4*>(P.pred_box) + n);
+  const float4 gb = __ldg(reinterpret_cast<const float4*>(P.gt_box) + n);
+  acc.l1 += (fabsf(pb.x - gb.x) + fabsf(pb.y - gb.y)) + (fabsf(pb.z - gb.z) + fabsf(pb.w - gb.w));
+  acc.npos += 1;
+}
+
+// The end of a CE pass (kCeThreads threads): the CTA's three sums in double, reduced in a fixed order into
+// ws->part[blockIdx.x]; the grid size, the integer positives count and the CTA's level-0 histogram.
+__device__ __forceinline__ void ce_pass_flush(const LossParams& P, const CeAcc& acc, const u32* hist,
+                                              double* red /*[3][kCeWarps]*/, int tid) {
+  const int lane = tid & 31, warp = tid >> 5;
+  double a = warp_sum((double)acc.pos_ce), b = warp_sum((double)acc.l1), c = warp_sum((double)acc.npos);
+  if (lane == 0) { red[warp] = a; red[kCeWarps + warp] = b; red[2 * kCeWarps + warp] = c; }
+  __syncthreads();
+  if (tid == 0) {
+    double sa = 0, sb = 0, sc = 0;
+    for (int w = 0; w < kCeWarps; ++w) { sa += red[w]; sb += red[kCeWarps + w]; sc += red[2 * kCeWarps + w]; }
+    P.ws->part[blockIdx.x][0] = sa; P.ws->part[blockIdx.x][1] = sb; P.ws->part[blockIdx.x][2] = sc;
+    if (blockIdx.x == 0) P.ws->nparts[0] = gridDim.x;
+    atomicAdd(&P.ws->xnpos, (unsigned long long)sc);   // integer, order-independent
+  }
+  for (int i = tid; i < kBins; i += kCeThreads) {
+    const u32 v = hist[i];
+    if (v) atomicAdd(&P.ws->hist[0][i], v);
+  }
+}
+
 // Per-prior work shared by the TMA path and the tail path.
 __device__ __forceinline__ void ce_one_prior(const LossParams& P, long long n, const float* row, u32* hist, CeAcc& acc) {
   const int C = P.C;
@@ -102,16 +138,7 @@ __device__ __forceinline__ void ce_one_prior(const LossParams& P, long long n, c
   const bool pos = P.gt_mask[n] != 0;
   float neg = 0.f;
   if (pos) {
-    int lab = P.gt_cls[n];
-    if (lab < 0 || lab >= C) {   // TensorFlow raises here (models/ssd_model.py:357): flagged through the status word
-      atomicAdd(&P.ws->nparts[1], 1u);
-      lab = lab < 0 ? 0 : C - 1;
-    }
-    acc.pos_ce += lg - (row[lab] - m);
-    const float4 pb = __ldg(reinterpret_cast<const float4*>(P.pred_box) + n);
-    const float4 gb = __ldg(reinterpret_cast<const float4*>(P.gt_box) + n);
-    acc.l1 += (fabsf(pb.x - gb.x) + fabsf(pb.y - gb.y)) + (fabsf(pb.z - gb.z) + fabsf(pb.w - gb.w));
-    acc.npos += 1;
+    add_positive(P, n, [&](int lab) { return lg - (row[lab] - m); }, acc);
   } else {
     neg = lg - (row[C - 1] - m);
   }
@@ -179,21 +206,7 @@ __global__ void __launch_bounds__(kCeThreads, 1) ce_kernel(LossParams P, int war
       if (lane < tail) ce_one_prior(P, (full_tiles << 5) + lane, buf + (size_t)lane * C, hist, acc);
     }
   }
-  // block reduction of the three sums (double), one partial per CTA
-  double a = warp_sum((double)acc.pos_ce), b = warp_sum((double)acc.l1), c = warp_sum((double)acc.npos);
-  if (lane == 0) { red[warp] = a; red[kCeWarps + warp] = b; red[2 * kCeWarps + warp] = c; }
-  __syncthreads();
-  if (tid == 0) {
-    double sa = 0, sb = 0, sc = 0;
-    for (int w = 0; w < kCeWarps; ++w) { sa += red[w]; sb += red[kCeWarps + w]; sc += red[2 * kCeWarps + w]; }
-    P.ws->part[blockIdx.x][0] = sa; P.ws->part[blockIdx.x][1] = sb; P.ws->part[blockIdx.x][2] = sc;
-    if (blockIdx.x == 0) P.ws->nparts[0] = gridDim.x;
-    atomicAdd(&P.ws->xnpos, (unsigned long long)sc);   // integer, order-independent
-  }
-  for (int i = tid; i < kBins; i += kCeThreads) {
-    u32 v = hist[i];
-    if (v) atomicAdd(&P.ws->hist[0][i], v);
-  }
+  ce_pass_flush(P, acc, hist, red, tid);
 }
 
 // ---- the CE pass without the logits ----------------------------------------------------------------------
@@ -201,31 +214,24 @@ __global__ void __launch_bounds__(kCeThreads, 1) ce_kernel(LossParams P, int war
 // with row statistics), the loss needs no second pass over them: the background CE is there, and the positives
 // (a few percent of the priors) gather their one ground-truth logit.  Same outputs as ce_kernel: the mining
 // vector, its level-0 histogram, the per-CTA partial sums, the positives count.
-__global__ void __launch_bounds__(256) lossprep_kernel(LossParams P) {
+__global__ void __launch_bounds__(kCeThreads) lossprep_kernel(LossParams P) {
   __shared__ u32 hist[kBins];
-  __shared__ double red[3][8];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  for (int i = tid; i < kBins; i += 256) hist[i] = 0u;
+  __shared__ double red[3 * kCeWarps];
+  const int tid = threadIdx.x;
+  for (int i = tid; i < kBins; i += kCeThreads) hist[i] = 0u;
   __syncthreads();
   CeAcc acc;
   acc.pos_ce = 0.f; acc.l1 = 0.f; acc.npos = 0;
   const int C = P.C;
   auto one = [&](long long n, bool pos, float negbg) -> float {
     if (!pos) return negbg;
-    int lab = P.gt_cls[n];
-    if (lab < 0 || lab >= C) {   // as in ce_one_prior
-      atomicAdd(&P.ws->nparts[1], 1u);
-      lab = lab < 0 ? 0 : C - 1;
-    }
-    const float2 ml = P.row_ml[n];
-    acc.pos_ce += ml.y - (__ldg(P.pred_cls + (size_t)n * C + lab) - ml.x);
-    const float4 pb = __ldg(reinterpret_cast<const float4*>(P.pred_box) + n);
-    const float4 gb = __ldg(reinterpret_cast<const float4*>(P.gt_box) + n);
-    acc.l1 += (fabsf(pb.x - gb.x) + fabsf(pb.y - gb.y)) + (fabsf(pb.z - gb.z) + fabsf(pb.w - gb.w));
-    acc.npos += 1;
+    add_positive(P, n, [&](int lab) {
+      const float2 ml = P.row_ml[n];
+      return ml.y - (__ldg(P.pred_cls + (size_t)n * C + lab) - ml.x);
+    }, acc);
     return 0.f;
   };
-  const long long gtid = (long long)blockIdx.x * 256 + tid, gstride = (long long)gridDim.x * 256;
+  const long long gtid = (long long)blockIdx.x * kCeThreads + tid, gstride = (long long)gridDim.x * kCeThreads;
   const bool vec = (((uintptr_t)P.gt_mask) & 3) == 0 && (((uintptr_t)P.row_negbg | (uintptr_t)P.neg_ce) & 15) == 0;
   long long done = 0;
   if (vec) {
@@ -247,20 +253,7 @@ __global__ void __launch_bounds__(256) lossprep_kernel(LossParams P) {
     P.neg_ce[n] = v;
     atomicAdd(&hist[key32(v) >> 21], 1u);
   }
-  double a = warp_sum((double)acc.pos_ce), b = warp_sum((double)acc.l1), c = warp_sum((double)acc.npos);
-  if (lane == 0) { red[0][warp] = a; red[1][warp] = b; red[2][warp] = c; }
-  __syncthreads();
-  if (tid == 0) {
-    double sa = 0, sb = 0, sc = 0;
-    for (int w = 0; w < 8; ++w) { sa += red[0][w]; sb += red[1][w]; sc += red[2][w]; }
-    P.ws->part[blockIdx.x][0] = sa; P.ws->part[blockIdx.x][1] = sb; P.ws->part[blockIdx.x][2] = sc;
-    if (blockIdx.x == 0) P.ws->nparts[0] = gridDim.x;
-    atomicAdd(&P.ws->xnpos, (unsigned long long)sc);
-  }
-  for (int i = tid; i < kBins; i += 256) {
-    const u32 v = hist[i];
-    if (v) atomicAdd(&P.ws->hist[0][i], v);
-  }
+  ce_pass_flush(P, acc, hist, red, tid);
 }
 
 // ---- radix select ------------------------------------------------------------------------------------
@@ -277,8 +270,7 @@ struct SelectState {
 // 256 threads, each owns nbins/256 consecutive bins (from the top) in registers: one round of global loads,
 // a shuffle scan per warp and an 8-entry cross-warp prefix.
 __device__ int scan_level(const u32* __restrict__ ghist, int nbins, long long& k, u32* sh /*[kBins]*/, int tid,
-                          int nthreads, int* sh_bin, long long* sh_above) {
-  (void)nthreads;   // launch bounds of the callers: 256
+                          int* sh_bin, long long* sh_above) {
   const int per = nbins >> 8;   // 8 or 4
   const int hi = nbins - 1 - tid * per;
   u32 c[8];
@@ -319,8 +311,8 @@ __device__ int scan_level(const u32* __restrict__ ghist, int nbins, long long& k
   return bin;
 }
 
-__device__ void derive_state(const LossParams& P, int levels_done, SelectState& st, u32* sh, int tid, int nthreads,
-                             int* sh_bin, long long* sh_above, double* sh_np) {
+__device__ void derive_state(const LossParams& P, int levels_done, SelectState& st, u32* sh, int tid, int* sh_bin,
+                             long long* sh_above, double* sh_np) {
   if (tid < 32) {
     // counts are integers < 2^53: the sum is exact in any order
     double np = 0;
@@ -336,9 +328,9 @@ __device__ void derive_state(const LossParams& P, int levels_done, SelectState& 
   st.status = 0;
   if (st.num_pos <= 0 || P.ratio <= 0) { st.status = SSDG_ERR_NO_POSITIVE; return; }
   if (st.k > P.N_all) { st.status = SSDG_ERR_TOPK_RANGE; return; }
-  if (levels_done >= 1) st.prefix = (u32)scan_level(P.ws->hist[0], kBins, st.k, sh, tid, nthreads, sh_bin, sh_above) << 21;
-  if (levels_done >= 2) st.prefix |= (u32)scan_level(P.ws->hist[1], kBins, st.k, sh, tid, nthreads, sh_bin, sh_above) << 10;
-  if (levels_done >= 3) st.prefix |= (u32)scan_level(P.ws->hist[2], 1024, st.k, sh, tid, nthreads, sh_bin, sh_above);
+  if (levels_done >= 1) st.prefix = (u32)scan_level(P.ws->hist[0], kBins, st.k, sh, tid, sh_bin, sh_above) << 21;
+  if (levels_done >= 2) st.prefix |= (u32)scan_level(P.ws->hist[1], kBins, st.k, sh, tid, sh_bin, sh_above) << 10;
+  if (levels_done >= 3) st.prefix |= (u32)scan_level(P.ws->hist[2], 1024, st.k, sh, tid, sh_bin, sh_above);
 }
 
 // level = 1: histogram bits 20..10 of keys whose bits 31..21 match; level = 2: bits 9..0.
@@ -349,7 +341,7 @@ __global__ void __launch_bounds__(256) select_kernel(LossParams P, int level) {
   __shared__ double sh_np;
   pdl_wait();      // the previous level's histogram must be complete
   SelectState st;
-  derive_state(P, level, st, sh, threadIdx.x, blockDim.x, &sh_bin, &sh_above, &sh_np);
+  derive_state(P, level, st, sh, threadIdx.x, &sh_bin, &sh_above, &sh_np);
   if (st.status) return;
   for (int i = threadIdx.x; i < kBins; i += blockDim.x) sh[i] = 0u;
   __syncthreads();
@@ -389,7 +381,7 @@ __global__ void __launch_bounds__(256) final_kernel(LossParams P) {
   __shared__ bool is_last;
   pdl_wait();      // the last level's histogram must be complete
   SelectState st;
-  derive_state(P, 3, st, sh, threadIdx.x, blockDim.x, &sh_bin, &sh_above, &sh_np);
+  derive_state(P, 3, st, sh, threadIdx.x, &sh_bin, &sh_above, &sh_np);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const u32 kth = st.prefix;
   double sum = 0;
@@ -621,9 +613,15 @@ extern "C" size_t ssdg_loss_workspace_bytes(int64_t batch, int32_t n_priors, int
   return align_up(sizeof(LossWs), 256) + align_up((size_t)batch * n_priors * 4, 256);
 }
 
-// stages: 1 = CE pass (+ level-0 histogram, positives count), 2 / 4 = radix levels 1 / 2, 8 = mask, sums, result,
-// 16 = gradient (reads the result block: in a cross-shard run AFTER its exchange, so that 1/num_neg is the global
-// count).  Between the stages of a cross-shard run the caller sums the exchange words over the shards.
+// The stages one loss_run call enqueues, a bit set; stage k of ssdg_multibox_loss_stage is bit k.  Between the stages
+// of a cross-shard run the caller sums the exchange words over the shards.
+constexpr int kStageCe = 1;                         // CE pass (+ level-0 histogram, positives count)
+constexpr int kStageLevel1 = 2, kStageLevel2 = 4;   // radix levels 1 and 2
+constexpr int kStageFinal = 8;                      // mask, sums, result
+constexpr int kStageGrad = 16;                      // gradient: in a cross-shard run AFTER the last exchange
+                                                    // (it reads the global num_neg from the result block)
+constexpr int kStageAll = kStageCe | kStageLevel1 | kStageLevel2 | kStageFinal | kStageGrad;
+
 static int loss_run(int stages, int global, long long n_all, const float* row_ml, const float* row_negbg,
                     const int32_t* gt_cls, const float* gt_box,
                     const uint8_t* gt_mask, const float* pred_box, const float* pred_cls, int64_t batch,
@@ -650,7 +648,7 @@ static int loss_run(int stages, int global, long long n_all, const float* row_ml
   P.ws = (LossWs*)workspace;
   P.neg_ce = out_neg_ce ? out_neg_ce : (float*)((unsigned char*)workspace + align_up(sizeof(LossWs), 256));
   P.neg_mask = out_neg_mask; P.result = out_result; P.grad_box = grad_box; P.grad_cls = grad_cls;
-  if (stages & 1) {
+  if (stages & kStageCe) {
     SSDG_CUDA_TRY(cudaMemsetAsync(&P.ws->hist[0][0], 0, sizeof(LossWs) - offsetof(LossWs, hist), st));
     prof_begin(SSDG_PROF_CE, st);
     if (row_ml) {
@@ -658,7 +656,7 @@ static int loss_run(int stages, int global, long long n_all, const float* row_ml
       if (grid > 256) grid = 256;   // LossWs::part
       if (grid < 1) grid = 1;
       SSDG_CUDA_TRY(cudaFuncSetAttribute(lossprep_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      lossprep_kernel<<<grid, 256, 0, st>>>(P);
+      lossprep_kernel<<<grid, kCeThreads, 0, st>>>(P);
     } else {
       const size_t smem = ce_smem_bytes(n_classes, warps);
       SSDG_CUDA_TRY(cudaFuncSetAttribute(ce_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -676,20 +674,20 @@ static int loss_run(int stages, int global, long long n_all, const float* row_ml
   const long long sneed = (P.N / 4 + 255) / 256;
   if (sneed < sgrid) sgrid = (int)(sneed > 0 ? sneed : 1);
   if (sgrid > 1024) sgrid = 1024;
-  if (stages & 6) prof_begin(SSDG_PROF_LOSS_TAIL, st);
-  if (stages & 6) {
+  if (stages & (kStageLevel1 | kStageLevel2)) {
+    prof_begin(SSDG_PROF_LOSS_TAIL, st);
     SSDG_CUDA_TRY(cudaFuncSetAttribute(select_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    if (stages & 2) SSDG_CUDA_TRY(launch_pdl(select_kernel, dim3(sgrid), dim3(256), 0, st, P, 1));
-    if (stages & 4) SSDG_CUDA_TRY(launch_pdl(select_kernel, dim3(sgrid), dim3(256), 0, st, P, 2));
+    if (stages & kStageLevel1) SSDG_CUDA_TRY(launch_pdl(select_kernel, dim3(sgrid), dim3(256), 0, st, P, 1));
+    if (stages & kStageLevel2) SSDG_CUDA_TRY(launch_pdl(select_kernel, dim3(sgrid), dim3(256), 0, st, P, 2));
     SSDG_LAUNCH_CHECK();
   }
-  if (stages & 8) {
+  if (stages & kStageFinal) {
     SSDG_CUDA_TRY(cudaFuncSetAttribute(final_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     SSDG_CUDA_TRY(launch_pdl(final_kernel, dim3(sgrid), dim3(256), 0, st, P));
     prof_end(SSDG_PROF_LOSS_TAIL, st);
     SSDG_LAUNCH_CHECK();
   }
-  if ((stages & 16) && grad_cls) {
+  if ((stages & kStageGrad) && grad_cls) {
     prof_begin(SSDG_PROF_GRAD, st);
     SSDG_CUDA_TRY(cudaMemsetAsync(grad_cls, 0, (size_t)P.N * n_classes * sizeof(float), st));
     {
@@ -709,8 +707,9 @@ extern "C" int ssdg_multibox_loss(const int32_t* gt_cls, const float* gt_box, co
                                   int32_t n_classes, int32_t neg_ratio, double* out_result, uint8_t* out_neg_mask,
                                   float* out_neg_ce, float* grad_box, float* grad_cls, void* workspace,
                                   size_t workspace_bytes, void* stream) {
-  return loss_run(31, 0, 0, nullptr, nullptr, gt_cls, gt_box, gt_mask, pred_box, pred_cls, batch, n_priors, n_classes, neg_ratio,
-                  out_result, out_neg_mask, out_neg_ce, grad_box, grad_cls, workspace, workspace_bytes, stream);
+  return loss_run(kStageAll, 0, 0, nullptr, nullptr, gt_cls, gt_box, gt_mask, pred_box, pred_cls, batch, n_priors,
+                  n_classes, neg_ratio, out_result, out_neg_mask, out_neg_ce, grad_box, grad_cls, workspace,
+                  workspace_bytes, stream);
 }
 
 extern "C" int ssdg_multibox_loss_stage(int32_t stage, int64_t global_priors, const float* row_ml,
@@ -734,8 +733,9 @@ extern "C" int ssdg_multibox_loss_fused(const float* row_ml, const float* row_ne
                                         float* out_neg_ce, float* grad_box, float* grad_cls, void* workspace,
                                         size_t workspace_bytes, void* stream) {
   if (!row_ml || !row_negbg) return SSDG_ERR_ARG;
-  return loss_run(31, 0, 0, row_ml, row_negbg, gt_cls, gt_box, gt_mask, pred_box, pred_cls, batch, n_priors, n_classes,
-                  neg_ratio, out_result, out_neg_mask, out_neg_ce, grad_box, grad_cls, workspace, workspace_bytes, stream);
+  return loss_run(kStageAll, 0, 0, row_ml, row_negbg, gt_cls, gt_box, gt_mask, pred_box, pred_cls, batch, n_priors,
+                  n_classes, neg_ratio, out_result, out_neg_mask, out_neg_ce, grad_box, grad_cls, workspace,
+                  workspace_bytes, stream);
 }
 
 extern "C" int ssdg_loss_exchange(void* workspace, int32_t which, void** out_ptr, int64_t* out_count) {

@@ -17,6 +17,12 @@ ERR_NCCL_BASE = 10000
 F32, F64, I32, I64 = 0, 1, 2, 3
 COMM_ID_BYTES = 128
 LOSS_RESULT_LEN = 16
+# words of the loss result block (include/ssdgeom.h, out_result)
+LOSS_TOTAL, LOSS_POS, LOSS_NEG, LOSS_LOC = 0, 1, 2, 3     # total, "cls loss pos", "cls loss neg", "loc loss"
+LOSS_NUM_POS, LOSS_NUM_NEG, LOSS_KTH, LOSS_STATUS = 4, 5, 6, 7
+LOSS_SUM_POS_CE, LOSS_SUM_NEG_CE, LOSS_SUM_L1 = 8, 9, 10
+LOSS_OWN_POS, LOSS_ERRORS = 11, 12     # this shard's own positives; its data-dependent error count
+LOSS_ADDITIVE = slice(LOSS_NUM_POS, LOSS_OWN_POS)   # [4, 11): summed over the shards with per-shard mining
 PROF_MATCH, PROF_CE, PROF_FILTER, PROF_NMS = 0, 1, 2, 3
 PROF_BUCKET, PROF_SEARCH, PROF_LOSS_TAIL, PROF_GRAD = 4, 5, 6, 7
 

@@ -41,7 +41,7 @@ class _MultiboxLoss(torch.autograd.Function):
         if need_grad:
             ctx.save_for_backward(out["grad_box"], out["grad_cls"])
         ctx.mark_non_differentiable(result)
-        return result[0].clone(), result
+        return result[N.LOSS_TOTAL].clone(), result
 
     @staticmethod
     def backward(ctx, g_total, _g_result):
@@ -63,6 +63,6 @@ def ssd_loss(y_true, y_pred, neg_ratio: int = 3, check: bool = False):
     total, result = _MultiboxLoss.apply(pred_box, pred_cls, gt_cls, gt_box, gt_mask, neg_ratio)
     if check:
         ops.loss_result_to_host(result)       # raises IndexError / ValueError / AssertionError like the reference
-    info = {"cls loss pos": result[1], "cls loss neg": result[2], "loc loss": result[3],
-            "num_pos": result[4], "num_neg": result[5]}
+    info = {"cls loss pos": result[N.LOSS_POS], "cls loss neg": result[N.LOSS_NEG], "loc loss": result[N.LOSS_LOC],
+            "num_pos": result[N.LOSS_NUM_POS], "num_neg": result[N.LOSS_NUM_NEG]}
     return total, info

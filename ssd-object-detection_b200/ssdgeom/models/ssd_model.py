@@ -29,21 +29,25 @@ def build_prior_box(size_list, s_k_refer=None, aspect_ratio=None, input_size=300
     return out if device_out else out.to_host()
 
 
-def ssd_loss(y_true, y_pred, neg_ratio=3, return_aux=False):
-    """``_ssd_loss(y_true, y_pred)`` (models/ssd_model.py:341-396):
-    y_true = (gt_cls int32[b,A], gt_box f32[b,A,4], gt_mask bool[b,A]); y_pred = (pred_box, pred_cls).
-    Returns (total, {"cls loss pos", "cls loss neg", "loc loss"})."""
+def _loss(y_true, y_pred, neg_ratio, **want):
+    """The device loss of host or device arrays: (host result dict, info, device outputs)."""
     gt_cls, gt_box, gt_mask = y_true
     pred_box, pred_cls = y_pred
     if not D.is_device(gt_mask):
         gt_mask = np.ascontiguousarray(np.asarray(gt_mask).astype(np.uint8))
-    shapes = [tuple(np.shape(v)) if not D.is_device(v) else tuple(v.shape) for v in (gt_cls, gt_box, gt_mask, pred_box, pred_cls)]
+    out = ops.multibox_loss(gt_cls, gt_box, gt_mask, pred_box, pred_cls, neg_ratio, **want)
+    r = ops.loss_result_to_host(out["result"])
+    return r, {k: r[k] for k in ("cls loss pos", "cls loss neg", "loc loss")}, out
+
+
+def ssd_loss(y_true, y_pred, neg_ratio=3, return_aux=False):
+    """``_ssd_loss(y_true, y_pred)`` (models/ssd_model.py:341-396):
+    y_true = (gt_cls int32[b,A], gt_box f32[b,A,4], gt_mask bool[b,A]); y_pred = (pred_box, pred_cls).
+    Returns (total, {"cls loss pos", "cls loss neg", "loc loss"})."""
+    shapes = [tuple(np.shape(v)) if not D.is_device(v) else tuple(v.shape) for v in (*y_true, *y_pred)]
     assert shapes[0][0] == shapes[1][0] == shapes[2][0] == shapes[3][0] == shapes[4][0]   # :347-348
     assert shapes[0][:2] == shapes[4][:2]                                                   # :350-351
-    out = ops.multibox_loss(gt_cls, gt_box, gt_mask, pred_box, pred_cls, neg_ratio,
-                            want_neg_mask=return_aux, want_neg_ce=return_aux)
-    r = ops.loss_result_to_host(out["result"])
-    info = {"cls loss pos": r["cls loss pos"], "cls loss neg": r["cls loss neg"], "loc loss": r["loc loss"]}
+    r, info, out = _loss(y_true, y_pred, neg_ratio, want_neg_mask=return_aux, want_neg_ce=return_aux)
     if return_aux:
         aux = dict(r, neg_mask=out["neg_mask"].to_host().astype(bool), neg_ce=out["neg_ce"].to_host())
         return r["total"], info, aux
@@ -53,13 +57,7 @@ def ssd_loss(y_true, y_pred, neg_ratio=3, return_aux=False):
 def ssd_loss_grad(y_true, y_pred, neg_ratio=3):
     """Loss plus what ``tape.gradient`` (models/ssd_model.py:248) propagates to the predictions:
     returns (total, info, grad_pred_box f32[b,A,4], grad_pred_cls f32[b,A,C])."""
-    gt_cls, gt_box, gt_mask = y_true
-    pred_box, pred_cls = y_pred
-    if not D.is_device(gt_mask):
-        gt_mask = np.ascontiguousarray(np.asarray(gt_mask).astype(np.uint8))
-    out = ops.multibox_loss(gt_cls, gt_box, gt_mask, pred_box, pred_cls, neg_ratio, want_grad=True)
-    r = ops.loss_result_to_host(out["result"])
-    info = {"cls loss pos": r["cls loss pos"], "cls loss neg": r["cls loss neg"], "loc loss": r["loc loss"]}
+    r, info, out = _loss(y_true, y_pred, neg_ratio, want_grad=True)
     return r["total"], info, out["grad_box"].to_host(), out["grad_cls"].to_host()
 
 

@@ -10,6 +10,7 @@ import numpy as np
 
 from . import _native as N
 from . import device as D
+from .parallel import loss_from_sums
 
 _DT = {np.dtype(np.float32): N.F32, np.dtype(np.float64): N.F64}
 
@@ -237,12 +238,10 @@ def iou_pairs(boxes_1, boxes_2, use_eps_clamp: bool, stream=None) -> D.DeviceArr
 
 
 # ---- A6 ----------------------------------------------------------------------------------------------
-def multibox_loss(gt_cls, gt_box, gt_mask, pred_box, pred_cls, neg_ratio: int = 3, want_neg_mask=False,
-                  want_neg_ce=False, want_grad=False, out=None, stream=None, ws_kind="loss", row_stats=None,
-                  pool=None) -> dict:
-    """models/ssd_model.py:341-396.  Returns {'result': float64[16] device block, ...}; see
-    include/ssdgeom.h for the block layout.  row_stats = (row_ml, row_negbg) from ``detect(..., want_row_stats=True)``
-    on the same pred_cls: the loss then skips its own pass over the logits (ssdg_multibox_loss_fused)."""
+def _loss_operands(gt_cls, gt_box, gt_mask, pred_box, pred_cls, want_neg_mask, want_neg_ce, want_grad, out, pool,
+                   ws_kind):
+    """The five operands as device arrays, the output dict (caller-supplied arrays, torch tensors included, are
+    used as they are; missing wanted ones are allocated) and the workspace."""
     gt_cls = D.as_device(gt_cls, np.int32)
     gt_box = D.as_device(gt_box, np.float32)
     gt_mask = D.as_device(gt_mask, np.uint8)
@@ -266,20 +265,43 @@ def multibox_loss(gt_cls, gt_box, gt_mask, pred_box, pred_cls, neg_ratio: int = 
             out["grad_box"] = D.empty((b, a, 4), np.float32)
         if "grad_cls" not in out:
             out["grad_cls"] = D.empty((b, a, c), np.float32)
-    lib = N.lib()
-    ws = (pool or POOL).get(ws_kind, lib.ssdg_loss_workspace_bytes(b, a, c))
-    args = (gt_cls.ptr, gt_box.ptr, gt_mask.ptr, pred_box.ptr, pred_cls.ptr, b, a, c,
-            int(neg_ratio), out["result"].ptr, _p(out.get("neg_mask")), _p(out.get("neg_ce")),
-            _p(out.get("grad_box")), _p(out.get("grad_cls")), ws.ptr, ws.nbytes, D.stream_handle(stream))
+    ws = pool.get(ws_kind, N.lib().ssdg_loss_workspace_bytes(b, a, c))
+    return (gt_cls, gt_box, gt_mask, pred_box, pred_cls), out, ws
+
+
+def _loss_args(x, neg_ratio, out, ws, stream) -> tuple:
+    """The arguments every loss entry point ends with (ssdg_multibox_loss's)."""
+    gt_cls, gt_box, gt_mask, pred_box, pred_cls = x
+    b, a, c = pred_cls.shape
+    return (gt_cls.ptr, gt_box.ptr, gt_mask.ptr, pred_box.ptr, pred_cls.ptr, b, a, c, int(neg_ratio),
+            out["result"].ptr, _p(out.get("neg_mask")), _p(out.get("neg_ce")), _p(out.get("grad_box")),
+            _p(out.get("grad_cls")), ws.ptr, ws.nbytes, D.stream_handle(stream))
+
+
+def multibox_loss(gt_cls, gt_box, gt_mask, pred_box, pred_cls, neg_ratio: int = 3, want_neg_mask=False,
+                  want_neg_ce=False, want_grad=False, out=None, stream=None, ws_kind="loss", row_stats=None,
+                  pool=None) -> dict:
+    """models/ssd_model.py:341-396.  Returns {'result': float64[16] device block, ...}; see
+    include/ssdgeom.h for the block layout.  row_stats = (row_ml, row_negbg) from ``detect(..., want_row_stats=True)``
+    on the same pred_cls: the loss then skips its own pass over the logits (ssdg_multibox_loss_fused)."""
+    x, out, ws = _loss_operands(gt_cls, gt_box, gt_mask, pred_box, pred_cls, want_neg_mask, want_neg_ce, want_grad,
+                                out, pool or POOL, ws_kind)
+    args = _loss_args(x, neg_ratio, out, ws, stream)
     if row_stats is None:
-        N.check(lib.ssdg_multibox_loss(*args), "multibox_loss")
+        N.check(N.lib().ssdg_multibox_loss(*args), "multibox_loss")
     else:
+        b, a, _ = x[4].shape
         row_ml, row_negbg = row_stats
         if row_ml.size != 2 * b * a or row_negbg.size != b * a:
             raise AssertionError("row statistics disagree with pred_cls in shape")
-        N.check(lib.ssdg_multibox_loss_fused(row_ml.ptr, row_negbg.ptr, *args), "multibox_loss_fused")
-    out["_keep"] = (gt_cls, gt_box, gt_mask, pred_box, pred_cls, ws)
+        N.check(N.lib().ssdg_multibox_loss_fused(row_ml.ptr, row_negbg.ptr, *args), "multibox_loss_fused")
+    out["_keep"] = (*x, ws)
     return out
+
+
+def loss_result_words(result, words: slice) -> D.DeviceArray:
+    """Device view of the words ``words`` (N.LOSS_*) of a loss result block, e.g. to sum them over the shards."""
+    return D.DeviceArray((words.stop - words.start,), np.float64, ptr=result.ptr + words.start * 8, owner=result)
 
 
 class StagedLoss:
@@ -294,55 +316,31 @@ class StagedLoss:
         total, info = sl.finish()
 
     The buffers are DeviceArrays over the workspace / result block, so a torch.distributed all_reduce on
-    torch.as_tensor(buf) works in place without a copy."""
+    torch.as_tensor(buf) works in place without a copy.  Arrays passed in ``out`` are written in place."""
 
     def __init__(self, gt_cls, gt_box, gt_mask, pred_box, pred_cls, global_priors: int, neg_ratio: int = 3,
                  want_neg_mask=False, want_neg_ce=False, want_grad=False, stream=None, ws_kind="loss_staged", out=None,
                  row_stats=None, pool=None):
-        self.gt_cls = D.as_device(gt_cls, np.int32)
-        self.gt_box = D.as_device(gt_box, np.float32)
-        self.gt_mask = D.as_device(gt_mask, np.uint8)
-        self.pred_box = D.as_device(pred_box, np.float32)
-        self.pred_cls = D.as_device(pred_cls, np.float32)
-        if len(self.pred_cls.shape) != 3:
-            raise AssertionError("pred_cls must be [B,A,C]")
-        b, a, c = self.pred_cls.shape
-        if not (self.gt_cls.size == b * a and self.gt_mask.size == b * a and self.gt_box.size == b * a * 4
-                and self.pred_box.size == b * a * 4):
-            raise AssertionError("y_true / y_pred disagree in shape")
-        self.shape = (b, a, c)
+        self.pool = pool or WorkspacePool()        # never shared: the stages keep state in the workspace
+        x, self.out, self.ws = _loss_operands(gt_cls, gt_box, gt_mask, pred_box, pred_cls, want_neg_mask,
+                                              want_neg_ce, want_grad, out, self.pool, ws_kind)
+        self.gt_cls, self.gt_box, self.gt_mask, self.pred_box, self.pred_cls = x
+        self.shape = self.pred_cls.shape
         self.global_priors = int(global_priors)
         self.row_stats = row_stats          # (row_ml, row_negbg) of detect(..., want_row_stats=True), or None
         self.neg_ratio = int(neg_ratio)
         self.stream = stream
-        self.out = dict(out or {})
-        if "result" not in self.out:
-            self.out["result"] = D.empty((N.LOSS_RESULT_LEN,), np.float64)
         self._xb = {}
-        if want_neg_mask:
-            self.out["neg_mask"] = D.empty((b, a), np.uint8)
-        if want_neg_ce:
-            self.out["neg_ce"] = D.empty((b, a), np.float32)
-        if want_grad:
-            self.out["grad_box"] = D.empty((b, a, 4), np.float32)
-            self.out["grad_cls"] = D.empty((b, a, c), np.float32)
-        lib = N.lib()
-        self.pool = pool or WorkspacePool()        # never shared: the stages keep state in the workspace
-        self.ws = self.pool.get(ws_kind, lib.ssdg_loss_workspace_bytes(b, a, c))
         self.n_stages = 5 if want_grad else 4
 
     def run(self, stage: int):
-        b, a, c = self.shape
-        o = self.out
-        N.check(N.lib().ssdg_multibox_loss_stage(
-            int(stage), self.global_priors, _p(self.row_stats[0] if self.row_stats else None),
-            _p(self.row_stats[1] if self.row_stats else None), self.gt_cls.ptr, self.gt_box.ptr, self.gt_mask.ptr, self.pred_box.ptr,
-            self.pred_cls.ptr, b, a, c, self.neg_ratio, o["result"].ptr, _p(o.get("neg_mask")), _p(o.get("neg_ce")),
-            _p(o.get("grad_box")), _p(o.get("grad_cls")), self.ws.ptr, self.ws.nbytes,
-            D.stream_handle(self.stream)), "multibox_loss_stage")
+        rs = self.row_stats or (None, None)
+        x = (self.gt_cls, self.gt_box, self.gt_mask, self.pred_box, self.pred_cls)
+        N.check(N.lib().ssdg_multibox_loss_stage(int(stage), self.global_priors, _p(rs[0]), _p(rs[1]),
+                                                 *_loss_args(x, self.neg_ratio, self.out, self.ws, self.stream)),
+                "multibox_loss_stage")
 
     def _xbuf(self, which: int, dtype):
-        import ctypes as C
         ptr, cnt = C.c_void_p(), C.c_int64()
         N.check(N.lib().ssdg_loss_exchange(self.ws.ptr, which, C.byref(ptr), C.byref(cnt)), "loss_exchange")
         return D.DeviceArray((int(cnt.value),), dtype, ptr=ptr.value, owner=self.ws)
@@ -361,41 +359,42 @@ class StagedLoss:
         if stage == 4:
             return []
         r = self.out["result"]
-        # the separable sums [8..10], the shard's own positives [11], its data-dependent error count [12] and its
-        # mined negatives [5]
-        return [D.DeviceArray((5,), np.float64, ptr=r.ptr + 8 * 8, owner=r),
-                D.DeviceArray((1,), np.float64, ptr=r.ptr + 5 * 8, owner=r)]
+        # the separable sums, the shard's own positives, its data-dependent error count and its mined negatives
+        return [loss_result_words(r, slice(N.LOSS_SUM_POS_CE, N.LOSS_ERRORS + 1)),
+                loss_result_words(r, slice(N.LOSS_NUM_NEG, N.LOSS_NUM_NEG + 1))]
 
     def finish(self) -> tuple:
         """After the stage-3 exchange: (total, info) of the whole batch, identical on every shard."""
         r = self.out["result"].to_host(self.stream)
-        status = int(r[7])
-        if status == N.ERR_NO_POSITIVE:
-            raise IndexError("no positive prior in the batch: hard-negative top-k is empty (models/ssd_model.py:369)")
-        if status == N.ERR_TOPK_RANGE:
-            raise ValueError("3*num_pos exceeds the number of priors in the batch (tf.math.top_k, models/ssd_model.py:368)")
-        N.check(status, "multibox_loss_stage")
-        if r[12] != 0:      # some shard mined a positive (models/ssd_model.py:375) or saw a class id out of range
+        d = decode_loss_result(r, "multibox_loss_stage")
+        # some shard mined a positive (models/ssd_model.py:375) or saw a class id out of range
+        if r[N.LOSS_ERRORS] != 0:
             raise AssertionError("a shard of the batch reported %d positives mined as negatives / class ids out of "
-                                 "range" % int(r[12]))
-        s_pos, s_neg, s_l1, n_pos, n_neg = r[8], r[9], r[10], r[11], r[5]
-        l_pos, l_neg, l_loc = s_pos / n_pos, s_neg / n_neg, s_l1 / n_pos
-        return (l_loc + l_pos) + l_neg, {"cls loss pos": l_pos, "cls loss neg": l_neg, "loc loss": l_loc,
-                                          "num_pos": int(n_pos), "num_neg": int(n_neg), "kth": r[6]}
+                                 "range" % int(r[N.LOSS_ERRORS]))
+        n_pos = r[N.LOSS_OWN_POS]      # summed over the shards: the positives of the batch
+        total, info = loss_from_sums(d["sum_pos_ce"], d["sum_neg_ce"], d["sum_l1"], n_pos, r[N.LOSS_NUM_NEG])
+        info.update(num_pos=int(n_pos), num_neg=d["num_neg"], kth=d["kth"])
+        return total, info
 
 
-def loss_result_to_host(result: D.DeviceArray, stream=None) -> dict:
-    """One synchronising read of the result block; raises like the reference on the device-side
-    guards (num_pos == 0 -> IndexError at models/ssd_model.py:369; k out of range -> top_k error)."""
-    r = result.to_host(stream)
-    status = int(r[7])
+def decode_loss_result(r, what: str = "multibox_loss") -> dict:
+    """A loss result block on the host as a dict; raises like the reference on the device-side guards
+    (num_pos == 0 -> IndexError at models/ssd_model.py:369; k out of range -> top_k error)."""
+    status = int(r[N.LOSS_STATUS])
     if status == N.ERR_NO_POSITIVE:
         raise IndexError("no positive prior in the batch: hard-negative top-k is empty (models/ssd_model.py:369)")
     if status == N.ERR_TOPK_RANGE:
         raise ValueError("3*num_pos exceeds the number of priors in the batch (tf.math.top_k, models/ssd_model.py:368)")
-    N.check(status, "multibox_loss")
-    return {"total": r[0], "cls loss pos": r[1], "cls loss neg": r[2], "loc loss": r[3], "num_pos": int(r[4]),
-            "num_neg": int(r[5]), "kth": r[6], "sum_pos_ce": r[8], "sum_neg_ce": r[9], "sum_l1": r[10]}
+    N.check(status, what)
+    return {"total": r[N.LOSS_TOTAL], "cls loss pos": r[N.LOSS_POS], "cls loss neg": r[N.LOSS_NEG],
+            "loc loss": r[N.LOSS_LOC], "num_pos": int(r[N.LOSS_NUM_POS]), "num_neg": int(r[N.LOSS_NUM_NEG]),
+            "kth": r[N.LOSS_KTH], "sum_pos_ce": r[N.LOSS_SUM_POS_CE], "sum_neg_ce": r[N.LOSS_SUM_NEG_CE],
+            "sum_l1": r[N.LOSS_SUM_L1]}
+
+
+def loss_result_to_host(result: D.DeviceArray, stream=None) -> dict:
+    """One synchronising read of the result block, decoded by ``decode_loss_result``."""
+    return decode_loss_result(result.to_host(stream))
 
 
 # ---- A7 + A8 + A9 ---------------------------------------------------------------------------------------

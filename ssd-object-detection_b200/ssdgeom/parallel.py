@@ -19,7 +19,9 @@ from __future__ import annotations
 
 import numpy as np
 
-SUM_SLICE = slice(4, 11)   # result-block entries that are additive across shards: see include/ssdgeom.h
+from . import _native as N
+
+SUM_SLICE = N.LOSS_ADDITIVE   # result-block words that are additive across shards: see include/ssdgeom.h
 
 
 def shard_range(n_items: int, world: int, rank: int):
@@ -46,20 +48,24 @@ def loss_from_sums(sum_pos_ce, sum_neg_ce, sum_l1, num_pos, num_neg):
     return (info["loc loss"] + info["cls loss pos"]) + info["cls loss neg"], info
 
 
+def _loss_of(s):
+    return loss_from_sums(s["sum_pos_ce"], s["sum_neg_ce"], s["sum_l1"], s["num_pos"], s["num_neg"])
+
+
 def block_sums(result_block):
-    """The additive entries of a loss result block (host array): order num_pos, num_neg, kth, status,
-    sum_pos_ce, sum_neg_ce, sum_l1 -> dict."""
+    """The additive entries of a loss result block (host array) -> dict."""
     r = np.asarray(result_block, dtype=np.float64)
-    return {"num_pos": r[4], "num_neg": r[5], "sum_pos_ce": r[8], "sum_neg_ce": r[9], "sum_l1": r[10]}
+    return {"num_pos": r[N.LOSS_NUM_POS], "num_neg": r[N.LOSS_NUM_NEG], "sum_pos_ce": r[N.LOSS_SUM_POS_CE],
+            "sum_neg_ce": r[N.LOSS_SUM_NEG_CE], "sum_l1": r[N.LOSS_SUM_L1]}
 
 
 def combine_loss(shard_sums, mode="pooled"):
     """Combine per-shard additive sums (list of dicts as from ``block_sums``)."""
     if mode == "pooled":
         tot = {k: float(sum(s[k] for s in shard_sums)) for k in ("num_pos", "num_neg", "sum_pos_ce", "sum_neg_ce", "sum_l1")}
-        return loss_from_sums(tot["sum_pos_ce"], tot["sum_neg_ce"], tot["sum_l1"], tot["num_pos"], tot["num_neg"])
+        return _loss_of(tot)
     if mode == "mean_of_shards":
-        parts = [loss_from_sums(s["sum_pos_ce"], s["sum_neg_ce"], s["sum_l1"], s["num_pos"], s["num_neg"]) for s in shard_sums]
+        parts = [_loss_of(s) for s in shard_sums]
         n = len(parts)
         info = {k: sum(p[1][k] for p in parts) / n for k in parts[0][1]}
         return sum(p[0] for p in parts) / n, info
@@ -77,17 +83,15 @@ def allreduce_sums(vec, group=None):
 def distributed_loss(result_block_tensor, group=None, mode="pooled"):
     """result_block_tensor: torch float64[16] view of one rank's loss result block (include/ssdgeom.h).
     Returns (total, info) identical on every rank."""
-    import torch
     import torch.distributed as dist
     r = result_block_tensor
     world = dist.get_world_size(group) if (dist.is_available() and dist.is_initialized()) else 1
     if mode == "pooled":
-        vec = r[SUM_SLICE].clone()
-        allreduce_sums(vec, group)
-        v = vec.double().cpu().numpy()
-        return loss_from_sums(v[4], v[5], v[6], v[0], v[1])
+        v = np.zeros(N.LOSS_RESULT_LEN)
+        v[SUM_SLICE] = allreduce_sums(r[SUM_SLICE].clone(), group).double().cpu().numpy()
+        return _loss_of(block_sums(v))
     if mode == "mean_of_shards":
-        vec = torch.stack([r[0], r[1], r[2], r[3]]).clone()
+        vec = r[N.LOSS_TOTAL:N.LOSS_LOC + 1].clone()
         allreduce_sums(vec, group)
         v = (vec.double().cpu().numpy()) / world
         return float(v[0]), {"cls loss pos": float(v[1]), "cls loss neg": float(v[2]), "loc loss": float(v[3])}

@@ -112,8 +112,7 @@ class HotPath:
         self.loss_exchange = None                        # a caller's own exchange (depth 1 only)
         if comm is not None and mining == "shard" and comm.world > 1:
             for sl in self._slots:
-                r = sl["loss"]["result"]
-                sums = D.DeviceArray((7,), np.float64, ptr=r.ptr + 4 * 8, owner=r)    # result[4..10], include/ssdgeom.h
+                sums = ops.loss_result_words(sl["loss"]["result"], N.LOSS_ADDITIVE)
                 sl["loss_exchange"] = (lambda stream, sums=sums: comm.allreduce(sums, stream))
         self.staged = None
         if mining == "global":
@@ -175,27 +174,22 @@ class HotPath:
                                            self.thresh, want=(), out=self.tgt, stream=stream, pool=self.pool)
 
     def loss_stage(self, stream, stats=False):
-        if stats and self.staged is None:
+        row_stats = (self.det_stats["row_ml"], self.det_stats["row_negbg"]) if stats else None
+        if self.staged is None:
             ops.multibox_loss(self.tgt["cls"], self.tgt["loc"], self.tgt["mask"], self.pred_box, self.pred_cls,
-                              self.neg_ratio, out=self.loss, stream=stream, pool=self.pool,
-                              row_stats=(self.det_stats["row_ml"], self.det_stats["row_negbg"]))
+                              self.neg_ratio, out=self.loss, stream=stream, pool=self.pool, row_stats=row_stats)
             return
-        if self.staged is not None:
-            self.staged.stream = stream
-            self.staged.row_stats = (self.det_stats["row_ml"], self.det_stats["row_negbg"]) if stats else None
-            for stage in range(self.staged.n_stages):
-                self.staged.run(stage)
-                bufs = self.staged.exchange(stage)
-                if not bufs:
-                    continue
-                if self.comm is not None:
-                    self.comm.allreduce_multi(bufs, stream)       # one NCCL group per stage
-                else:
-                    for buf in bufs:
-                        self.allreduce(buf, stream)
-            return
-        ops.multibox_loss(self.tgt["cls"], self.tgt["loc"], self.tgt["mask"], self.pred_box, self.pred_cls,
-                          self.neg_ratio, out=self.loss, stream=stream, pool=self.pool)
+        self.staged.stream, self.staged.row_stats = stream, row_stats
+        for stage in range(self.staged.n_stages):
+            self.staged.run(stage)
+            bufs = self.staged.exchange(stage)
+            if not bufs:
+                continue
+            if self.comm is not None:
+                self.comm.allreduce_multi(bufs, stream)       # one NCCL group per stage
+            else:
+                for buf in bufs:
+                    self.allreduce(buf, stream)
 
     def detect_stage(self, stream, stage=None, stats=False, part=None):
         out = dict(self.det, **self.det_stats) if stats else self.det

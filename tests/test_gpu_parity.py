@@ -474,6 +474,27 @@ def test_loss_cross_shard_global_mining(shards, priors300):
     assert not np.array_equal(local, want_mask[spans[0][0]:spans[0][1]])
 
 
+def test_staged_loss_writes_caller_outputs(priors300):
+    """Arrays passed in ``out`` receive the staged loss's mask and gradient, as they do for multibox_loss."""
+    batch = 2
+    boxes, cls, off = synth.make_gt(33, batch, 100, "coco")
+    y_true = _targets(boxes, cls, off, priors300, batch)
+    pred_cls, pred_box = synth.make_predictions(33, batch, 8732)
+    full = ops.multibox_loss(*y_true, pred_box, pred_cls, want_neg_mask=True, want_grad=True)
+    mine = {"neg_mask": D.empty((batch, 8732), np.uint8), "grad_box": D.empty(pred_box.shape, np.float32),
+            "grad_cls": D.empty(pred_cls.shape, np.float32)}
+    for v in mine.values():
+        v.zero_()
+    sl = ops.StagedLoss(*y_true, pred_box, pred_cls, global_priors=batch * 8732, want_neg_mask=True, want_grad=True,
+                        out=mine)
+    for stage in range(sl.n_stages):       # one shard: the exchanges have nothing to sum
+        sl.run(stage)
+    assert sl.finish()[1]["num_neg"] == ops.loss_result_to_host(full["result"])["num_neg"]
+    for k, v in mine.items():
+        assert sl.out[k] is v
+        assert np.array_equal(v.to_host(), full[k].to_host()), k
+
+
 # ---- A7 / A8 / A9 -----------------------------------------------------------------------------------------
 def _check_detect(pred_cls, pred_box, priors, **kw):
     kept, count, aux = M.detect(pred_cls, pred_box, priors, return_aux=True, **kw)
