@@ -22,7 +22,6 @@
 //                  iterating "kept(i) <=> no kept j < i suppresses i" to its fixed point.
 #include <math_constants.h>
 #include <algorithm>
-#include <cstdlib>
 #include <type_traits>
 #include "common.cuh"
 
@@ -32,15 +31,15 @@ namespace ssdg {
 // than 64 registers per thread, which leaves a third of the register file to the matcher's search CTAs that run
 // beside the pass.  Measured (B200, SSD300 B=256): 16 warps 0.163 ms, 20 warps 0.152 ms (0.83 of the copy peak) and
 // the chained step 0.520 -> 0.513 ms; without the register cap (96 registers) the pass is as fast but the step is not.
-#ifndef SSDG_FILTER_THREADS
-#define SSDG_FILTER_THREADS 640
-#endif
-#ifndef SSDG_FILTER_MAXNREG
-#define SSDG_FILTER_MAXNREG 64
-#endif
-#define SSDG_FILTER_BOUNDS __maxnreg__(SSDG_FILTER_MAXNREG)
-constexpr int kFThreads = SSDG_FILTER_THREADS;
+constexpr int kFThreads = 640;
+constexpr int kFilterMaxRegs = 64;
 constexpr int kFWarps = kFThreads / 32;
+// L2 prefetch distance of a filter warp, in tiles.  Measured (B200, SSD300 B=256, filter pass / chained step):
+// none 0.1603 / 0.5455 ms, 1 tile 0.1542 / 0.5451 ms (0.82 of the copy peak), 2 tiles 0.1614 / 0.5492 ms,
+// 3 tiles 0.1828 / 0.5598 ms; the pass gets slower with every tile beyond the first.
+constexpr int kFilterPrefetch = 1;
+// Classes between two updates of the filter's pre-filter bound.
+constexpr int kFilterPreStep = 16;
 constexpr int kNmsThreads = 128;
 constexpr int kNmsWarps = kNmsThreads / 32;
 constexpr int kSlabs = 32;   // slabs per axis of the NMS candidate join
@@ -200,10 +199,7 @@ __device__ __forceinline__ void filter_tile(const DetectParams& P, int b, int j,
           if (two_pass) row[C - 1] = eb;
           s0 = eb;
         }
-#ifndef SSDG_FILTER_PRE_STEP
-#define SSDG_FILTER_PRE_STEP 16
-#endif
-        constexpr int kPs = SSDG_FILTER_PRE_STEP;   // classes between two updates of the bound
+        constexpr int kPs = kFilterPreStep;
         auto word32 = [&](int c0) {
           u32 bits = 0u;
 #pragma unroll
@@ -367,7 +363,7 @@ __device__ __forceinline__ void prefetch_l2_bulk(const void* gsrc, u32 bytes) {
 }
 
 template <typename TP, bool kProbs, bool kWrite>
-__global__ void SSDG_FILTER_BOUNDS filter_kernel(DetectParams P, int warps_per_cta, int prefetch) {   // <= 64 registers: leaves room for a matcher CTA
+__global__ void __maxnreg__(kFilterMaxRegs) filter_kernel(DetectParams P, int warps_per_cta, int prefetch) {   // <= 64 registers: leaves room for a matcher CTA
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int C = P.C, A = P.A, tpi = P.tpi, nfg = P.C - 1;
   const size_t tile_floats = (size_t)32 * C;
@@ -1068,8 +1064,7 @@ static int run_filter(DetectParams& P, int prior_dtype, cudaStream_t st) {
   const bool wr = !kProbs && (P.probs || P.head_score || P.head_cls || P.head_mask);
   auto go = [&](auto kern) -> int {
     SSDG_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
-    static const char* env_pf = getenv("SSDG_FILTER_PREFETCH");   // tiles of L2 prefetch distance per warp; experiment knob
-    kern<<<g.grid, kFThreads, g.smem, st>>>(P, g.warps, env_pf ? atoi(env_pf) : 1);
+    kern<<<g.grid, kFThreads, g.smem, st>>>(P, g.warps, kFilterPrefetch);
     return SSDG_OK;
   };
   int rc;

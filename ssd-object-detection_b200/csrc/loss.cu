@@ -13,7 +13,6 @@
 //   grad_kernel    optional second pass: d total / d logits and d total / d pred_box (:248).
 #include <math_constants.h>
 #include <cstddef>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace ssdg {
@@ -591,11 +590,13 @@ __global__ void __launch_bounds__(kGradThreads) grad_kernel(LossParams P) {
   }
 }
 
+// Shared memory for the tile rings of a ce_kernel CTA: all kCeWarps warps up to C = 100, fewer beyond.  The warp count
+// decides how tiles map to CTAs, and so how the per-CTA partial sums are grouped: changing it changes the loss bits.
+constexpr size_t kCeSmemBudget = 200 * 1024;
+
 static int ce_warps_for(int C) {
-  static const char* env = getenv("SSDG_CE_SMEM_KB");   // experiment knob
-  const size_t budget = (env ? (size_t)atoi(env) : 200) * 1024;
   size_t per_warp = (size_t)kStages * 32 * C * 4;
-  int w = (int)(budget / per_warp);
+  int w = (int)(kCeSmemBudget / per_warp);
   if (w > kCeWarps) w = kCeWarps;
   return w;
 }

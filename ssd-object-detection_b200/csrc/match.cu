@@ -32,19 +32,12 @@
 #include <unordered_map>
 #include <utility>
 #include <vector>
-#include <cstdlib>
 #include "common.cuh"
 
 namespace ssdg {
 
-#ifndef SSDG_MATCH_THREADS
-#define SSDG_MATCH_THREADS 512
-#endif
-#ifndef SSDG_MATCH_CTAS_PER_SM
-#define SSDG_MATCH_CTAS_PER_SM 2
-#endif
-constexpr int kMatchThreads = SSDG_MATCH_THREADS;
-constexpr int kMatchCtasPerSm = SSDG_MATCH_CTAS_PER_SM;
+constexpr int kMatchThreads = 512;
+constexpr int kMatchCtasPerSm = 2;
 constexpr int kMatchMaxCtas = 1024;
 constexpr int kCandCap = 8192;          // listed (row, prior) pairs above the threshold per image
 constexpr int kABits = 21;
@@ -293,14 +286,12 @@ static size_t match_smem_bytes(int tm, int ntiles_s, int bit_words) {
 // image's list.  The per-image kernel below consumes both.
 constexpr int kSearchThreads = 128;
 constexpr int kSearchWarps = kSearchThreads / 32;
+// 10 CTAs per SM (48 registers): four instead of three of them fit beside a filter CTA of the other branch
+// (chained step 0.513 -> 0.508 ms; alone 0.141 -> 0.139 ms).  Both the launch bounds and the grid use it.
+constexpr int kSearchCtasPerSm = 10;
 
 template <typename TG, typename TP, bool kHier>   // kHier: two-level bound (super-tiles of kSuper tiles, then tiles); up to kTileSmemMax tiles
-// 10 CTAs per SM (48 registers): four instead of three of them fit beside a filter CTA of the other branch
-// (chained step 0.513 -> 0.508 ms; alone 0.141 -> 0.139 ms).
-#ifndef SSDG_SEARCH_MINB
-#define SSDG_SEARCH_MINB 10
-#endif
-__global__ void __launch_bounds__(kSearchThreads, SSDG_SEARCH_MINB) search_kernel(MatchParams P) {
+__global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kernel(MatchParams P) {
   typedef typename Promote<TG, TP>::type R;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31;
@@ -943,16 +934,11 @@ static int launch_match(const MatchParams& P, int grid, size_t smem, cudaStream_
   SSDG_CUDA_TRY(cudaFuncSetAttribute(match_kernel<TG, TP>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
   prof_begin(SSDG_PROF_MATCH, st);
   {
-#ifdef SSDG_SEARCH_FLAT
-    const bool hier = false;
-#else
     const bool hier = P.ntiles <= kTileSmemMax;
-#endif
     const size_t ssm = 0;
     auto skern = hier ? search_kernel<TG, TP, true> : search_kernel<TG, TP, false>;
     SSDG_CUDA_TRY(cudaFuncSetAttribute(skern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-    static const char* env = getenv("SSDG_SEARCH_CTAS_PER_SM");   // experiment knob
-    long long sgrid = (long long)sm_count() * (env ? atoi(env) : SSDG_SEARCH_MINB);
+    long long sgrid = (long long)sm_count() * kSearchCtasPerSm;
     const long long want = ((long long)P.B * (P.max_gt > 0 ? P.max_gt : 1) + kSearchWarps - 1) / kSearchWarps;
     if (want < sgrid) sgrid = want;
     prof_begin(SSDG_PROF_SEARCH, st);

@@ -14,14 +14,14 @@ class Stream:
     """Owning CUDA stream (non-blocking)."""
 
     def __init__(self, priority=None):
-        """priority: None (default), "high" / "low" (the device's extreme stream priorities), or an int k >= 1:
-        k-1 levels below the highest."""
+        """priority: None (default), or "high" / "low" (the device's extreme stream priorities)."""
+        if priority not in (None, "high", "low"):
+            raise ValueError("stream priority must be None, 'high' or 'low', not %r" % (priority,))
         h = C.c_void_p()
         if priority is None:
             N.check(N.lib().ssdg_stream_create(C.byref(h)), "stream_create")
         else:
-            level = {"high": 1, "low": 0}.get(priority, priority)
-            N.check(N.lib().ssdg_stream_create_priority(C.byref(h), int(level)), "stream_create")
+            N.check(N.lib().ssdg_stream_create_priority(C.byref(h), 1 if priority == "high" else 0), "stream_create")
         self.handle = h.value
 
     def sync(self):

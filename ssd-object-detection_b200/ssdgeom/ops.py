@@ -400,10 +400,9 @@ def loss_result_to_host(result: D.DeviceArray, stream=None) -> dict:
 # ---- A7 + A8 + A9 ---------------------------------------------------------------------------------------
 def detect(pred_cls, pred_box, priors, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores=False,
            want_boxes=False, want_probs=False, head_thresh=None, out=None, stream=None, stage=None,
-           want_row_stats=False, ws_key="detect", pool=None) -> dict:
+           want_row_stats=False, pool=None) -> dict:
     """stage: None = the whole post-processing; 0 = filter + decode + candidate lists only; 1 = the NMS of a previous
-    stage-0 call with the same arguments (include/ssdgeom.h, ssdg_detect_stage).  ws_key names the pooled
-    workspace: calls that overlap on different streams need different keys."""
+    stage-0 call with the same arguments (include/ssdgeom.h, ssdg_detect_stage)."""
     pred_cls = D.as_device(pred_cls, np.float32)
     pred_box = D.as_device(pred_box, np.float32)
     priors = D.as_device(priors)
@@ -432,7 +431,7 @@ def detect(pred_cls, pred_box, priors, score_thresh=0.01, top_k=200, iou_thresh=
         need("head_cls", (b, a), np.int32)
         need("head_mask", (b, a), np.uint8)
     lib = N.lib()
-    ws = (pool or POOL).get(ws_key, lib.ssdg_detect_workspace_bytes(b, a, c, top_k))
+    ws = (pool or POOL).get("detect", lib.ssdg_detect_workspace_bytes(b, a, c, top_k))
     args = (pred_cls.ptr, pred_box.ptr, priors.ptr, _code(priors.dtype), b, a, c, float(score_thresh),
             int(top_k), float(iou_thresh), out["kept"].ptr, out["count"].ptr, _p(out.get("kept_score")),
             _p(out.get("boxes")), _p(out.get("probs")),

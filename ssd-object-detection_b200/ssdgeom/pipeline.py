@@ -4,8 +4,6 @@ batch.  The two branches only share the predictions, so they run on separate str
 matcher is latency-bound and the loss/filter passes are HBM-bound, so they overlap."""
 from __future__ import annotations
 
-import os
-
 import numpy as np
 
 from . import _native as N
@@ -73,31 +71,20 @@ class HotPath:
         # occupy every SM ahead of everything else) at low.  With the matcher at low priority a step of 128 images per
         # GPU -- where the assignment chain is the longer one -- took 0.370 instead of 0.347 ms; at 256 images there is
         # no difference (profiles/r15_stream_priorities.txt).
-        import os
-
-        def prio(name, default):          # SSDGEOM_PRIO_A / _D / _N / _L: "high", "low" or levels below the highest (measurements)
-            v = os.environ.get("SSDGEOM_PRIO_" + name, default)
-            return int(v) if v.lstrip("-").isdigit() else v
-        self.s_main, self.s_a, self.s_d = D.Stream(), D.Stream(prio("A", "high")), D.Stream(prio("D", "high"))
-        self.s_n, self.s_l = D.Stream(prio("N", "low")), D.Stream(prio("L", "high"))
+        self.s_main, self.s_a, self.s_d = D.Stream(), D.Stream("high"), D.Stream("high")
+        self.s_n, self.s_l = D.Stream("low"), D.Stream("high")
         self.s_x = D.Stream("high")                      # loss exchange (data parallel)
         self.ev_begin, self.ev_mid, self.ev_m = (D.Event() for _ in range(3))
         self.split = True
-        # the post-processing chain can run in `detect_parts` slices of the batch: the NMS of a slice then overlaps
-        # the filter pass of the next one (kernels bound by different resources) instead of waiting for the whole
-        # batch.  SSDGEOM_DETECT_PARTS overrides for measurements.
-        self.detect_parts = max(1, min(int(os.environ.get("SSDGEOM_DETECT_PARTS", "1")), self.batch))
         # Who takes the SMs first.  Both branches become ready at the same moment (ev_begin); the filter's 148 CTAs of
         # 171 KB shared memory and the search's 1184 small CTAs then compete for every SM.  Below ~240 images per GPU the
         # assignment chain (search -> per-image matching -> loss, all latency-bound) is the longer one, and the step is
         # shorter when the search gets its CTAs placed first and the filter's fill in as they drain: a small zeroing
         # node in front of the filter pass (a few microseconds) decides that race (128 images: 0.34 -> 0.31 ms per
         # step; 256 images: 0.530 -> 0.539, so not there).  Ordering the filter behind the search with an event costs
-        # the kernel boundary and is slower than either (0.35 ms).  SSDGEOM_LEAD_ASSIGN=0/1 overrides.
-        la = os.environ.get("SSDGEOM_LEAD_ASSIGN")
-        self.lead_assign = (la == "1") if la in ("0", "1") else self.batch < 240
+        # the kernel boundary and is slower than either (0.35 ms).
+        self.lead_assign = self.batch < 240
         self._lead_pad = D.empty((64 * 1024,), np.uint8)
-        self.ev_parts = [D.Event() for _ in range(self.detect_parts)]
         # one pass over the logits serves both branches: the filter leaves per-prior softmax statistics and the
         # loss gathers from them instead of streaming the 724 MB again (only in the chained step)
         self.fused = True
@@ -120,8 +107,8 @@ class HotPath:
                 raise ValueError("global mining needs comm / allreduce and global_priors")
             self.staged = ops.StagedLoss(self.tgt["cls"], self.tgt["loc"], self.tgt["mask"], self.pred_box, self.pred_cls,
                                          int(global_priors), self.neg_ratio, out=self.loss)
-        # search, match | lossprep (or ce), select x2, final | filter, nms per slice of the post-processing
-        self.kernel_launches_per_step = 6 + 2 * self.detect_parts + (1 if evaluator is not None else 0)
+        # search, match | lossprep (or ce), select x2, final | filter, nms
+        self.kernel_launches_per_step = 8 + (1 if evaluator is not None else 0)
         # matcher head + loss histograms (cudaMemsetAsync), + the lead node of small batches
         self.memsets_per_step = 2 + (1 if self.lead_assign else 0)
         self.h2d_bytes = sum(self._sets[0][k].nbytes for k in INPUT_NAMES)
@@ -191,23 +178,10 @@ class HotPath:
                 for buf in bufs:
                     self.allreduce(buf, stream)
 
-    def detect_stage(self, stream, stage=None, stats=False, part=None):
+    def detect_stage(self, stream, stage=None, stats=False):
         out = dict(self.det, **self.det_stats) if stats else self.det
-        if part is None:
-            ops.detect(self.pred_cls, self.pred_box, self.priors, self.score_thresh, self.top_k, self.iou_thresh,
-                       out=out, stream=stream, stage=stage, want_row_stats=stats, pool=self.pool)
-            return
-        # images [lo, hi) of the batch, with a workspace of their own
-        lo = self.batch * part // self.detect_parts
-        hi = self.batch * (part + 1) // self.detect_parts
-
-        def rows(x):
-            per = x.nbytes // self.batch
-            return D.DeviceArray((hi - lo,) + x.shape[1:], x.dtype, ptr=x.ptr + lo * per, owner=x)
-
-        ops.detect(rows(self.pred_cls), rows(self.pred_box), self.priors, self.score_thresh, self.top_k,
-                   self.iou_thresh, out={k: rows(v) for k, v in out.items()}, stream=stream, stage=stage,
-                   want_row_stats=stats, ws_key="detect%d" % part, pool=self.pool)
+        ops.detect(self.pred_cls, self.pred_box, self.priors, self.score_thresh, self.top_k, self.iou_thresh,
+                   out=out, stream=stream, stage=stage, want_row_stats=stats, pool=self.pool)
 
     def evaluate_stage(self, stream, image_base=None):
         self.evaluator.add(self.det, self.gt_boxes, self.gt_cls, self.gt_off, image_base, stream, max_gt=self.max_gt)
@@ -238,19 +212,14 @@ class HotPath:
         loss_exchange = self._cur["loss_exchange"] or self.loss_exchange
         fused = self.fused
         if self.split:
-            parts = self.detect_parts
             if self.lead_assign:
                 self._lead_pad.zero_(self.s_d)
-            for part in range(parts):
-                self.detect_stage(self.s_d, stage=0, stats=fused, part=part if parts > 1 else None)
-                self.ev_parts[part].record(self.s_d)
-                if part == 0:
-                    self.assign(self.s_a)
-                    self.ev_m.record(self.s_a)
+            self.detect_stage(self.s_d, stage=0, stats=fused)
+            self.assign(self.s_a)
+            self.ev_m.record(self.s_a)
             self.ev_mid.record(self.s_d)
-            for part in range(parts):
-                D.stream_wait_event(self.s_n, self.ev_parts[part])
-                self.detect_stage(self.s_n, stage=1, stats=fused, part=part if parts > 1 else None)
+            D.stream_wait_event(self.s_n, self.ev_mid)
+            self.detect_stage(self.s_n, stage=1, stats=fused)
             if self.evaluator is not None:      # before ev_d: the waits on ev_d cover its reads of GT and lists
                 self.evaluate_stage(self.s_n, image_base)
             D.stream_wait_event(self.s_l, self.ev_m)

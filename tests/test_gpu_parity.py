@@ -46,6 +46,20 @@ def priors512():
     return O.build_prior_box(t["sizes"], t["s_k_refer"], t["aspect_ratio"], t["input_size"])
 
 
+@pytest.fixture(scope="module")
+def priors_large():
+    """SSD512's table with a 96 x 96 first feature map: 45 044 priors, 1 408 tiles of 32."""
+    t = synth.SSD512
+    return O.build_prior_box([(96, 96)] + t["sizes"][1:], t["s_k_refer"], t["aspect_ratio"], t["input_size"])
+
+
+def _check_large_prior_path(priors, out):
+    # more than kTileSmemMax (csrc/match.cu) tiles of 32 priors: the single-level row search, and match_kernel
+    # reads the tile statistics from global memory
+    assert priors.shape[0] > 32 * 1024
+    assert ops.match_status(out) & 4 == 0     # every pair fit the pair list: no exhaustive rescan
+
+
 # ---- A1 ----------------------------------------------------------------------------------------------
 def test_priors_ssd300_bit_exact(golden_dir, priors300):
     got = M.build_prior_box(synth.SSD300["sizes"])
@@ -203,12 +217,14 @@ def test_assign_config1_golden(golden_dir, priors300):
 
 @pytest.mark.parametrize("table,batch,max_t,mode,seed", [
     ("ssd300", 16, 100, "max", 3), ("ssd300", 32, 100, "coco", 4), ("ssd300", 8, 37, "max", 5),
-    ("ssd512", 4, 100, "max", 6), ("ssd512", 2, 500, "max", 7)])
-def test_assign_random_bit_exact(table, batch, max_t, mode, seed, priors300, priors512):
-    priors = priors300 if table == "ssd300" else priors512
+    ("ssd512", 4, 100, "max", 6), ("ssd512", 2, 500, "max", 7), ("large", 3, 100, "max", 8)])
+def test_assign_random_bit_exact(table, batch, max_t, mode, seed, priors300, priors512, priors_large):
+    priors = {"ssd300": priors300, "ssd512": priors512, "large": priors_large}[table]
     boxes, cls, off = synth.make_gt(seed, batch, max_t, mode)
     o_cls, o_loc, o_mask = bbox.match_encode_batch(boxes, cls, off, priors, 0.5)
     out = ops.match_encode(boxes, cls, off, priors, batch, int(np.diff(off).max()), 0.5, want=("box", "match"))
+    if table == "large":
+        _check_large_prior_path(priors, out)
     o_box, o_match = out["box"].to_host(), out["match"].to_host()
     for i in range(batch):
         s, e = off[i], off[i + 1]
@@ -224,18 +240,23 @@ def test_assign_random_bit_exact(table, batch, max_t, mode, seed, priors300, pri
 
 
 @pytest.mark.parametrize("table,batch,max_t,mode", [("ssd300", 12, 100, "max"), ("ssd300", 16, 100, "coco"),
-                                                   ("ssd512", 3, 100, "max"), ("ssd512", 2, 500, "max")])
-def test_assign_with_prior_index(table, batch, max_t, mode, priors300, priors512):
+                                                   ("ssd512", 3, 100, "max"), ("ssd512", 2, 500, "max"),
+                                                   ("large", 3, 100, "max")])
+def test_assign_with_prior_index(table, batch, max_t, mode, priors300, priors512, priors_large):
     """The shape-sorted prior index is an acceleration structure only: identical outputs with and
     without it, and equal to the oracle."""
-    priors = priors300 if table == "ssd300" else priors512
+    priors = {"ssd300": priors300, "ssd512": priors512, "large": priors_large}[table]
     boxes, cls, off = synth.make_gt(41, batch, max_t, mode)
     want = ("cls", "box", "loc", "mask", "match")
     plain = ops.match_encode(boxes, cls, off, priors, batch, int(np.diff(off).max()), 0.5, want=want)
+    if table == "large":
+        _check_large_prior_path(priors, plain)
     d_pri = D.to_device(priors)
     idx = ops.prior_index(d_pri)
     assert ops.prior_index(d_pri) is idx                      # cached on the array
     fast = ops.match_encode(boxes, cls, off, d_pri, batch, int(np.diff(off).max()), 0.5, want=want)
+    if table == "large":
+        _check_large_prior_path(priors, fast)
     for k in want:
         assert np.array_equal(plain[k].to_host(), fast[k].to_host()), k
     for i in (0, batch - 1):

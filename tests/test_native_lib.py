@@ -79,6 +79,10 @@ def test_argument_errors_need_no_gpu(native):
         native.check(native.ERR_TOO_MANY_GT)
     with pytest.raises(ValueError):
         native.check(native.ERR_ARG)
+    from ssdgeom import device as D
+    for priority in (0, 2, "medium"):          # "high", "low" or None only
+        with pytest.raises(ValueError):
+            D.Stream(priority)
 
 
 def test_no_cpu_fallback(native):
