@@ -404,6 +404,33 @@ SSDG_API int ssdg_eval_finalize(void* state, size_t state_bytes, int32_t n_class
                        int32_t n_recall, double* out_precision, double* out_recall, int64_t* out_n_gt,
                        int64_t* out_n_det, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- A12: per-image keep_top_k -----------------------------------------------------------------------------
+ * The reference has no post-processing beyond the score head.  The final detections of each image (the original
+ * SSD's DetectionOutput keep_top_k, torchvision's detections_per_img): the kept lists of ssdg_detect /
+ * ssdg_detect_stage / ssdg_nms ranked across classes and capped at keep_top_k = K (spec: tests/keep_top_k_oracle.py;
+ * PARITY UNPINNED like A9).
+ *   candidates of image b: the first clamp(count[b][c], 0, top_k) entries of every class list c (score
+ *     non-increasing, as those entry points write them), ranked by kept_score descending (compared as floats:
+ *     -0 == +0), then class ascending, then position in the list ascending; the first min(K, total) are kept.
+ *   The survivors of every class form a prefix of its list, so out_count is itself a count array:
+ *     (kept, out_count, kept_score, boxes) goes unchanged to everything that reads kept lists (ssdg_eval_accumulate).
+ * Outputs (K slots per image, in rank order):
+ *   out_prior int32 [B,K]   prior index (-1 padded)      out_class int32 [B,K]  foreground class in [0, C-1) (-1 padded)
+ *   out_score float [B,K]   kept_score (0 padded)        out_box   float [B,K,4] or NULL: decoded cxcywh of the
+ *     prior from `boxes` [B,A,4] (needs boxes and n_priors = A; 0 padded, and 0 for a prior index outside [0, A),
+ *     which is never dereferenced)
+ *   out_n int32 [B]  detections per image             out_count int32 [B,C-1] or NULL: survivors per class list
+ * No workspace.  Limits: 1 <= keep_top_k <= 1024, top_k <= 1024, n_classes <= 2048, the batch limit of ssdg_detect.
+ * boxes and out_box 16-byte aligned.  Lists that are not score-sorted are outside the contract (nothing outside the
+ * arrays is read or written for them either).
+ */
+SSDG_API int ssdg_detect_keep_top_k(const int32_t* kept, const int32_t* count, const float* kept_score, int32_t top_k,
+                                    const float* boxes /* [B,A,4] decoded, 16-byte aligned, or NULL */,
+                                    int64_t batch, int32_t n_priors, int32_t n_classes, int32_t keep_top_k,
+                                    int32_t* out_prior /* [B,K], -1 padded */, int32_t* out_class /* [B,K], -1 padded */,
+                                    float* out_score /* [B,K], 0 padded */, float* out_box /* [B,K,4] or NULL, 0 padded */,
+                                    int32_t* out_n /* [B] */, int32_t* out_count /* [B,C-1] or NULL */, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -1122,6 +1122,242 @@ static int run_nms(const DetectWs& ws, const float* boxes, long long batch, int 
   return SSDG_OK;
 }
 
+// ---- per-image keep_top_k (A12) -----------------------------------------------------------------------
+// One CTA per image ranks the candidates of its class lists -- the first min(clamp(count, 0, top_k), K) entries of
+// each (nothing beyond can be selected) -- by (score desc, class asc, position asc) and keeps the first K:
+//   * the per-class lengths and their prefix in shared memory;
+//   * more than K candidates: a radix select (8 bits x 4 passes) finds the K-th largest score key t and how many of
+//     the entries equal to t are taken.  When every list's candidate slots fit (kTopkCache keys: SSD300's 80 x 200
+//     do), one coalesced pass copies the score keys into shared memory first; otherwise every pass reads them from
+//     global memory.  A pass walks each class list with one warp and counts RUNS of equal digits (a run of digit d
+//     over [s, e] adds e + 1 - s to bin d): score-sorted lists have a handful of runs, so the shared-memory atomics
+//     are few and rarely contended -- and the counts are exact for any order of the entries;
+//   * per class, one warp counts the entries > t and == t; the ties go to the classes in ascending order (a prefix
+//     over the tie counts), so every class keeps a prefix m_c of its list -- a valid count array itself;
+//   * the survivors get the unique key  key32(score) << 32 | (2047 - class) << 10 | (1023 - position)  and a rank
+//     sort (rank = number of larger keys, K <= 1024) puts them in place; the outputs are written in rank order.
+constexpr int kTopkThreads = 512;
+constexpr int kTopkWarps = kTopkThreads / 32;
+constexpr int kTopkCache = 16384;   // score keys cached in shared memory (64 KB)
+
+struct TopkParams {
+  const int* kept;           // [B][nfg][top_k]
+  const int* count;          // [B][nfg]
+  const float* score;        // [B][nfg][top_k]
+  const float* boxes;        // [B][A][4] or null
+  int A, nfg, top_k, K;
+  int cache;                 // nfg * min(top_k, K) when that fits kTopkCache (the cache holds [nfg][min(top_k, K)]), else 0
+  int* out_prior;            // [B][K]
+  int* out_class;            // [B][K]
+  float* out_score;          // [B][K]
+  float* out_box;            // [B][K][4] or null
+  int* out_n;                // [B]
+  int* out_count;            // [B][nfg] or null
+};
+
+// In-place exclusive scan of a[0, n) in shared memory, a[n] = total; every thread calls it.
+__device__ __forceinline__ void topk_block_scan(u32* a, int n, u32* wsum) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int per = (n + kTopkThreads - 1) / kTopkThreads;
+  const int lo = min(n, tid * per), hi = min(n, lo + per);
+  u32 s = 0u;
+  for (int i = lo; i < hi; ++i) s += a[i];
+  u32 incl = s;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const u32 v = __shfl_up_sync(SSDG_FULL, incl, o);
+    if (lane >= o) incl += v;
+  }
+  if (lane == 31) wsum[warp] = incl;
+  __syncthreads();
+  u32 run = incl - s + __reduce_add_sync(SSDG_FULL, lane < warp ? wsum[lane] : 0u);   // the warps before this one
+  for (int i = lo; i < hi; ++i) {
+    const u32 v = a[i];
+    a[i] = run;
+    run += v;
+  }
+  if (tid == kTopkThreads - 1) a[n] = run;   // the last thread's range ends the array (later ranges are empty)
+  __syncthreads();
+}
+
+__global__ void __launch_bounds__(kTopkThreads) keep_top_k_kernel(TopkParams P) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int nfg = P.nfg, K = P.K, top_k = P.top_k;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  u64* skey = reinterpret_cast<u64*>(smem_raw);                    // [K] survivor keys
+  u32* len = reinterpret_cast<u32*>(skey + K);                     // [nfg] candidates, later survivors, per class
+  u32* off = len + nfg;                                            // [nfg + 1] their prefix
+  u32* cgt = off + nfg + 1;                                        // [nfg] entries > t per class
+  u32* ceq = cgt + nfg;                                            // [nfg + 1] entries == t per class, then their prefix
+  u32* hist = ceq + nfg + 1;                                       // [256]
+  u32* wsum = hist + 256;                                          // [kTopkWarps]
+  u32* cache = wsum + kTopkWarps;                                  // [nfg][lim] score keys (P.cache > 0)
+  __shared__ u32 sel_prefix, sel_k;
+
+  const long long b = blockIdx.x;
+  const int* cnt = P.count + b * nfg;
+  const size_t row0 = (size_t)b * nfg;                              // first list of the image
+  const int lim = min(top_k, K);
+  for (int c = tid; c < nfg; c += kTopkThreads) {
+    off[c] = len[c] = (u32)min(max(cnt[c], 0), lim);
+  }
+  __syncthreads();
+  topk_block_scan(off, nfg, wsum);
+  const u32 total = off[nfg];
+  u32 n = total;
+  const bool cached = P.cache > 0 && total > (u32)K;   // the keys are copied only for a select
+  auto key = [&](int c, int j) {
+    return cached ? cache[c * lim + j] : key32(P.score[(row0 + c) * top_k + j]);
+  };
+  if (total > (u32)K) {
+    if (cached) {   // eight independent loads in flight per thread; slots past a list's length are never read
+      const u32 nslot = (u32)P.cache;
+      for (u32 i0 = tid; i0 < nslot; i0 += 8 * kTopkThreads) {
+        float v[8];
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          const u32 i = i0 + u * kTopkThreads, c = i / (u32)lim, j = i - c * (u32)lim;
+          v[u] = (i < nslot && j < len[c]) ? P.score[(row0 + c) * top_k + j] : 0.f;
+        }
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          const u32 i = i0 + u * kTopkThreads;
+          if (i < nslot) cache[i] = key32(v[u]);
+        }
+      }
+    }
+    if (tid == 0) { sel_prefix = 0u; sel_k = (u32)K; }
+    // Radix select of the K-th largest score key (with multiplicity), 8 bits per pass.
+#pragma unroll 1
+    for (int shift = 24; shift >= 0; shift -= 8) {
+      for (int i = tid; i < 256; i += kTopkThreads) hist[i] = 0u;
+      __syncthreads();
+      const u32 pre = sel_prefix;
+      const u32 hmask = shift == 24 ? 0u : (~0u << (shift + 8));
+      constexpr u32 kNone = 0xffffffffu;   // an entry outside the prefix (or past the list)
+      for (int c = warp; c < nfg; c += kTopkWarps) {
+        const int L = (int)len[c];
+        u32 prev = kNone;                  // digit of entry j0 - 1
+        for (int j0 = 0; j0 < L; j0 += 32) {
+          const int j = j0 + lane;
+          u32 d = kNone;
+          if (j < L) {
+            const u32 k = key(c, j);
+            if ((k & hmask) == pre) d = (k >> shift) & 255u;
+          }
+          u32 dp = __shfl_up_sync(SSDG_FULL, d, 1);
+          if (lane == 0) dp = prev;
+          prev = __shfl_sync(SSDG_FULL, d, min(31, L - 1 - j0));
+          if (j < L && d != dp) {          // a run of dp ends at j - 1, a run of d starts at j
+            if (dp != kNone) atomicAdd(&hist[dp], (u32)j);
+            if (d != kNone) atomicSub(&hist[d], (u32)j);
+          }
+        }
+        if (lane == 0 && prev != kNone) atomicAdd(&hist[prev], (u32)L);   // the last run ends the list
+      }
+      __syncthreads();
+      if (warp == 0) {   // lane l owns digits 255-8l .. 248-8l; the digit where the count from the top reaches sel_k
+        u32 h[8], tot = 0u;
+#pragma unroll
+        for (int r = 0; r < 8; ++r) { h[r] = hist[255 - 8 * lane - r]; tot += h[r]; }
+        u32 incl = tot;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+          const u32 v = __shfl_up_sync(SSDG_FULL, incl, o);
+          if (lane >= o) incl += v;
+        }
+        const u32 kk = sel_k;
+        u32 above = incl - tot;
+        __syncwarp();
+#pragma unroll
+        for (int r = 0; r < 8; ++r) {
+          if (above < kk && above + h[r] >= kk) {
+            sel_prefix = pre | ((u32)(255 - 8 * lane - r) << shift);
+            sel_k = kk - above;
+          }
+          above += h[r];
+        }
+      }
+      __syncthreads();
+    }
+    const u32 t = sel_prefix, take = sel_k;   // the K-th largest key; how many of the keys == t are kept
+    for (int c = warp; c < nfg; c += kTopkWarps) {
+      const int L = (int)len[c];
+      u32 g = 0u, e = 0u;
+      for (int j = lane; j < L; j += 32) {
+        const u32 k = key(c, j);
+        g += k > t;
+        e += k == t;
+      }
+      g = __reduce_add_sync(SSDG_FULL, g);
+      e = __reduce_add_sync(SSDG_FULL, e);
+      if (lane == 0) { cgt[c] = g; ceq[c] = e; }
+    }
+    __syncthreads();
+    topk_block_scan(ceq, nfg, wsum);
+    for (int c = tid; c < nfg; c += kTopkThreads) {   // the ties go to the classes in ascending order
+      const u32 e = ceq[c + 1] - ceq[c];
+      const u32 rest = take > ceq[c] ? take - ceq[c] : 0u;
+      off[c] = len[c] = cgt[c] + min(e, rest);
+    }
+    __syncthreads();
+    topk_block_scan(off, nfg, wsum);
+    n = off[nfg];   // == K: the histograms are exact, so t is the K-th largest key and take <= its multiplicity
+  }
+  // the survivors: the prefix len[c] of every list, at off[c] in class order
+  for (int c = warp; c < nfg; c += kTopkWarps) {
+    const int m = (int)len[c];
+    for (int j = lane; j < m; j += 32)
+      skey[off[c] + j] = ((u64)key(c, j) << 32) | ((u64)(2047 - c) << 10) | (u64)(1023 - j);
+  }
+  if (P.out_count)
+    for (int c = tid; c < nfg; c += kTopkThreads) P.out_count[row0 + c] = (int)len[c];
+  __syncthreads();
+  // rank sort, descending (the keys are unique): each thread ranks up to K / kTopkThreads keys in one sweep
+  constexpr int kPer = 1024 / kTopkThreads;
+  u64 v[kPer];
+  u32 rank[kPer];
+#pragma unroll
+  for (int q = 0; q < kPer; ++q) {
+    const u32 i = (u32)(tid + q * kTopkThreads);
+    v[q] = i < n ? skey[i] : ~0ull;
+    rank[q] = 0u;
+  }
+  for (u32 s = 0; s < n; ++s) {
+    const u64 x = skey[s];
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) rank[q] += x > v[q];
+  }
+  const size_t o0 = (size_t)b * K;
+#pragma unroll
+  for (int q = 0; q < kPer; ++q) {
+    if ((u32)(tid + q * kTopkThreads) >= n) break;
+    const int c = 2047 - (int)((v[q] >> 10) & 2047u), j = 1023 - (int)(v[q] & 1023u);
+    const size_t g = (row0 + c) * top_k + j;
+    const int p = P.kept[g];
+    const size_t o = o0 + rank[q];
+    P.out_prior[o] = p;
+    P.out_class[o] = c;
+    P.out_score[o] = P.score[g];
+    if (P.out_box) {   // a prior index outside [0, A) is never dereferenced
+      const float4 bx = (p >= 0 && p < P.A) ? __ldg(reinterpret_cast<const float4*>(P.boxes) + (size_t)b * P.A + p)
+                                            : make_float4(0.f, 0.f, 0.f, 0.f);
+      reinterpret_cast<float4*>(P.out_box)[o] = bx;
+    }
+  }
+  for (u32 r = n + tid; r < (u32)K; r += kTopkThreads) {
+    P.out_prior[o0 + r] = -1;
+    P.out_class[o0 + r] = -1;
+    P.out_score[o0 + r] = 0.f;
+    if (P.out_box) reinterpret_cast<float4*>(P.out_box)[o0 + r] = make_float4(0.f, 0.f, 0.f, 0.f);
+  }
+  if (tid == 0) P.out_n[b] = (int)n;
+}
+
+static size_t topk_smem_bytes(int nfg, int K, int cache) {
+  return (size_t)K * 8 + ((size_t)4 * nfg + 2 + 256 + kTopkWarps + (size_t)cache) * 4;
+}
+
 static void fill_params(DetectParams& P, const DetectWs& ws, long long batch, int A, int C) {
   P.B = (int)batch; P.A = A; P.C = C; P.tpi = (A + 31) / 32;
   P.lists = ws.lists; P.run_cnt = ws.run_cnt;
@@ -1221,4 +1457,30 @@ extern "C" int ssdg_nms(const float* probs, const float* boxes, int64_t batch, i
   int rc = run_filter<true>(P, SSDG_F32, st);
   if (rc) return rc;
   return run_nms(ws, boxes, batch, n_priors, n_classes, top_k, iou_thresh, out_kept, out_count, out_kept_score, st);
+}
+
+extern "C" int ssdg_detect_keep_top_k(const int32_t* kept, const int32_t* count, const float* kept_score, int32_t top_k,
+                                      const float* boxes, int64_t batch, int32_t n_priors, int32_t n_classes,
+                                      int32_t keep_top_k, int32_t* out_prior, int32_t* out_class, float* out_score,
+                                      float* out_box, int32_t* out_n, int32_t* out_count, void* stream) {
+  if (!kept || !count || !kept_score || !out_prior || !out_class || !out_score || !out_n) return SSDG_ERR_ARG;
+  if (out_box && (!boxes || n_priors <= 0)) return SSDG_ERR_ARG;
+  if (batch <= 0 || top_k <= 0 || n_classes < 2 || keep_top_k <= 0) return SSDG_ERR_ARG;
+  if (top_k > 1024 || keep_top_k > 1024 || n_classes > 2048 || batch > 0x7fffffff / 64) return SSDG_ERR_LIMIT;
+  if (((uintptr_t)boxes | (uintptr_t)out_box) & 15) return SSDG_ERR_ALIGN;
+  TopkParams P;
+  P.kept = kept; P.count = count; P.score = kept_score; P.boxes = boxes;
+  P.A = n_priors; P.nfg = n_classes - 1; P.top_k = top_k; P.K = keep_top_k;
+  // every list's candidate slots in shared memory when they fit kTopkCache keys (else the select reads global memory)
+  const long long slots = (long long)P.nfg * std::min(top_k, keep_top_k);
+  P.cache = slots <= kTopkCache ? (int)slots : 0;
+  P.out_prior = out_prior; P.out_class = out_class; P.out_score = out_score; P.out_box = out_box;
+  P.out_n = out_n; P.out_count = out_count;
+  const size_t smem = topk_smem_bytes(P.nfg, P.K, P.cache);
+  if ((int)smem > max_smem_optin()) return SSDG_ERR_LIMIT;
+  if (smem > 48 * 1024)
+    SSDG_CUDA_TRY(cudaFuncSetAttribute(keep_top_k_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  keep_top_k_kernel<<<(unsigned)batch, kTopkThreads, smem, (cudaStream_t)stream>>>(P);
+  SSDG_LAUNCH_CHECK();
+  return SSDG_OK;
 }

@@ -85,6 +85,8 @@ PROTOTYPES = {
     "ssdg_multibox_loss_fused": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp,
                                            _vp, _vp, _vp, _sz, _vp]),
     "ssdg_nms": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _i32, _f32, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "ssdg_detect_keep_top_k": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
+                                         _vp]),
     "ssdg_eval_state_bytes": (_sz, [_i32, _i64, _i32, _i32]),
     "ssdg_eval_reset": (C.c_int, [_vp, _sz, _vp]),
     "ssdg_eval_accumulate": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _pf64, _i32,

@@ -8,6 +8,13 @@ Only the finished precision / recall arrays cross to the host.
         ev.add(det, gt_boxes, gt_cls, gt_off)        # CSR ground truth, as ops.match_encode
     ev.exchange(comm)                                # data parallel only: sum the slots over the processes
     res = ev.summarize()                             # {"AP", "AP50", "AP75", "AR", "per_class_AP", ...}
+
+The evaluator caps each (image, class) list at ``max_dets``.  For a detector that emits at most K detections per image,
+feed it the per-image capped lists of ``ops.keep_top_k``: their survivors are a prefix of every list, so only the counts
+change --
+
+        top = ops.keep_top_k(det, 100)
+        ev.add(dict(det, count=top["count"]), gt_boxes, gt_cls, gt_off)
 """
 from __future__ import annotations
 

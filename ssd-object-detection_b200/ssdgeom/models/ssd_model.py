@@ -85,6 +85,18 @@ def detect(pred_conf, pred_bbox, prior_box, score_thresh=0.01, top_k=200, iou_th
     return kept, count
 
 
+def detections(pred_conf, pred_bbox, prior_box, score_thresh=0.01, top_k=200, iou_thresh=0.45, keep_top_k=200):
+    """The final detections of every image: decode + softmax + per-class NMS, then the lists ranked across classes
+    (score desc, class asc) and capped at ``keep_top_k`` on the device -- what ``visualize`` (models/ssd_model.py:477-490)
+    draws, with NMS and a per-image cap.  Returns host arrays {"boxes": f32[b,K,4] decoded cxcywh (relative units),
+    "scores": f32[b,K], "labels": i32[b,K], "priors": i32[b,K], "n": i32[b]}; slots past n are -1 / 0."""
+    det = ops.detect(pred_conf, pred_bbox, prior_box, score_thresh, top_k, iou_thresh, want_scores=True,
+                     want_boxes=True)
+    top = ops.keep_top_k(det, keep_top_k)
+    return {"boxes": top["box"].to_host(), "scores": top["score"].to_host(), "labels": top["class"].to_host(),
+            "priors": top["prior"].to_host(), "n": top["n"].to_host()}
+
+
 def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45):
     """Per-class NMS on given probabilities f32[b,A,C] and decoded boxes f32[b,A,4]."""
     out = ops.nms(np.ascontiguousarray(np.asarray(probs, dtype=np.float32)) if not D.is_device(probs) else probs,
@@ -125,6 +137,9 @@ class SSDBoxGeometry:
 
     def detect(self, pred_conf, pred_bbox, score_thresh=0.01, top_k=200, iou_thresh=0.45):
         return detect(pred_conf, pred_bbox, self._prior_dev, score_thresh, top_k, iou_thresh)
+
+    def detections(self, pred_conf, pred_bbox, score_thresh=0.01, top_k=200, iou_thresh=0.45, keep_top_k=200):
+        return detections(pred_conf, pred_bbox, self._prior_dev, score_thresh, top_k, iou_thresh, keep_top_k)
 
     def visualize_scores(self, pred_conf, thresh=0.5):
         return score_head(pred_conf, thresh)

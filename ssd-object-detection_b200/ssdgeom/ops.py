@@ -466,6 +466,41 @@ def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores
     return out
 
 
+# ---- A12 ------------------------------------------------------------------------------------------------
+def keep_top_k(det: dict, keep_top_k: int, out=None, stream=None) -> dict:
+    """The final detections of every image (include/ssdgeom.h, ssdg_detect_keep_top_k): the kept lists of a ``detect``
+    / ``nms`` output with ``kept_score`` ranked across classes (score desc, class asc, position asc) and capped at
+    ``keep_top_k``.  Returns device arrays prior i32[B,K], class i32[B,K], score f32[B,K], n i32[B] and count
+    i32[B,C-1] (the survivors per class list, a prefix of each: ``dict(det, count=top["count"])`` is a capped
+    detection output), plus box f32[B,K,4] when ``det`` has ``boxes``.  ``out`` may carry preallocated arrays."""
+    if "kept_score" not in det:
+        raise ValueError("detect output lacks 'kept_score': call ops.detect(..., want_scores=True)")
+    kept, count = D.as_device(det["kept"], np.int32, stream), D.as_device(det["count"], np.int32, stream)
+    kept_score = D.as_device(det["kept_score"], np.float32, stream)
+    boxes = D.as_device(det["boxes"], np.float32, stream) if det.get("boxes") is not None else None
+    if len(kept.shape) != 3:
+        raise AssertionError("kept must be [B,C-1,top_k]")
+    b, k, top_k = kept.shape
+    if count.size != b * k or kept_score.size != kept.size or (boxes is not None and
+                                                               (len(boxes.shape) != 3 or boxes.shape[0] != b)):
+        raise AssertionError("kept, count, kept_score and boxes disagree in shape")
+    kk = int(keep_top_k)
+    out = dict(out or {})
+    spec = {"prior": ((b, kk), np.int32), "class": ((b, kk), np.int32), "score": ((b, kk), np.float32),
+            "n": ((b,), np.int32), "count": ((b, k), np.int32)}
+    if boxes is not None:
+        spec["box"] = ((b, kk, 4), np.float32)
+    for key, (shape, dt) in spec.items():
+        if key not in out:
+            out[key] = D.empty(shape, dt)
+    a = int(boxes.shape[1]) if boxes is not None else 0
+    N.check(N.lib().ssdg_detect_keep_top_k(kept.ptr, count.ptr, kept_score.ptr, top_k, _p(boxes), b, a, k + 1, kk,
+                                           out["prior"].ptr, out["class"].ptr, out["score"].ptr, _p(out.get("box")),
+                                           out["n"].ptr, out["count"].ptr, D.stream_handle(stream)), "keep_top_k")
+    out["_keep"] = (kept, count, kept_score, boxes)
+    return out
+
+
 # ---- A11 ------------------------------------------------------------------------------------------------
 EVAL_STATUS_BAD_CLASS, EVAL_STATUS_TOO_MANY_GT, EVAL_STATUS_DUPLICATE, EVAL_STATUS_BAD_PRIOR = 1, 2, 4, 8
 

@@ -17,7 +17,7 @@ INPUT_NAMES = ("gt_boxes", "gt_cls", "gt_off", "pred_cls", "pred_box")
 class HotPath:
     def __init__(self, table=None, batch=256, max_gt=100, classes=81, thresh=0.5, neg_ratio=3,
                  score_thresh=0.01, top_k=200, iou_thresh=0.45, total_gt=None, mining="shard", global_priors=None,
-                 allreduce=None, comm=None, depth=1, evaluator=None):
+                 allreduce=None, comm=None, depth=1, evaluator=None, keep_top_k=None):
         """depth: steps in flight.  1 -- ``step()`` joins both branches on ``s_main`` before it returns the stream to
         the caller (a step is a closed unit).  2 -- every per-step buffer (targets, row statistics, candidate lists,
         workspaces, results) exists twice and consecutive steps use them in turn: step k+1 starts as soon as its
@@ -35,7 +35,11 @@ class HotPath:
         ``loss_exchange(stream)`` callables (a torch.distributed or gloo stand-in) do.
 
         evaluator: an ``evaluate.DetectionEvaluator``; every step then also matches its kept lists to its ground truth
-        (``step(image_base)``) after the NMS, on the NMS stream.  None (the default) changes nothing."""
+        (``step(image_base)``) after the NMS, on the NMS stream.  None (the default) changes nothing.
+
+        keep_top_k: an int K in [1, 1024]; every step then also ranks the kept lists of each image across classes and
+        keeps the first K (ops.keep_top_k) on the NMS stream, right after the NMS; ``download_detections`` copies them
+        out.  An evaluator then matches the capped lists.  None (the default) changes nothing."""
         table = SSD300 if table is None else table
         self.batch, self.max_gt, self.classes = int(batch), int(max_gt), int(classes)
         self.thresh, self.neg_ratio = float(thresh), int(neg_ratio)
@@ -53,15 +57,24 @@ class HotPath:
         self.evaluator = evaluator
         if evaluator is not None and (evaluator.n_classes != c or evaluator.max_dets > self.top_k):
             raise ValueError("the evaluator needs n_classes == classes and max_dets <= top_k")
+        if keep_top_k is not None and not 1 <= int(keep_top_k) <= 1024:
+            raise ValueError("keep_top_k must be None or in [1, 1024]")
+        self.keep_top_k = None if keep_top_k is None else int(keep_top_k)
 
         def make_slot():   # everything a step writes
             det = {"kept": D.empty((b, c - 1, self.top_k), np.int32), "count": D.empty((b, c - 1), np.int32)}
-            if evaluator is not None:   # the filter then writes the decoded boxes here instead of into its workspace
+            if evaluator is not None or self.keep_top_k is not None:   # the filter then writes the decoded boxes here
                 det.update(kept_score=D.empty((b, c - 1, self.top_k), np.float32), boxes=D.empty((b, a, 4), np.float32))
+            top = None
+            if self.keep_top_k is not None:
+                kk = self.keep_top_k
+                top = {"prior": D.empty((b, kk), np.int32), "class": D.empty((b, kk), np.int32),
+                       "score": D.empty((b, kk), np.float32), "box": D.empty((b, kk, 4), np.float32),
+                       "n": D.empty((b,), np.int32), "count": D.empty((b, c - 1), np.int32)}
             return {"tgt": {"cls": D.empty((b, a), np.int32), "loc": D.empty((b, a, 4), np.float32),
                             "mask": D.empty((b, a), np.uint8)},
                     "loss": {"result": D.empty((N.LOSS_RESULT_LEN,), np.float64)},
-                    "det": det,
+                    "det": det, "top": top,
                     "det_stats": {"row_ml": D.empty((b, a, 2), np.float32), "row_negbg": D.empty((b, a), np.float32)},
                     "pool": ops.WorkspacePool(), "ev_a": D.Event(), "ev_d": D.Event(), "ev_x": D.Event(),
                     "x_pending": False, "used": False, "loss_exchange": None}
@@ -108,7 +121,7 @@ class HotPath:
             self.staged = ops.StagedLoss(self.tgt["cls"], self.tgt["loc"], self.tgt["mask"], self.pred_box, self.pred_cls,
                                          int(global_priors), self.neg_ratio, out=self.loss)
         # search, match | lossprep (or ce), select x2, final | filter, nms
-        self.kernel_launches_per_step = 8 + (1 if evaluator is not None else 0)
+        self.kernel_launches_per_step = 8 + (1 if evaluator is not None else 0) + (1 if self.keep_top_k is not None else 0)
         # matcher head + loss histograms (cudaMemsetAsync), + the lead node of small batches
         self.memsets_per_step = 2 + (1 if self.lead_assign else 0)
         self.h2d_bytes = sum(self._sets[0][k].nbytes for k in INPUT_NAMES)
@@ -123,6 +136,7 @@ class HotPath:
         sl = self._slots[k]
         self._cur = sl
         self.tgt, self.loss, self.det, self.det_stats, self.pool = sl["tgt"], sl["loss"], sl["det"], sl["det_stats"], sl["pool"]
+        self.top = sl["top"]
         self.ev_a, self.ev_d, self.ev_x = sl["ev_a"], sl["ev_d"], sl["ev_x"]
 
     @property
@@ -183,8 +197,12 @@ class HotPath:
         ops.detect(self.pred_cls, self.pred_box, self.priors, self.score_thresh, self.top_k, self.iou_thresh,
                    out=out, stream=stream, stage=stage, want_row_stats=stats, pool=self.pool)
 
+    def keep_top_k_stage(self, stream):
+        ops.keep_top_k(self.det, self.keep_top_k, out=self.top, stream=stream)
+
     def evaluate_stage(self, stream, image_base=None):
-        self.evaluator.add(self.det, self.gt_boxes, self.gt_cls, self.gt_off, image_base, stream, max_gt=self.max_gt)
+        det = self.det if self.top is None else dict(self.det, count=self.top["count"])   # the capped lists
+        self.evaluator.add(det, self.gt_boxes, self.gt_cls, self.gt_off, image_base, stream, max_gt=self.max_gt)
 
     def step(self, image_base=None):
         """One pass of the chain over the resident batch; work is ordered on ``s_main``.  With an evaluator the batch's
@@ -220,6 +238,8 @@ class HotPath:
             self.ev_mid.record(self.s_d)
             D.stream_wait_event(self.s_n, self.ev_mid)
             self.detect_stage(self.s_n, stage=1, stats=fused)
+            if self.top is not None:
+                self.keep_top_k_stage(self.s_n)
             if self.evaluator is not None:      # before ev_d: the waits on ev_d cover its reads of GT and lists
                 self.evaluate_stage(self.s_n, image_base)
             D.stream_wait_event(self.s_l, self.ev_m)
@@ -241,6 +261,8 @@ class HotPath:
             self.ev_d.record(self.s_n)
         else:
             self.detect_stage(self.s_d)
+            if self.top is not None:
+                self.keep_top_k_stage(self.s_d)
             if self.evaluator is not None:
                 self.evaluate_stage(self.s_d, image_base)
             self.assign(self.s_a)
@@ -302,6 +324,21 @@ class HotPath:
         if self._match_out is not None:      # the matcher's status word travels with the results (include/ssdgeom.h)
             ws = self._match_out["_match_ws"]
             N.check(lib.ssdg_memcpy_d2h(self._status_host.ptr, ws.ptr, 8, D.stream_handle(st)), "d2h")
+
+    def download_detections(self, out: dict, stream=None):
+        """Copy the last step's final detections (``keep_top_k``) into host arrays: ``out`` maps any of "prior",
+        "class", "score", "box", "n", "count" to a host array of that shape and dtype.  Waits for the last step as
+        ``download`` does; the copies are asynchronous on ``stream`` (s_main)."""
+        if self.top is None:
+            raise RuntimeError("this HotPath was built without keep_top_k")
+        st = self.s_main if stream is None else stream
+        if self.depth > 1:
+            self.join(st)
+        lib = N.lib()
+        for key, dst in out.items():
+            src = self.top[key]
+            assert dst.nbytes == src.nbytes and dst.dtype == src.dtype and dst.flags["C_CONTIGUOUS"]
+            N.check(lib.ssdg_memcpy_d2h(dst.ctypes.data, src.ptr, src.nbytes, D.stream_handle(st)), "d2h")
 
     def check_status(self, sync=False):
         """Raise if the device had to skip an image or saw a stale prior index: from the status word the last
