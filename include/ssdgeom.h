@@ -99,7 +99,6 @@ SSDG_API int ssdg_event_elapsed_ms(void* start, void* stop, float* ms); /* synch
 #define SSDG_PROF_CE 1
 #define SSDG_PROF_FILTER 2
 #define SSDG_PROF_NMS 3
-#define SSDG_PROF_BUCKET 4      /* unused (the bucketing pass is gone: the filter appends to the class lists) */
 #define SSDG_PROF_SEARCH 5      /* search_kernel (SSDG_PROF_MATCH covers search + per-image kernel) */
 #define SSDG_PROF_LOSS_TAIL 6   /* select_kernel x2 + final_kernel */
 #define SSDG_PROF_GRAD 7        /* grad_kernel */

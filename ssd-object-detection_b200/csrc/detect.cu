@@ -3,7 +3,7 @@
 // nms_per_class, IoU formula utils/bbox.py:13-25 in float32).
 //
 //   filter_kernel  one streaming pass over the logits [B,A,C].  Tiles are 32 priors of ONE image; every CTA owns
-//                  one contiguous run of tiles and each of its 16 warps one shared-memory tile at a time, filled
+//                  one contiguous run of tiles and each of its warps one shared-memory tile at a time, filled
 //                  by 1-D bulk TMA (cp.async.bulk + mbarrier).  Row phase, lane r owns row r (stride C words:
 //                  conflict-free for odd C): e_c = 2^((x_c - ref) log2e) with the background logit as reference
 //                  (one pass; rows that would overflow or lose precision are redone with their maximum), the
@@ -44,7 +44,7 @@ constexpr int kNmsThreads = 128;
 constexpr int kNmsWarps = kNmsThreads / 32;
 constexpr int kSlabs = 32;   // slabs per axis of the NMS candidate join
 constexpr int kSizeCls = 16; // width / height classes of the join
-constexpr int kABitsD = 21;     // limit on the prior index (A < 2^21) kept from the staged format
+constexpr int kABitsD = 21;     // limit on the prior count of a detection call (A < 2^21)
 
 struct DetectParams {
   const float* pred_cls;   // logits (filter) or probabilities (kProbs)
@@ -399,7 +399,7 @@ __global__ void __maxnreg__(kFilterMaxRegs) filter_kernel(DetectParams P, int wa
       mbar_arrive_expect_tx(mybar, bytes);
       tma_load_hint(tile, P.pred_cls + ((size_t)ib * A + (size_t)ij * 32) * C, bytes, mybar, pol);
     };
-    // One tile in flight per warp; the other 15 warps of the CTA hide its latency.  That alone leaves too few bytes
+    // One tile in flight per warp; the other warps of the CTA hide its latency.  That alone leaves too few bytes
     // in flight towards DRAM (a buffer that is being computed on requests nothing): the warp also asks L2 for the
     // tile it will load `prefetch` rounds later, so the bulk copy into shared memory finds its lines in L2.
     // (image, tile) of the tile `prefetch` + 1 rounds ahead, walked like (b, j)
@@ -1053,23 +1053,27 @@ static size_t detect_ws_layout(long long batch, int A, int C, DetectWs* out, uns
   return o;
 }
 
-template <bool kProbs>
-static int run_filter(DetectParams& P, int prior_dtype, cudaStream_t st) {
+// What the filter pass reads: logits with box offsets and priors (ssdg_detect, ssdg_detect_stage), or probabilities
+// with the caller's decoded boxes (ssdg_nms; no priors, no side outputs).
+enum class DetectMode { kLogits, kProbs };
+
+static int run_filter(DetectParams& P, DetectMode mode, int prior_dtype, cudaStream_t st) {
   FilterGeom g;
   if (!filter_geom(P.B, P.A, P.C, &g)) return SSDG_ERR_LIMIT;
   P.chunk = g.chunk; P.max_li = g.max_li; P.max_slots = g.max_slots;
   P.tma_ok = (((long long)P.A * P.C) % 4 == 0) && (((uintptr_t)P.pred_cls & 15) == 0);
   prof_begin(SSDG_PROF_FILTER, st);
   // kWrite: the rows must hold exp(x - max) after the pass (probabilities output, score head)
-  const bool wr = !kProbs && (P.probs || P.head_score || P.head_cls || P.head_mask);
+  const bool wr = P.probs || P.head_score || P.head_cls || P.head_mask;
   auto go = [&](auto kern) -> int {
     SSDG_CUDA_TRY(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)g.smem));
     kern<<<g.grid, kFThreads, g.smem, st>>>(P, g.warps, kFilterPrefetch);
     return SSDG_OK;
   };
   int rc;
-  if (prior_dtype == SSDG_F64) rc = wr ? go(filter_kernel<double, kProbs, true>) : go(filter_kernel<double, kProbs, false>);
-  else rc = wr ? go(filter_kernel<float, kProbs, true>) : go(filter_kernel<float, kProbs, false>);
+  if (mode == DetectMode::kProbs) rc = go(filter_kernel<float, true, false>);
+  else if (prior_dtype == SSDG_F64) rc = wr ? go(filter_kernel<double, false, true>) : go(filter_kernel<double, false, false>);
+  else rc = wr ? go(filter_kernel<float, false, true>) : go(filter_kernel<float, false, false>);
   if (rc != SSDG_OK) return rc;
   prof_end(SSDG_PROF_FILTER, st);
   SSDG_LAUNCH_CHECK();
@@ -1358,12 +1362,6 @@ static size_t topk_smem_bytes(int nfg, int K, int cache) {
   return (size_t)K * 8 + ((size_t)4 * nfg + 2 + 256 + kTopkWarps + (size_t)cache) * 4;
 }
 
-static void fill_params(DetectParams& P, const DetectWs& ws, long long batch, int A, int C) {
-  P.B = (int)batch; P.A = A; P.C = C; P.tpi = (A + 31) / 32;
-  P.lists = ws.lists; P.run_cnt = ws.run_cnt;
-  P.list_cap = (size_t)P.tpi * 32;
-}
-
 }  // namespace ssdg
 
 using namespace ssdg;
@@ -1374,38 +1372,48 @@ extern "C" size_t ssdg_detect_workspace_bytes(int64_t batch, int32_t n_priors, i
   return detect_ws_layout(batch, n_priors, n_classes, nullptr, nullptr);
 }
 
-// stages: 1 = softmax filter + decode + candidate bucketing, 2 = per-class NMS (reads what stage 1 left in the workspace)
-static int detect_run(int stages, const float* pred_cls, const float* pred_box, const void* priors, int32_t prior_dtype,
-                      int64_t batch, int32_t n_priors, int32_t n_classes, float score_thresh, int32_t top_k,
-                      float iou_thresh, int32_t* out_kept, int32_t* out_count, float* out_kept_score,
-                      float* out_boxes, float* out_probs, float head_thresh, float* head_score,
-                      int32_t* head_cls, uint8_t* head_mask, float* out_row_ml, float* out_row_negbg, void* workspace,
+// Stage bits of detect_run.
+constexpr int kDetectFilter = 1;   // softmax filter + decode + the per-(image, class) candidate lists
+constexpr int kDetectNms = 2;      // per-class NMS of the lists the filter left in the workspace
+
+// The core of ssdg_detect, ssdg_detect_stage and ssdg_nms.  scores: logits (DetectMode::kLogits, with pred_box, priors
+// and the optional side outputs) or probabilities (kProbs: prior_dtype is SSDG_F32 and pred_box, priors, out_probs,
+// head_* and the row statistics are NULL, so their checks pass).  boxes: the decoded boxes the NMS reads -- for logits an optional output of the
+// filter (NULL: they stay in the workspace), for probabilities the caller's input (only read).
+static int detect_run(DetectMode mode, int stages, const float* scores, const float* pred_box, const void* priors,
+                      int32_t prior_dtype, int64_t batch, int32_t n_priors, int32_t n_classes, float score_thresh,
+                      int32_t top_k, float iou_thresh, int32_t* out_kept, int32_t* out_count, float* out_kept_score,
+                      float* boxes, float* out_probs, float head_thresh, float* head_score, int32_t* head_cls,
+                      uint8_t* head_mask, float* out_row_ml, float* out_row_negbg, void* workspace,
                       size_t workspace_bytes, void* stream) {
   if ((out_row_ml == nullptr) != (out_row_negbg == nullptr)) return SSDG_ERR_ARG;
   if (((uintptr_t)out_row_ml & 7) || ((uintptr_t)out_row_negbg & 3)) return SSDG_ERR_ALIGN;
-  if (!pred_cls || !pred_box || !priors || !out_kept || !out_count) return SSDG_ERR_ARG;
+  if (!scores || !out_kept || !out_count) return SSDG_ERR_ARG;
+  if (mode == DetectMode::kLogits ? (!pred_box || !priors) : !boxes) return SSDG_ERR_ARG;
   if (batch <= 0 || n_priors <= 0 || n_classes < 2 || top_k <= 0) return SSDG_ERR_ARG;
   if (prior_dtype != SSDG_F32 && prior_dtype != SSDG_F64) return SSDG_ERR_ARG;
   if (top_k > 1024 || batch > 0x7fffffff / 64 || n_priors >= (1 << kABitsD) || n_classes > 2048) return SSDG_ERR_LIMIT;
-  if (((uintptr_t)pred_box | (uintptr_t)priors | (uintptr_t)out_boxes) & 15) return SSDG_ERR_ALIGN;
-  if (((uintptr_t)pred_cls | (uintptr_t)out_probs) & 3) return SSDG_ERR_ALIGN;
+  if (((uintptr_t)pred_box | (uintptr_t)priors | (uintptr_t)boxes) & 15) return SSDG_ERR_ALIGN;
+  if (((uintptr_t)scores | (uintptr_t)out_probs) & 3) return SSDG_ERR_ALIGN;
   if (!workspace || ((uintptr_t)workspace & 255) ||
       workspace_bytes < ssdg_detect_workspace_bytes(batch, n_priors, n_classes, top_k))
     return SSDG_ERR_WORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
   DetectWs ws;
   detect_ws_layout(batch, n_priors, n_classes, &ws, (unsigned char*)workspace);
-  DetectParams P;
-  fill_params(P, ws, batch, n_priors, n_classes);
-  P.pred_cls = pred_cls; P.pred_box = pred_box; P.priors = priors; P.score_thresh = score_thresh;
-  P.boxes = out_boxes ? out_boxes : ws.boxes; P.probs = out_probs;
+  DetectParams P{};
+  P.pred_cls = scores; P.pred_box = pred_box; P.priors = priors;
+  P.B = (int)batch; P.A = n_priors; P.C = n_classes; P.tpi = (n_priors + 31) / 32;
+  P.score_thresh = score_thresh;
+  P.lists = ws.lists; P.run_cnt = ws.run_cnt; P.list_cap = (size_t)P.tpi * 32;
+  P.boxes = boxes ? boxes : ws.boxes; P.probs = out_probs;
   P.head_thresh = head_thresh; P.head_score = head_score; P.head_cls = head_cls; P.head_mask = head_mask;
   P.row_ml = reinterpret_cast<float2*>(out_row_ml); P.row_negbg = out_row_negbg;
-  if (stages & 1) {
-    const int rc = run_filter<false>(P, prior_dtype, st);
+  if (stages & kDetectFilter) {
+    const int rc = run_filter(P, mode, prior_dtype, st);
     if (rc) return rc;
   }
-  if (stages & 2)
+  if (stages & kDetectNms)
     return run_nms(ws, P.boxes, batch, n_priors, n_classes, top_k, iou_thresh, out_kept, out_count, out_kept_score, st);
   return SSDG_OK;
 }
@@ -1416,9 +1424,10 @@ extern "C" int ssdg_detect(const float* pred_cls, const float* pred_box, const v
                            float* out_boxes, float* out_probs, float head_thresh, float* head_score,
                            int32_t* head_cls, uint8_t* head_mask, void* workspace, size_t workspace_bytes,
                            void* stream) {
-  return detect_run(3, pred_cls, pred_box, priors, prior_dtype, batch, n_priors, n_classes, score_thresh, top_k,
-                    iou_thresh, out_kept, out_count, out_kept_score, out_boxes, out_probs, head_thresh, head_score,
-                    head_cls, head_mask, nullptr, nullptr, workspace, workspace_bytes, stream);
+  return detect_run(DetectMode::kLogits, kDetectFilter | kDetectNms, pred_cls, pred_box, priors, prior_dtype, batch,
+                    n_priors, n_classes, score_thresh, top_k, iou_thresh, out_kept, out_count, out_kept_score,
+                    out_boxes, out_probs, head_thresh, head_score, head_cls, head_mask, nullptr, nullptr, workspace,
+                    workspace_bytes, stream);
 }
 
 extern "C" int ssdg_detect_stage(int32_t stage, const float* pred_cls, const float* pred_box, const void* priors,
@@ -1429,34 +1438,19 @@ extern "C" int ssdg_detect_stage(int32_t stage, const float* pred_cls, const flo
                                  float* out_row_ml, float* out_row_negbg, void* workspace, size_t workspace_bytes,
                                  void* stream) {
   if (stage != 0 && stage != 1) return SSDG_ERR_ARG;
-  return detect_run(1 << stage, pred_cls, pred_box, priors, prior_dtype, batch, n_priors, n_classes, score_thresh,
-                    top_k, iou_thresh, out_kept, out_count, out_kept_score, out_boxes, out_probs, head_thresh,
-                    head_score, head_cls, head_mask, out_row_ml, out_row_negbg, workspace, workspace_bytes, stream);
+  return detect_run(DetectMode::kLogits, stage == 0 ? kDetectFilter : kDetectNms, pred_cls, pred_box, priors,
+                    prior_dtype, batch, n_priors, n_classes, score_thresh, top_k, iou_thresh, out_kept, out_count,
+                    out_kept_score, out_boxes, out_probs, head_thresh, head_score, head_cls, head_mask, out_row_ml,
+                    out_row_negbg, workspace, workspace_bytes, stream);
 }
 
 extern "C" int ssdg_nms(const float* probs, const float* boxes, int64_t batch, int32_t n_priors, int32_t n_classes,
                         float score_thresh, int32_t top_k, float iou_thresh, int32_t* out_kept, int32_t* out_count,
                         float* out_kept_score, void* workspace, size_t workspace_bytes, void* stream) {
-  if (!probs || !boxes || !out_kept || !out_count) return SSDG_ERR_ARG;
-  if (batch <= 0 || n_priors <= 0 || n_classes < 2 || top_k <= 0) return SSDG_ERR_ARG;
-  if (top_k > 1024 || batch > 0x7fffffff / 64 || n_priors >= (1 << kABitsD) || n_classes > 2048) return SSDG_ERR_LIMIT;
-  if ((uintptr_t)boxes & 15) return SSDG_ERR_ALIGN;
-  if ((uintptr_t)probs & 3) return SSDG_ERR_ALIGN;
-  if (!workspace || ((uintptr_t)workspace & 255) ||
-      workspace_bytes < ssdg_detect_workspace_bytes(batch, n_priors, n_classes, top_k))
-    return SSDG_ERR_WORKSPACE;
-  cudaStream_t st = (cudaStream_t)stream;
-  DetectWs ws;
-  detect_ws_layout(batch, n_priors, n_classes, &ws, (unsigned char*)workspace);
-  DetectParams P;
-  fill_params(P, ws, batch, n_priors, n_classes);
-  P.pred_cls = probs; P.pred_box = nullptr; P.priors = nullptr; P.score_thresh = score_thresh;
-  P.boxes = nullptr; P.probs = nullptr;
-  P.head_thresh = 0.f; P.head_score = nullptr; P.head_cls = nullptr; P.head_mask = nullptr;
-  P.row_ml = nullptr; P.row_negbg = nullptr;
-  int rc = run_filter<true>(P, SSDG_F32, st);
-  if (rc) return rc;
-  return run_nms(ws, boxes, batch, n_priors, n_classes, top_k, iou_thresh, out_kept, out_count, out_kept_score, st);
+  return detect_run(DetectMode::kProbs, kDetectFilter | kDetectNms, probs, nullptr, nullptr, SSDG_F32, batch, n_priors,
+                    n_classes, score_thresh, top_k, iou_thresh, out_kept, out_count, out_kept_score,
+                    const_cast<float*>(boxes), nullptr, 0.f, nullptr, nullptr, nullptr, nullptr, nullptr, workspace,
+                    workspace_bytes, stream);
 }
 
 extern "C" int ssdg_detect_keep_top_k(const int32_t* kept, const int32_t* count, const float* kept_score, int32_t top_k,

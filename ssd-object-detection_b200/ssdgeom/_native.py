@@ -24,7 +24,7 @@ LOSS_SUM_POS_CE, LOSS_SUM_NEG_CE, LOSS_SUM_L1 = 8, 9, 10
 LOSS_OWN_POS, LOSS_ERRORS = 11, 12     # this shard's own positives; its data-dependent error count
 LOSS_ADDITIVE = slice(LOSS_NUM_POS, LOSS_OWN_POS)   # [4, 11): summed over the shards with per-shard mining
 PROF_MATCH, PROF_CE, PROF_FILTER, PROF_NMS = 0, 1, 2, 3
-PROF_BUCKET, PROF_SEARCH, PROF_LOSS_TAIL, PROF_GRAD = 4, 5, 6, 7
+PROF_SEARCH, PROF_LOSS_TAIL, PROF_GRAD = 5, 6, 7
 
 _vp, _i32, _i64, _f32, _f64, _sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double, C.c_size_t
 _pi32, _pf64 = C.POINTER(C.c_int32), C.POINTER(C.c_double)

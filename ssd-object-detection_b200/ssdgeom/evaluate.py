@@ -63,15 +63,12 @@ class DetectionEvaluator:
     def add(self, detect_out: dict, gt_boxes, gt_cls, gt_off, image_base=None, stream=None, max_gt=None) -> int:
         """Enqueue the matching of one batch (``ops.detect`` outputs with ``kept_score`` and ``boxes``) on ``stream``.
         image_base None continues after the highest image added so far.  Returns the batch's image_base."""
-        for k in ("kept", "count", "kept_score", "boxes"):
-            if k not in detect_out:
-                raise ValueError("detect output lacks %r: call ops.detect(..., want_scores=True, want_boxes=True)" % k)
-        b = int(detect_out["kept"].shape[0])
         base = self.next_image if image_base is None else int(image_base)
         if max_gt is None:
             max_gt = self.max_gt if D.is_device(gt_off) else max(int(np.max(np.diff(np.asarray(gt_off)), initial=0)), 0)
-        ops.eval_accumulate(detect_out, gt_boxes, gt_cls, gt_off, self.state, self.iou_thresholds, base, max_gt, stream)
-        self.next_image = max(self.next_image, base + b)
+        kept = ops.eval_accumulate(detect_out, gt_boxes, gt_cls, gt_off, self.state, self.iou_thresholds, base, max_gt,
+                                   stream)[0]     # the kept lists as a device array [B,C-1,top_k]
+        self.next_image = max(self.next_image, base + kept.shape[0])
         return base
 
     def exchange_buffers(self) -> list:

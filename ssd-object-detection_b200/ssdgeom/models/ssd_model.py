@@ -99,9 +99,7 @@ def detections(pred_conf, pred_bbox, prior_box, score_thresh=0.01, top_k=200, io
 
 def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45):
     """Per-class NMS on given probabilities f32[b,A,C] and decoded boxes f32[b,A,4]."""
-    out = ops.nms(np.ascontiguousarray(np.asarray(probs, dtype=np.float32)) if not D.is_device(probs) else probs,
-                  np.ascontiguousarray(np.asarray(boxes, dtype=np.float32)) if not D.is_device(boxes) else boxes,
-                  score_thresh, top_k, iou_thresh)
+    out = ops.nms(probs, boxes, score_thresh, top_k, iou_thresh)
     return out["kept"].to_host(), out["count"].to_host()
 
 
@@ -151,12 +149,9 @@ def evaluate_detections(kept, count, kept_score, boxes, gt_boxes, gt_cls, gt_off
     the decoded boxes) against CSR ground truth (relative cxcywh, class ids as float32), evaluated on the device.
     Returns {"AP", "AP50", "AP75", "AR", "per_class_AP", "precision", "recall", "n_gt", "n_det"}."""
     from ..evaluate import DetectionEvaluator
-    kept = np.ascontiguousarray(kept, np.int32)
-    b, k, _ = kept.shape
+    b, k, _ = np.shape(kept)
     ev = DetectionEvaluator(n_classes=k + 1, max_images=b, max_dets=max_dets, iou_thresholds=iou_thresholds,
                             recall_thresholds=recall_thresholds)
-    det = {"kept": kept, "count": np.ascontiguousarray(count, np.int32),
-           "kept_score": np.ascontiguousarray(kept_score, np.float32), "boxes": np.ascontiguousarray(boxes, np.float32)}
-    ev.add(det, np.ascontiguousarray(gt_boxes, np.float32), np.ascontiguousarray(gt_cls, np.float32),
-           np.ascontiguousarray(gt_offsets, np.int32), image_base=0)
+    ev.add({"kept": kept, "count": count, "kept_score": kept_score, "boxes": boxes}, gt_boxes, gt_cls, gt_offsets,
+           image_base=0)
     return ev.summarize()

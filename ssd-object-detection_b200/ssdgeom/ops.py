@@ -50,6 +50,19 @@ def _p(x):
     return None if x is None else x.ptr
 
 
+def _outputs(out, spec: dict) -> dict:
+    """The output dict of a call: the caller's ``out`` entries, device-interface objects (torch CUDA tensors etc.) as
+    zero-copy views, plus a new array for every key of ``spec`` {key: (shape, dtype)} the caller did not supply."""
+    out = dict(out or {})
+    for key, v in out.items():
+        if not isinstance(v, D.DeviceArray) and D.is_device(v):
+            out[key] = D.as_device(v)
+    for key, (shape, dtype) in spec.items():
+        if key not in out:            # never dict.setdefault here: it would allocate (and free) eagerly
+            out[key] = D.empty(shape, dtype)
+    return out
+
+
 # ---- A1 ------------------------------------------------------------------------------------------
 def prior_boxes(size_list, s_k_refer, aspect_ratio, input_size=300, stream=None, clip=False) -> D.DeviceArray:
     """models/ssd_model.py:173-194 with the tables lifted to arguments; float64 [A,4] on the device.
@@ -128,12 +141,9 @@ def match_encode(gt_boxes, gt_cls, gt_offsets, priors, batch: int, max_gt: int, 
     gt_cls = D.as_device(gt_cls, np.float32)
     gt_offsets = D.as_device(gt_offsets, np.int32)
     a = int(priors.shape[0])
-    out = dict(out or {})
     spec = {"cls": ((batch, a), np.int32), "box": ((batch, a, 4), np.float32), "loc": ((batch, a, 4), np.float32),
             "mask": ((batch, a), np.uint8), "match": ((batch, a), np.int32)}
-    for k in want:
-        if k not in out:
-            out[k] = D.empty(*spec[k])
+    out = _outputs(out, {k: spec[k] for k in want})
     lib = N.lib()
     nbytes = lib.ssdg_match_workspace_bytes(batch, a, max_gt)
     ws = (pool or POOL).get("match", nbytes)
@@ -253,18 +263,14 @@ def _loss_operands(gt_cls, gt_box, gt_mask, pred_box, pred_cls, want_neg_mask, w
     # models/ssd_model.py:347-351
     if not (gt_cls.size == b * a and gt_mask.size == b * a and gt_box.size == b * a * 4 and pred_box.size == b * a * 4):
         raise AssertionError("y_true / y_pred disagree in shape")
-    out = {k: (D.as_device(v) if D.is_device(v) else v) for k, v in (out or {}).items()}   # torch tensors etc.: zero-copy views
-    if "result" not in out:
-        out["result"] = D.empty((N.LOSS_RESULT_LEN,), np.float64)
-    if want_neg_mask and "neg_mask" not in out:
-        out["neg_mask"] = D.empty((b, a), np.uint8)
-    if want_neg_ce and "neg_ce" not in out:
-        out["neg_ce"] = D.empty((b, a), np.float32)
+    spec = {"result": ((N.LOSS_RESULT_LEN,), np.float64)}
+    if want_neg_mask:
+        spec["neg_mask"] = ((b, a), np.uint8)
+    if want_neg_ce:
+        spec["neg_ce"] = ((b, a), np.float32)
     if want_grad:
-        if "grad_box" not in out:
-            out["grad_box"] = D.empty((b, a, 4), np.float32)
-        if "grad_cls" not in out:
-            out["grad_cls"] = D.empty((b, a, c), np.float32)
+        spec.update(grad_box=((b, a, 4), np.float32), grad_cls=((b, a, c), np.float32))
+    out = _outputs(out, spec)
     ws = pool.get(ws_kind, N.lib().ssdg_loss_workspace_bytes(b, a, c))
     return (gt_cls, gt_box, gt_mask, pred_box, pred_cls), out, ws
 
@@ -398,6 +404,16 @@ def loss_result_to_host(result: D.DeviceArray, stream=None) -> dict:
 
 
 # ---- A7 + A8 + A9 ---------------------------------------------------------------------------------------
+def _detect_outputs(out, pool, b, a, c, top_k, want_scores, spec) -> tuple:
+    """Output dict and workspace of ``detect`` / ``nms``: the kept lists, their counts, the kept scores when wanted and
+    the outputs of ``spec``."""
+    spec = dict(spec, kept=((b, c - 1, top_k), np.int32), count=((b, c - 1), np.int32))
+    if want_scores:
+        spec["kept_score"] = ((b, c - 1, top_k), np.float32)
+    ws = (pool or POOL).get("detect", N.lib().ssdg_detect_workspace_bytes(b, a, c, top_k))
+    return _outputs(out, spec), ws
+
+
 def detect(pred_cls, pred_box, priors, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores=False,
            want_boxes=False, want_probs=False, head_thresh=None, out=None, stream=None, stage=None,
            want_row_stats=False, pool=None) -> dict:
@@ -409,29 +425,17 @@ def detect(pred_cls, pred_box, priors, score_thresh=0.01, top_k=200, iou_thresh=
     b, a, c = pred_cls.shape
     if pred_box.size != b * a * 4 or priors.shape[0] != a:
         raise AssertionError("pred_cls / pred_box / priors disagree in shape")
-    out = dict(out or {})
-
-    def need(key, shape, dtype):
-        if key not in out:            # never dict.setdefault here: it would allocate (and free) eagerly
-            out[key] = D.empty(shape, dtype)
-
-    need("kept", (b, c - 1, top_k), np.int32)
-    need("count", (b, c - 1), np.int32)
-    if want_scores:
-        need("kept_score", (b, c - 1, top_k), np.float32)
+    spec = {}
     if want_boxes:
-        need("boxes", (b, a, 4), np.float32)
+        spec["boxes"] = ((b, a, 4), np.float32)
     if want_probs:
-        need("probs", (b, a, c), np.float32)
+        spec["probs"] = ((b, a, c), np.float32)
     if want_row_stats:           # per-prior softmax statistics for multibox_loss(row_stats=...)
-        need("row_ml", (b, a, 2), np.float32)
-        need("row_negbg", (b, a), np.float32)
+        spec.update(row_ml=((b, a, 2), np.float32), row_negbg=((b, a), np.float32))
     if head_thresh is not None:
-        need("head_score", (b, a), np.float32)
-        need("head_cls", (b, a), np.int32)
-        need("head_mask", (b, a), np.uint8)
+        spec.update(head_score=((b, a), np.float32), head_cls=((b, a), np.int32), head_mask=((b, a), np.uint8))
+    out, ws = _detect_outputs(out, pool, b, a, c, top_k, want_scores, spec)
     lib = N.lib()
-    ws = (pool or POOL).get("detect", lib.ssdg_detect_workspace_bytes(b, a, c, top_k))
     args = (pred_cls.ptr, pred_box.ptr, priors.ptr, _code(priors.dtype), b, a, c, float(score_thresh),
             int(top_k), float(iou_thresh), out["kept"].ptr, out["count"].ptr, _p(out.get("kept_score")),
             _p(out.get("boxes")), _p(out.get("probs")),
@@ -448,17 +452,16 @@ def detect(pred_cls, pred_box, priors, score_thresh=0.01, top_k=200, iou_thresh=
     return out
 
 
-def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores=False, stream=None) -> dict:
+def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores=False, stream=None, out=None) -> dict:
+    """Per-class NMS on given probabilities f32[B,A,C] and decoded boxes f32[B,A,4] (ssdg_nms): the ``detect``
+    outputs kept, count and, when wanted, kept_score.  ``out`` may carry preallocated arrays."""
     probs = D.as_device(probs, np.float32)
     boxes = D.as_device(boxes, np.float32)
     b, a, c = probs.shape
     if boxes.size != b * a * 4:
         raise AssertionError("probs / boxes disagree in shape")
-    out = {"kept": D.empty((b, c - 1, top_k), np.int32), "count": D.empty((b, c - 1), np.int32)}
-    if want_scores:
-        out["kept_score"] = D.empty((b, c - 1, top_k), np.float32)
+    out, ws = _detect_outputs(out, None, b, a, c, top_k, want_scores, {})
     lib = N.lib()
-    ws = POOL.get("detect", lib.ssdg_detect_workspace_bytes(b, a, c, top_k))
     N.check(lib.ssdg_nms(probs.ptr, boxes.ptr, b, a, c, float(score_thresh), int(top_k), float(iou_thresh),
                          out["kept"].ptr, out["count"].ptr, _p(out.get("kept_score")), ws.ptr, ws.nbytes,
                          D.stream_handle(stream)), "nms")
@@ -467,32 +470,38 @@ def nms(probs, boxes, score_thresh=0.01, top_k=200, iou_thresh=0.45, want_scores
 
 
 # ---- A12 ------------------------------------------------------------------------------------------------
+def _kept_lists(det: dict, need_boxes: bool, stream=None) -> tuple:
+    """(kept i32[B,C-1,top_k], count i32[B,C-1], kept_score f32[B,C-1,top_k], boxes f32[B,A,4]) of a ``detect`` /
+    ``nms`` output as device arrays; boxes is None when ``det`` has none and ``need_boxes`` is false."""
+    flags = "want_scores=True, want_boxes=True" if need_boxes else "want_scores=True"
+    for key in ("kept", "count", "kept_score", "boxes") if need_boxes else ("kept", "count", "kept_score"):
+        if det.get(key) is None:
+            raise ValueError("detect output lacks %r: call ops.detect(..., %s)" % (key, flags))
+    kept, count = D.as_device(det["kept"], np.int32, stream), D.as_device(det["count"], np.int32, stream)
+    kept_score = D.as_device(det["kept_score"], np.float32, stream)
+    boxes = D.as_device(det["boxes"], np.float32, stream) if det.get("boxes") is not None else None
+    if len(kept.shape) != 3 or (boxes is not None and len(boxes.shape) != 3):
+        raise AssertionError("kept must be [B,C-1,top_k] and boxes [B,A,4]")
+    b, k, _ = kept.shape
+    if count.size != b * k or kept_score.size != kept.size or (boxes is not None and boxes.shape[0] != b):
+        raise AssertionError("kept, count, kept_score and boxes disagree in shape")
+    return kept, count, kept_score, boxes
+
+
 def keep_top_k(det: dict, keep_top_k: int, out=None, stream=None) -> dict:
     """The final detections of every image (include/ssdgeom.h, ssdg_detect_keep_top_k): the kept lists of a ``detect``
     / ``nms`` output with ``kept_score`` ranked across classes (score desc, class asc, position asc) and capped at
     ``keep_top_k``.  Returns device arrays prior i32[B,K], class i32[B,K], score f32[B,K], n i32[B] and count
     i32[B,C-1] (the survivors per class list, a prefix of each: ``dict(det, count=top["count"])`` is a capped
     detection output), plus box f32[B,K,4] when ``det`` has ``boxes``.  ``out`` may carry preallocated arrays."""
-    if "kept_score" not in det:
-        raise ValueError("detect output lacks 'kept_score': call ops.detect(..., want_scores=True)")
-    kept, count = D.as_device(det["kept"], np.int32, stream), D.as_device(det["count"], np.int32, stream)
-    kept_score = D.as_device(det["kept_score"], np.float32, stream)
-    boxes = D.as_device(det["boxes"], np.float32, stream) if det.get("boxes") is not None else None
-    if len(kept.shape) != 3:
-        raise AssertionError("kept must be [B,C-1,top_k]")
+    kept, count, kept_score, boxes = _kept_lists(det, False, stream)
     b, k, top_k = kept.shape
-    if count.size != b * k or kept_score.size != kept.size or (boxes is not None and
-                                                               (len(boxes.shape) != 3 or boxes.shape[0] != b)):
-        raise AssertionError("kept, count, kept_score and boxes disagree in shape")
     kk = int(keep_top_k)
-    out = dict(out or {})
     spec = {"prior": ((b, kk), np.int32), "class": ((b, kk), np.int32), "score": ((b, kk), np.float32),
             "n": ((b,), np.int32), "count": ((b, k), np.int32)}
     if boxes is not None:
         spec["box"] = ((b, kk, 4), np.float32)
-    for key, (shape, dt) in spec.items():
-        if key not in out:
-            out[key] = D.empty(shape, dt)
+    out = _outputs(out, spec)
     a = int(boxes.shape[1]) if boxes is not None else 0
     N.check(N.lib().ssdg_detect_keep_top_k(kept.ptr, count.ptr, kept_score.ptr, top_k, _p(boxes), b, a, k + 1, kk,
                                            out["prior"].ptr, out["class"].ptr, out["score"].ptr, _p(out.get("box")),
@@ -532,16 +541,11 @@ def eval_accumulate(det: dict, gt_boxes, gt_cls, gt_offsets, state: EvalState, i
                     max_gt: int, stream=None):
     """Match one batch of ``detect`` outputs (``kept``, ``count``, ``kept_score``, ``boxes``) to its ground truth
     (CSR, as ``match_encode``) and write the slots of global images ``image_base ..`` (ssdg_eval_accumulate)."""
-    kept, count = D.as_device(det["kept"], np.int32, stream), D.as_device(det["count"], np.int32, stream)
-    kept_score = D.as_device(det["kept_score"], np.float32, stream)
-    boxes = D.as_device(det["boxes"], np.float32, stream)
+    kept, count, kept_score, boxes = _kept_lists(det, True, stream)
     gt_boxes, gt_cls = D.as_device(gt_boxes, np.float32, stream), D.as_device(gt_cls, np.float32, stream)
     gt_offsets = D.as_device(gt_offsets, np.int32, stream)
-    if len(kept.shape) != 3 or len(boxes.shape) != 3:
-        raise AssertionError("kept must be [B,C-1,top_k] and boxes [B,A,4]")
     b, k, top_k = kept.shape
-    if k + 1 != state.n_classes or count.size != b * k or kept_score.size != kept.size or boxes.shape[0] != b \
-            or gt_offsets.size != b + 1:
+    if k + 1 != state.n_classes or gt_offsets.size != b + 1:
         raise AssertionError("detections, ground truth and evaluation state disagree in shape")
     thr = np.ascontiguousarray(iou_thresholds, np.float64)
     if thr.size != state.n_thresholds:
@@ -576,8 +580,8 @@ def eval_finalize(state: EvalState, recall_thresholds, stream=None, pool=None) -
     n_gt i64[K], n_det i64[K].  The state is left unchanged."""
     rec = np.ascontiguousarray(recall_thresholds, np.float64)
     k, t, r = state.n_classes - 1, state.n_thresholds, rec.size
-    out = {"precision": D.empty((t, r, k), np.float64), "recall": D.empty((t, k), np.float64),
-           "n_gt": D.empty((k,), np.int64), "n_det": D.empty((k,), np.int64)}
+    out = _outputs(None, {"precision": ((t, r, k), np.float64), "recall": ((t, k), np.float64),
+                          "n_gt": ((k,), np.int64), "n_det": ((k,), np.int64)})
     lib = N.lib()
     nbytes = int(lib.ssdg_eval_finalize_workspace_bytes(state.n_classes, state.max_images, state.max_dets))
     if nbytes == 0:
