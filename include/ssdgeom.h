@@ -430,6 +430,62 @@ SSDG_API int ssdg_detect_keep_top_k(const int32_t* kept, const int32_t* count, c
                                     float* out_score /* [B,K], 0 padded */, float* out_box /* [B,K,4] or NULL, 0 padded */,
                                     int32_t* out_n /* [B] */, int32_t* out_count /* [B,C-1] or NULL */, void* stream);
 
+/* ---- A13: SSD training augmentation ---------------------------------------------------------------------------
+ * The reference's loader only resizes and normalises.  The SSD paper's augmentation of a batch already on the device
+ * (spec: tests/augment_oracle.py; PARITY UNPINNED against torchvision 0.26 like A9, every discrete output bit-exact
+ * against that restatement): torchvision's RandomZoomOut(fill, side_range=(side_lo, side_hi), p=zoom_p) ->
+ * RandomIoUCrop(min_scale, max_scale, min_aspect, max_aspect, min_ious, trials) -> RandomHorizontalFlip(flip_p), then
+ * a bilinear resize back to height x width.  Images float32 [B,H,W,3] (one size for the batch); ground truth as
+ * ssdg_match_encode reads it: boxes float32 [rows,4] relative cxcywh, cls float32 [rows], offsets int32 [B+1].
+ *
+ * Random numbers: Philox4x32-10 (Random123), key = seed, counter = (g lo, g hi, stream, index) with g = image_base + b
+ *   the global image index; a draw is u = (x >> 8) * 2^-24 (float32 in [0,1)).
+ *     stream 0, index 0: zoom gate, zoom r, pad left, pad top      stream 0, index 1: flip gate
+ *     stream 1, index q: the option of crop round q, (x0 * n_options) >> 32
+ *     stream 2+q, index t: trial t of round q (scale w, scale h, left, top)
+ *   Every draw has a fixed address: an image's result depends only on (seed, g, configuration).
+ * Decisions (torchvision's float32 arithmetic where it decides an integer; p, side_lo, min_scale, fl32(side_hi -
+ * side_lo), fl32(max_scale - min_scale) are rounded to float32 as torch does):
+ *   a gate applies iff u < p.  Zoom: r = side_lo + u*(side_hi - side_lo), canvas_w = trunc(W*r), pad_left =
+ *     trunc((canvas_w - W)*u) (float32 products), the same for h / top.
+ *   crop round q: option m = min_ious[...]; m >= 1 means no crop.  Trial t: new_w = trunc(canvas_w * (min_scale +
+ *     u*(max_scale - min_scale))), the same for h; it fails when new_h or new_w is 0 or new_w/new_h (float64) is outside
+ *     [min_aspect, max_aspect]; left = trunc((canvas_w - new_w)*u), top alike.  Rows are tested in float64 from the
+ *     exactly promoted inputs: pixel corners (cx -/+ 0.5w)*W + pad; a row is within iff left < 0.5(x0+x1) < left+new_w
+ *     and the same in y (strict); the trial succeeds iff some within row has !(iou < m), iou by torchvision's box_iou
+ *     formula (a NaN IoU passes, as torch.max propagates it).  The first successful trial by index ends the round.
+ *   Deviations from torchvision: at most max_rounds rounds, then the image is not cropped and its record says so
+ *   (torchvision loops until it draws a 1.0 option); n_options = 0 disables the crop; centres and IoU in float64.
+ * Kept rows: with a crop, the within rows in input order, shifted by (left, top), clamped to [0,new_w] x [0,new_h],
+ *   relative cxcywh of the crop; without one, every row affine-mapped only (not clamped).  A flip maps cx -> 1 - cx.
+ *   Float64, rounded once to float32.  Labels travel with their rows (no SanitizeBoundingBoxes).  Rows are only ever
+ *   dropped, so a max_gt bound of the input bounds the output for ssdg_match_encode.
+ * Outputs of ssdg_augment_boxes (rows = gt_offsets[B]):
+ *   out_boxes float32 [rows,4]  out_cls float32 [rows]  out_offsets int32 [B+1]  (rows past out_offsets[B]: 0)
+ *   out_src_row int32 [rows]    input row of each output row (-1 past out_offsets[B])
+ *   out_transform int32 [B,SSDG_AUG_RECORD]: canvas w, canvas h, pad left, pad top, crop left, top, w, h (the whole
+ *     canvas without a crop), flip, rounds drawn (0 when n_options == 0, -1 when the cap was hit)
+ *   No workspace.  Limits: max_gt <= 2048 (rows beyond it are read from global memory, not an error), n_options <= 16,
+ *   height, width <= 16384, side_hi <= 64.  Argument errors (SSDG_ERR_ARG: nulls, p outside [0,1], 1 <= side_lo <=
+ *   side_hi, 0 <= min_scale <= max_scale <= 1, 0 < min_aspect <= max_aspect, trials >= 1, max_rounds >= 1, a NaN option;
+ *   SSDG_ERR_ALIGN: boxes not 16-byte aligned, other arrays not 4-byte aligned) return before any CUDA call.
+ * ssdg_augment_images: output pixel (i,j) samples the crop [left, left+w) x [top, top+h) of a virtual canvas that is
+ *   fill[c] (host float[3]) except where the image is pasted at (pad left, pad top), bilinear with align_corners=False
+ *   and no antialiasing (F.interpolate's source x = max(0, (j+0.5)*(w/W) - 0.5) in float32, upper neighbour clamped to
+ *   w-1); a flip reads column W-1-j.  It reads only the record, so a record can be replayed.  images and out_images
+ *   must not overlap.
+ */
+#define SSDG_AUG_RECORD 10
+SSDG_API int ssdg_augment_boxes(const float* gt_boxes, const float* gt_cls, const int32_t* gt_offsets, int32_t batch,
+                                int32_t max_gt, int32_t height, int32_t width, uint64_t seed, int64_t image_base,
+                                double zoom_p, double side_lo, double side_hi, const double* min_ious /* host */,
+                                int32_t n_options, double min_scale, double max_scale, double min_aspect,
+                                double max_aspect, int32_t trials, int32_t max_rounds, double flip_p, float* out_boxes,
+                                float* out_cls, int32_t* out_offsets, int32_t* out_src_row, int32_t* out_transform,
+                                void* stream);
+SSDG_API int ssdg_augment_images(const float* images, const int32_t* transform, int32_t batch, int32_t height,
+                                 int32_t width, const float* fill /* host float[3] */, float* out_images, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -33,6 +33,7 @@ UNITS = {
     "detect.cu": [],
     "comm.cu": [],
     "eval.cu": ["-fmad=false"],
+    "augment.cu": ["-fmad=false"],
 }
 
 

@@ -16,6 +16,7 @@ ERR_NO_NCCL, ERR_LABEL_RANGE, ERR_STALE_INDEX = -11, -12, -13
 ERR_NCCL_BASE = 10000
 F32, F64, I32, I64 = 0, 1, 2, 3
 COMM_ID_BYTES = 128
+AUG_RECORD = 10
 LOSS_RESULT_LEN = 16
 # words of the loss result block (include/ssdgeom.h, out_result)
 LOSS_TOTAL, LOSS_POS, LOSS_NEG, LOSS_LOC = 0, 1, 2, 3     # total, "cls loss pos", "cls loss neg", "loc loss"
@@ -87,6 +88,9 @@ PROTOTYPES = {
     "ssdg_nms": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _f32, _i32, _f32, _vp, _vp, _vp, _vp, _sz, _vp]),
     "ssdg_detect_keep_top_k": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _i64, _i32, _i32, _i32, _vp, _vp, _vp, _vp, _vp, _vp,
                                          _vp]),
+    "ssdg_augment_boxes": (C.c_int, [_vp, _vp, _vp, _i32, _i32, _i32, _i32, C.c_uint64, _i64, _f64, _f64, _f64, _pf64,
+                                     _i32, _f64, _f64, _f64, _f64, _i32, _i32, _f64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "ssdg_augment_images": (C.c_int, [_vp, _vp, _i32, _i32, _i32, C.POINTER(_f32), _vp, _vp]),
     "ssdg_eval_state_bytes": (_sz, [_i32, _i64, _i32, _i32]),
     "ssdg_eval_reset": (C.c_int, [_vp, _sz, _vp]),
     "ssdg_eval_accumulate": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _i32, _i32, _i32, _vp, _vp, _vp, _i32, _pf64, _i32,

@@ -57,16 +57,24 @@ class TrainBatches:
 
     ``prefetch`` mirrors ``.prefetch(10)`` (:225): a producer thread packs, assigns and downloads up to that many
     batches ahead of the consumer on a stream of its own (the library releases the GIL inside its calls), so the
-    assignment of batch k+1 overlaps whatever the training step does with batch k.  ``prefetch=0`` is synchronous."""
+    assignment of batch k+1 overlaps whatever the training step does with batch k.  ``prefetch=0`` is synchronous.
+
+    ``augment``: None, or a dict of ``ops.augment`` options (``seed`` among them, default 0) to apply the SSD training
+    augmentation (zoom-out, min-IoU crop, flip) to every batch on the device: images and boxes are uploaded,
+    (``gt_prepare``), augmented, normalised and matched.  Image ``k`` emitted by this iterator draws its random numbers
+    at global index ``image_base + k``; give each data-parallel rank its own ``image_base`` range."""
 
     def __init__(self, source, priors, batch_size=1, thresh=0.5, coco_pixels=False, device=False, stream=None,
-                 prefetch=10):
+                 prefetch=10, augment=None, image_base=0):
         self.source, self.batch_size, self.thresh = source, int(batch_size), float(thresh)
         self.priors = D.as_device(priors)
         ops.prior_index(self.priors)
         self.coco_pixels, self.device, self.stream = bool(coco_pixels), bool(device), stream
         self.prefetch = int(prefetch)
         self.pool = ops.WorkspacePool()      # this iterator's own matcher scratch (its calls are in stream order)
+        self.augment = None if augment is None else dict(augment)
+        self.seed = self.augment.pop("seed", 0) if augment is not None else None
+        self.image_base = int(image_base)
 
     def _emit(self, images, cls_list, box_list, wh):
         cls, boxes, off = pack_gt(cls_list, box_list)
@@ -76,9 +84,18 @@ class TrainBatches:
         else:
             d_boxes = D.as_device(boxes.astype(np.float32, copy=False), np.float32)
         max_gt = int(np.diff(off).max()) if b else 0
+        img = np.stack(images).astype(np.float32, copy=False)
+        if self.augment is not None:
+            # rows are only dropped, so max_gt still bounds every image of the augmented batch
+            aug = ops.augment(img, d_boxes, cls, off, self.seed, self.image_base, max_gt=max_gt, stream=self.stream,
+                              **self.augment)
+            self.image_base += b
+            img = ops.image_normalize(aug["images"], stream=self.stream)
+            d_boxes, cls, off = aug["boxes"], aug["cls"], aug["offsets"]
         tgt = ops.match_encode(d_boxes, cls, off, self.priors, b, max(max_gt, 1), self.thresh, stream=self.stream,
                                pool=self.pool)
-        img = ops.image_normalize(np.stack(images).astype(np.float32, copy=False), stream=self.stream)
+        if self.augment is None:
+            img = ops.image_normalize(img, stream=self.stream)
         if self.device:
             ops.raise_for_match_status(ops.match_status(tgt, self.stream))      # synchronises: the batch is ready
             return img, (tgt["cls"], tgt["loc"], tgt["mask"])

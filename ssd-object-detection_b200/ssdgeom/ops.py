@@ -510,6 +510,74 @@ def keep_top_k(det: dict, keep_top_k: int, out=None, stream=None) -> dict:
     return out
 
 
+# ---- A13 ------------------------------------------------------------------------------------------------
+# torchvision's SSD recipe: RandomZoomOut(fill, side_range=(1, 4), p=0.5) -> RandomIoUCrop() -> RandomHorizontalFlip(0.5),
+# filled with the SSD mean
+AUGMENT_DEFAULTS = dict(zoom_p=0.5, side_range=(1.0, 4.0), min_ious=(0.0, 0.1, 0.3, 0.5, 0.7, 0.9, 1.0), min_scale=0.3,
+                        max_scale=1.0, min_aspect=0.5, max_aspect=2.0, trials=40, max_rounds=50, flip_p=0.5,
+                        fill=(123 / 255, 117 / 255, 104 / 255))
+
+
+def augment(images, gt_boxes, gt_cls, gt_offsets, seed: int, image_base: int = 0, max_gt=None, out=None, stream=None,
+            **config) -> dict:
+    """SSD training augmentation of a batch (include/ssdgeom.h, A13): zoom-out, min-IoU crop and horizontal flip of
+    images f32[B,H,W,3] and their ground truth (CSR as ``match_encode`` reads it), then a bilinear resize back to H x W.
+    ``config`` overrides ``AUGMENT_DEFAULTS``.  Image ``b`` draws its random numbers at global index
+    ``image_base + b`` from ``seed``.  ``max_gt`` bounds the rows of any image (taken from host offsets when omitted).
+    Returns device arrays images f32[B,H,W,3], boxes f32[rows,4], cls f32[rows], offsets i32[B+1], src_row i32[rows]
+    and transform i32[B,10] (one record per image; ``augment_images`` replays it).  ``out`` may carry preallocated
+    arrays."""
+    unknown = set(config) - set(AUGMENT_DEFAULTS)
+    if unknown:
+        raise TypeError("unknown augmentation options: %s" % sorted(unknown))
+    cfg = dict(AUGMENT_DEFAULTS, **config)
+    if max_gt is None:
+        if D.is_device(gt_offsets):
+            raise ValueError("augment: pass max_gt with device offsets")
+        off = np.asarray(gt_offsets)
+        max_gt = int(np.diff(off).max()) if off.size > 1 else 0
+    images = D.as_device(images, np.float32, stream)
+    gt_boxes, gt_cls = D.as_device(gt_boxes, np.float32, stream), D.as_device(gt_cls, np.float32, stream)
+    gt_offsets = D.as_device(gt_offsets, np.int32, stream)
+    if len(images.shape) != 4 or images.shape[3] != 3:
+        raise AssertionError("images must be [B,H,W,3]")
+    b, h, w, _ = images.shape
+    rows = gt_boxes.size // 4
+    if gt_offsets.size != b + 1 or gt_cls.size != rows or gt_boxes.size != rows * 4:
+        raise AssertionError("images, gt_boxes, gt_cls and gt_offsets disagree in shape")
+    out = _outputs(out, {"images": ((b, h, w, 3), np.float32), "boxes": ((rows, 4), np.float32),
+                         "cls": ((rows,), np.float32), "offsets": ((b + 1,), np.int32), "src_row": ((rows,), np.int32),
+                         "transform": ((b, N.AUG_RECORD), np.int32)})
+    opts = np.ascontiguousarray(cfg["min_ious"], np.float64)
+    lo, hi = (float(v) for v in cfg["side_range"])
+    lib, st = N.lib(), D.stream_handle(stream)
+    N.check(lib.ssdg_augment_boxes(
+        gt_boxes.ptr, gt_cls.ptr, gt_offsets.ptr, b, int(max_gt), h, w, int(seed) & (2**64 - 1), int(image_base),
+        float(cfg["zoom_p"]), lo, hi, opts.ctypes.data_as(C.POINTER(C.c_double)), opts.size, float(cfg["min_scale"]),
+        float(cfg["max_scale"]), float(cfg["min_aspect"]), float(cfg["max_aspect"]), int(cfg["trials"]),
+        int(cfg["max_rounds"]), float(cfg["flip_p"]), out["boxes"].ptr, out["cls"].ptr, out["offsets"].ptr,
+        out["src_row"].ptr, out["transform"].ptr, st), "augment_boxes")
+    augment_images(images, out["transform"], cfg["fill"], out=out["images"], stream=stream)
+    out["_keep"] = (images, gt_boxes, gt_cls, gt_offsets)
+    return out
+
+
+def augment_images(images, transform, fill=AUGMENT_DEFAULTS["fill"], out=None, stream=None) -> D.DeviceArray:
+    """The image half of ``augment``: images f32[B,H,W,3] resampled through transform records i32[B,10]
+    (ssdg_augment_images)."""
+    images = D.as_device(images, np.float32, stream)
+    transform = D.as_device(transform, np.int32, stream)
+    if len(images.shape) != 4 or images.shape[3] != 3 or transform.size != images.shape[0] * N.AUG_RECORD:
+        raise AssertionError("images must be [B,H,W,3] and transform [B,%d]" % N.AUG_RECORD)
+    b, h, w, _ = images.shape
+    out = D.empty(images.shape, np.float32) if out is None else D.as_device(out, np.float32)
+    f = (C.c_float * 3)(*[float(v) for v in fill])
+    N.check(N.lib().ssdg_augment_images(images.ptr, transform.ptr, b, h, w, f, out.ptr, D.stream_handle(stream)),
+            "augment_images")
+    out._keep = (images, transform)
+    return out
+
+
 # ---- A11 ------------------------------------------------------------------------------------------------
 EVAL_STATUS_BAD_CLASS, EVAL_STATUS_TOO_MANY_GT, EVAL_STATUS_DUPLICATE, EVAL_STATUS_BAD_PRIOR = 1, 2, 4, 8
 
