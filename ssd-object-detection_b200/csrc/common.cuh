@@ -143,6 +143,62 @@ __device__ __forceinline__ R iou_corners(const Corners<R>& g, const Corners<R>& 
   return div_rn(inter, den);
 }
 
+// The helpers below are bit-exact only in units compiled with -fmad=false (match.cu, geom.cu): their plain
+// operators must not be contracted into FMA.
+
+// Result dtype of an IoU between a T1 and a T2 box (NumPy promotion): float only when both are float.
+template <typename T1, typename T2>
+struct Promote {
+  typedef double type;
+};
+template <>
+struct Promote<float, float> {
+  typedef float type;
+};
+
+// Row i of a [n,4] float32 / float64 array.
+template <typename T>
+struct Vec4;
+template <>
+struct Vec4<float> {
+  static __device__ __forceinline__ void load(const void* base, long long i, float& a, float& b, float& c,
+                                              float& d) {
+    float4 v = __ldg(reinterpret_cast<const float4*>(base) + i);
+    a = v.x; b = v.y; c = v.z; d = v.w;
+  }
+};
+template <>
+struct Vec4<double> {
+  static __device__ __forceinline__ void load(const void* base, long long i, double& a, double& b, double& c,
+                                              double& d) {
+    const double2* p = reinterpret_cast<const double2*>(base) + 2 * i;
+    double2 u = __ldg(p), v = __ldg(p + 1);
+    a = u.x; b = u.y; c = v.x; d = v.y;
+  }
+};
+
+// Corners of (cx, cy, w, h) row i of a TIn array, computed in TIn and promoted to R.
+template <typename TIn, typename R>
+__device__ __forceinline__ Corners<R> load_corners(const void* base, long long i) {
+  TIn cx, cy, w, h;
+  Vec4<TIn>::load(base, i, cx, cy, w, h);
+  const Corners<TIn> c = corners_of<TIn>(cx, cy, w, h);
+  Corners<R> r;
+  r.x1 = (R)c.x1; r.y1 = (R)c.y1; r.x2 = (R)c.x2; r.y2 = (R)c.y2; r.area = (R)c.area;
+  return r;
+}
+
+// apply_anchor_box (utils/bbox.py:98-99) of box b against prior d in float64; callers cast the result.  The 1e-5
+// clamp is applied in each operand's own dtype (NumPy promotes the Python scalar to the array dtype).
+template <typename TB, typename TP>
+__device__ __forceinline__ double4 anchor_offsets(TB bx, TB by, TB bw, TB bh, TP dx, TP dy, TP dw, TP dh) {
+  const double tx = ((double)bx - (double)dx) / (double)dw;
+  const double ty = ((double)by - (double)dy) / (double)dh;
+  const double rw = (double)max_nn(bw, (TB)1e-5) / (double)max_nn(dw, (TP)1e-5);
+  const double rh = (double)max_nn(bh, (TB)1e-5) / (double)max_nn(dh, (TP)1e-5);
+  return make_double4(tx, ty, log(rw), log(rh));
+}
+
 // ---------------------------------------------------------------------------------------------
 // mbarrier + 1-D bulk TMA (cp.async.bulk, SASS UBLKCP) for streaming contiguous tiles.
 // ---------------------------------------------------------------------------------------------

@@ -32,34 +32,18 @@ __global__ void prior_kernel(const __grid_constant__ PriorTable tab, double* __r
   o[1] = make_double2(tab.shape_w[l][s], tab.shape_h[l][s]);
 }
 
-template <typename T>
-__device__ __forceinline__ void load4(const void* base, long long i, double& a, double& b, double& c, double& d);
-template <>
-__device__ __forceinline__ void load4<float>(const void* base, long long i, double& a, double& b, double& c, double& d) {
-  float4 v = __ldg(reinterpret_cast<const float4*>(base) + i);
-  a = v.x; b = v.y; c = v.z; d = v.w;
-}
-template <>
-__device__ __forceinline__ void load4<double>(const void* base, long long i, double& a, double& b, double& c, double& d) {
-  const double2* p = reinterpret_cast<const double2*>(base) + 2 * i;
-  double2 u = __ldg(p), v = __ldg(p + 1);
-  a = u.x; b = u.y; c = v.x; d = v.y;
-}
-
-// utils/bbox.py:98-99.  The 1e-5 clamp is applied in each operand's own dtype (NumPy promotes
-// the Python scalar to the array dtype).
+// utils/bbox.py:98-99.
 template <typename TB, typename TP, typename TO>
 __global__ void encode_kernel(const void* __restrict__ boxes, const void* __restrict__ priors, TO* __restrict__ out,
                               long long n, int A) {
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  double bx, by, bw, bh, dx, dy, dw, dh;
-  load4<TB>(boxes, i, bx, by, bw, bh);
-  load4<TP>(priors, i % A, dx, dy, dw, dh);
-  const double cb = (double)(TB)1e-5, cp = (double)(TP)1e-5;
-  double tx = (bx - dx) / dw, ty = (by - dy) / dh;
-  double tw = log(fmax(bw, cb) / fmax(dw, cp)), th = log(fmax(bh, cb) / fmax(dh, cp));
-  out[4 * i + 0] = (TO)tx; out[4 * i + 1] = (TO)ty; out[4 * i + 2] = (TO)tw; out[4 * i + 3] = (TO)th;
+  TB bx, by, bw, bh;
+  TP dx, dy, dw, dh;
+  Vec4<TB>::load(boxes, i, bx, by, bw, bh);
+  Vec4<TP>::load(priors, i % A, dx, dy, dw, dh);
+  const double4 t = anchor_offsets<TB, TP>(bx, by, bw, bh, dx, dy, dw, dh);
+  out[4 * i + 0] = (TO)t.x; out[4 * i + 1] = (TO)t.y; out[4 * i + 2] = (TO)t.z; out[4 * i + 3] = (TO)t.w;
 }
 
 // models/ssd_model.py:466-467.
@@ -69,8 +53,8 @@ __global__ void decode_kernel(const float* __restrict__ loc, const void* __restr
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   float4 t = __ldg(reinterpret_cast<const float4*>(loc) + i);
-  double dx, dy, dw, dh;
-  load4<TP>(priors, i % A, dx, dy, dw, dh);
+  TP dx, dy, dw, dh;
+  Vec4<TP>::load(priors, i % A, dx, dy, dw, dh);
   float4 o;
   o.x = (float)(((double)t.x * dw + dx) * scale);
   o.y = (float)(((double)t.y * dh + dy) * scale);
@@ -80,36 +64,13 @@ __global__ void decode_kernel(const float* __restrict__ loc, const void* __restr
 }
 
 template <typename T1, typename T2>
-struct Prom { typedef double type; };
-template <>
-struct Prom<float, float> { typedef float type; };
-
-template <typename T>
-__device__ __forceinline__ Corners<T> load_corners(const void* base, long long i);
-template <>
-__device__ __forceinline__ Corners<float> load_corners<float>(const void* base, long long i) {
-  float4 v = __ldg(reinterpret_cast<const float4*>(base) + i);
-  return corners_of<float>(v.x, v.y, v.z, v.w);
-}
-template <>
-__device__ __forceinline__ Corners<double> load_corners<double>(const void* base, long long i) {
-  const double2* p = reinterpret_cast<const double2*>(base) + 2 * i;
-  double2 u = __ldg(p), v = __ldg(p + 1);
-  return corners_of<double>(u.x, u.y, v.x, v.y);
-}
-
-template <typename T1, typename T2>
 __global__ void iou_pairs_kernel(const void* __restrict__ b1, const void* __restrict__ b2, void* __restrict__ out,
                                  long long n, int use_eps) {
-  typedef typename Prom<T1, T2>::type R;
+  typedef typename Promote<T1, T2>::type R;
   long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
-  Corners<T1> c1 = load_corners<T1>(b1, i);
-  Corners<T2> c2 = load_corners<T2>(b2, i);
-  Corners<R> g, p;
-  g.x1 = (R)c1.x1; g.y1 = (R)c1.y1; g.x2 = (R)c1.x2; g.y2 = (R)c1.y2; g.area = (R)c1.area;
-  p.x1 = (R)c2.x1; p.y1 = (R)c2.y1; p.x2 = (R)c2.x2; p.y2 = (R)c2.y2; p.area = (R)c2.area;
-  reinterpret_cast<R*>(out)[i] = iou_corners<R>(g, p, use_eps ? (R)1e-10 : (R)0);
+  reinterpret_cast<R*>(out)[i] =
+      iou_corners<R>(load_corners<T1, R>(b1, i), load_corners<T2, R>(b2, i), use_eps ? (R)1e-10 : (R)0);
 }
 
 static inline unsigned blocks_for(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }

@@ -72,7 +72,7 @@ struct MatchParams {
   float* out_loc;
   uint8_t* out_mask;
   int* out_match;
-  u32* ws_head;             // [0] next image, [1] status bits, [2] next row of the search kernel, [3] tiles evaluated
+  u32* ws_head;             // head words H_*
   u32* ws_ncand;            // [B] listed pairs of the image
   u64* ws_rowkey;           // [B*tm] row maximum (key64) found by the search kernel
   int* ws_rowcol;           // [B*tm] its first arg-max prior
@@ -83,7 +83,7 @@ struct MatchParams {
   const TileStat* tiles;    // [ntiles]
   const TileStat* supers;   // [ceil(ntiles / kSuper)] statistics of kSuper consecutive tiles each
   const int* perm;          // [ntiles*32] slot -> prior index (-1: padding); NULL: identity
-  const void* pprior;       // [ntiles*32,4] the priors in slot order (same dtype); NULL: gather through perm
+  const void* pprior;       // [ntiles*32,4] the priors in slot order (same dtype); without an index the priors themselves
   const float4* unmatched;  // [A] encoding of an all-zero box per prior; NULL: compute
   int ntiles;
   int elim_words;
@@ -92,38 +92,14 @@ struct MatchParams {
   long long prior_words;    // 8-byte words of the prior array
 };
 
+// Words of the workspace head (ws_head).  ssdg_match_status and the pipeline read H_STATUS, bench.py H_TILES.
+enum { H_NEXT_IMG = 0, H_STATUS = 1, H_NEXT_ROW = 2, H_TILES = 3 };
+// Status bits of H_STATUS (ssdgeom.ops.MATCH_STATUS_*).
+enum : u32 { ST_TOO_MANY_GT = 1u, ST_MORE_GT_THAN_PRIORS = 2u, ST_RESCAN = 4u, ST_STALE_INDEX = 8u };
+
 // Position-weighted sum of the 8-byte words of the prior array (mod 2^64): order-independent to accumulate, sensitive
 // to any changed, moved or swapped word.  Host (index build) and device (every launch with an index) agree exactly.
 __host__ __device__ __forceinline__ u64 checksum_term(u64 word, long long i) { return word * (2ull * (u64)i + 1ull); }
-
-template <typename TG, typename TP>
-struct Promote {
-  typedef double type;
-};
-template <>
-struct Promote<float, float> {
-  typedef float type;
-};
-
-template <typename T>
-struct Vec4;
-template <>
-struct Vec4<float> {
-  static __device__ __forceinline__ void load(const void* base, long long i, float& a, float& b, float& c,
-                                              float& d) {
-    float4 v = __ldg(reinterpret_cast<const float4*>(base) + i);
-    a = v.x; b = v.y; c = v.z; d = v.w;
-  }
-};
-template <>
-struct Vec4<double> {
-  static __device__ __forceinline__ void load(const void* base, long long i, double& a, double& b, double& c,
-                                              double& d) {
-    const double2* p = reinterpret_cast<const double2*>(base) + 2 * i;
-    double2 u = __ldg(p), v = __ldg(p + 1);
-    a = u.x; b = u.y; c = v.x; d = v.y;
-  }
-};
 
 __device__ __forceinline__ float f_down(double v) { return __double2float_rd(v); }
 __device__ __forceinline__ float f_up(double v) { return __double2float_ru(v); }
@@ -131,22 +107,19 @@ __device__ __forceinline__ bool finite4(double a, double b, double c, double d) 
   return isfinite(a) && isfinite(b) && isfinite(c) && isfinite(d);
 }
 
-// apply_anchor_box for one row (utils/bbox.py:98-99), float64 arithmetic, float32 result
-// (the TensorSpec cast at models/ssd_model.py:222).
+// apply_anchor_box for one row (utils/bbox.py:98-99): float64 arithmetic, float32 result (the TensorSpec cast at
+// models/ssd_model.py:222).
 template <typename TP>
-__device__ __forceinline__ float4 encode_row(float bx, float by, float bw, float bh, TP dx, TP dy, TP dw,
-                                             TP dh) {
-  double tx = ((double)bx - (double)dx) / (double)dw;
-  double ty = ((double)by - (double)dy) / (double)dh;
-  double rw = (double)fmaxf(bw, 1e-5f) / (double)max_nn(dw, (TP)1e-5);
-  double rh = (double)fmaxf(bh, 1e-5f) / (double)max_nn(dh, (TP)1e-5);
-  return make_float4((float)tx, (float)ty, (float)log(rw), (float)log(rh));
+__device__ __forceinline__ float4 encode_row(float bx, float by, float bw, float bh, TP dx, TP dy, TP dw, TP dh) {
+  const double4 t = anchor_offsets<float, TP>(bx, by, bw, bh, dx, dy, dw, dh);
+  return make_float4((float)t.x, (float)t.y, (float)t.z, (float)t.w);
 }
 
-// Conservative float bound of the IoU the exact path would compute for a ground truth against any prior
-// of a tile: iub bounds the intersection from above, dlb the denominator from below (outward-rounded
-// corners, directed rounding).  A NaN anywhere leaves dlb NaN.
-__device__ __forceinline__ void iou_bound(const float4& g, float ga_lo, const TileStat& s, float& iub, float& dlb) {
+// Conservative float bound of the IoU the exact path would compute for ground truth (gb, ga_lo) against any prior
+// of a tile: the intersection is bounded from above, the denominator from below (outward-rounded corners,
+// directed rounding).  Always > 0; +inf when the tile holds a non-finite prior, a NaN leaves the denominator
+// bound NaN, or the denominator bound is at least 2^126 (__fdividef returns 0 there: a huge finite ground truth).
+__device__ __forceinline__ float tile_ub(const float4& g, float ga_lo, const TileStat& s) {
   float ex = fmaxf(__fsub_ru(fminf(g.z, s.x2), fmaxf(g.x, s.x1)), 1.0001e-10f);
   float ey = fmaxf(__fsub_ru(fminf(g.w, s.y2), fmaxf(g.y, s.y1)), 1.0001e-10f);
   // a prior with mid-point c and half-extent h overlaps the ground truth by at most  g.hi - (c - h)  and
@@ -156,14 +129,31 @@ __device__ __forceinline__ void iou_bound(const float4& g, float ga_lo, const Ti
   ey = fminf(ey, fminf(__fadd_ru(__fsub_ru(g.w, s.cy1), hh), __fsub_ru(__fadd_ru(s.cy2, hh), g.y)));
   ex = fmaxf(fminf(ex, s.wmax), 1.0001e-10f);
   ey = fmaxf(fminf(ey, s.hmax), 1.0001e-10f);
-  iub = __fmul_ru(ex, ey);
-  dlb = __fadd_rd(__fsub_rd(__fadd_rd(ga_lo, s.amin), iub), 0.9999e-10f);
+  const float iub = __fmul_ru(ex, ey);
+  const float dlb = __fadd_rd(__fsub_rd(__fadd_rd(ga_lo, s.amin), iub), 0.9999e-10f);
+  return (s.safe && dlb > 0.f && dlb < 0x1p126f) ? __fdividef(iub, dlb) * 1.0002f : CUDART_INF_F;
 }
-// true unless  iou < bound  is certain for every prior of the tile
-__device__ __forceinline__ bool may_reach(const float4& g, float ga_lo, const TileStat& s, float bound) {
-  float iub, dlb;
-  iou_bound(g, ga_lo, s, iub, dlb);
-  return !s.safe || !(dlb > 0.f && iub * 1.0001f < bound * dlb);
+
+// Ground-truth row i for the search and the re-search: corners in R, the outward-rounded float box `gb` and the
+// float lower bound `ga_lo` of the area (NaN when a corner or the area is not finite: never culled).
+template <typename TG, typename R>
+__device__ __forceinline__ Corners<R> gt_row(const void* gt_boxes, long long i, float4& gb, float& ga_lo) {
+  const Corners<R> g = load_corners<TG, R>(gt_boxes, i);
+  const bool ok = finite4((double)g.x1, (double)g.y1, (double)g.x2, (double)g.y2) && isfinite((double)g.area);
+  gb = make_float4(f_down((double)g.x1), f_down((double)g.y1), f_up((double)g.x2), f_up((double)g.y2));
+  ga_lo = ok ? f_down((double)g.area) : CUDART_NAN_F;
+  return g;
+}
+
+// Exact IoU key of this lane's slot of tile `tile` against ground truth g, from the priors in slot order (P.pprior);
+// 0 for a padding slot or a prior knocked out in `elim` (null: none).  a receives the slot's prior index.
+template <typename TP, typename R>
+__device__ __forceinline__ u64 slot_key(const MatchParams& P, const Corners<R>& g, int tile, int lane, const u32* elim,
+                                        int& a) {
+  const int slot = (tile << 5) + lane;
+  a = P.perm ? __ldg(P.perm + slot) : slot;
+  if (a < 0 || a >= P.A || (elim && ((elim[a >> 5] >> (a & 31)) & 1u))) return 0ull;
+  return key64((double)iou_corners<R>(g, load_corners<TP, R>(P.pprior, slot), (R)1e-10));
 }
 
 // ---- per-tile statistics of the priors ---------------------------------------------------------------------
@@ -180,17 +170,15 @@ __global__ void __launch_bounds__(256) tile_stats_kernel(const void* __restrict_
   u32 kc1 = ~0u, kd1 = ~0u, kc2 = 0u, kd2 = 0u;
   bool safe = true;
   if (valid) {
-    TP cx, cy, w, h;
-    Vec4<TP>::load(priors, a, cx, cy, w, h);
-    Corners<TP> c = corners_of<TP>(cx, cy, w, h);
-    safe = finite4((double)c.x1, (double)c.y1, (double)c.x2, (double)c.y2) && isfinite((double)c.area);
+    const Corners<double> c = load_corners<TP, double>(priors, a);
+    safe = finite4(c.x1, c.y1, c.x2, c.y2) && isfinite(c.area);
     if (safe) {
-      const float x1 = f_down((double)c.x1), y1 = f_down((double)c.y1);
-      const float x2 = f_up((double)c.x2), y2 = f_up((double)c.y2);
+      const float x1 = f_down(c.x1), y1 = f_down(c.y1);
+      const float x2 = f_up(c.x2), y2 = f_up(c.y2);
       kx1 = key32(x1); ky1 = key32(y1); kx2 = key32(x2); ky2 = key32(y2);
       kw = key32(__fsub_ru(x2, x1)); kh = key32(__fsub_ru(y2, y1));
-      ka = key32(f_down((double)c.area));
-      const double mx = 0.5 * ((double)c.x1 + (double)c.x2), my = 0.5 * ((double)c.y1 + (double)c.y2);
+      ka = key32(f_down(c.area));
+      const double mx = 0.5 * (c.x1 + c.x2), my = 0.5 * (c.y1 + c.y2);
       kc1 = key32(f_down(mx - 1e-12 * fabs(mx))); kc2 = key32(f_up(mx + 1e-12 * fabs(mx)));
       kd1 = key32(f_down(my - 1e-12 * fabs(my))); kd2 = key32(f_up(my + 1e-12 * fabs(my)));
     }
@@ -293,23 +281,21 @@ constexpr int kSearchCtasPerSm = 10;
 template <typename TG, typename TP, bool kHier>   // kHier: two-level bound (super-tiles of kSuper tiles, then tiles); up to kTileSmemMax tiles
 __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kernel(MatchParams P) {
   typedef typename Promote<TG, TP>::type R;
-  extern __shared__ __align__(128) unsigned char smem_raw[];
   const int lane = threadIdx.x & 31;
-  const int A = P.A, ntiles = P.ntiles;
+  const int ntiles = P.ntiles;
   // the tile statistics stay in global memory (L1/L2-resident, 14 KB for SSD300): staging them per CTA costs
   // shared memory that decides how many of these CTAs fit beside a streaming kernel of the other branch
   const TileStat* tiles = P.tiles;
-  const R EPS = (R)1e-10;
   const u64 thr_key = key64((double)(R)P.thresh);
   const float thr_lo = f_down((double)(R)P.thresh);
   const int total_rows = P.gt_off[P.B];
-  u32 n_eval = 0u;   // tiles this warp evaluated exactly (ws_head[3]: the matcher's work counter, bench.py)
+  u32 n_eval = 0u;   // tiles this warp evaluated exactly (H_TILES: the matcher's work counter, bench.py)
   for (;;) {
     int gr = 0;
-    if (lane == 0) gr = (int)atomicAdd(&P.ws_head[2], 1u);
+    if (lane == 0) gr = (int)atomicAdd(&P.ws_head[H_NEXT_ROW], 1u);
     gr = __shfl_sync(SSDG_FULL, gr, 0);
     if (gr >= total_rows) {
-      if (lane == 0 && n_eval) atomicAdd(&P.ws_head[3], n_eval);
+      if (lane == 0 && n_eval) atomicAdd(&P.ws_head[H_TILES], n_eval);
       break;
     }
     // image of the row: last b with gt_off[b] <= gr
@@ -320,19 +306,10 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
     }
     const int img = lo, g0 = __ldg(P.gt_off + img);
     const int T = __ldg(P.gt_off + img + 1) - g0, t = gr - g0;
-    if (t < 0 || t >= T || T > P.max_gt || T > A) continue;   // malformed offsets / flagged images: no rows
-    Corners<R> g;
+    if (t < 0 || t >= T || T > P.max_gt || T > P.A) continue;   // malformed offsets / flagged images: no rows
     float4 gb;
     float galo;
-    {
-      TG cx, cy, w, h;
-      Vec4<TG>::load(P.gt_boxes, gr, cx, cy, w, h);
-      const Corners<TG> c = corners_of<TG>(cx, cy, w, h);
-      g.x1 = (R)c.x1; g.y1 = (R)c.y1; g.x2 = (R)c.x2; g.y2 = (R)c.y2; g.area = (R)c.area;
-      const bool ok = finite4((double)g.x1, (double)g.y1, (double)g.x2, (double)g.y2) && isfinite((double)g.area);
-      gb = make_float4(f_down((double)g.x1), f_down((double)g.y1), f_up((double)g.x2), f_up((double)g.y2));
-      galo = ok ? f_down((double)g.area) : CUDART_NAN_F;
-    }
+    const Corners<R> g = gt_row<TG, R>(P.gt_boxes, gr, gb, galo);
     Cand* cand = P.ws_cand + (size_t)img * kCandCap;
     u64 best_key = 0ull;
     int best_a = 0x7fffffff;
@@ -341,18 +318,8 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
     // exact evaluation of one tile for this row (all lanes)
     auto evaluate = [&](int tile) {
       ++n_eval;
-      const int slot = (tile << 5) + lane;
-      const int a = P.perm ? __ldg(P.perm + slot) : slot;
-      const bool valid = a >= 0 && a < A;
-      u64 key = 0ull;
-      if (valid) {
-        Corners<R> p;
-        TP dx, dy, dw, dh;
-        Vec4<TP>::load(P.pprior ? P.pprior : P.priors, P.pprior ? slot : a, dx, dy, dw, dh);
-        const Corners<TP> c = corners_of<TP>(dx, dy, dw, dh);
-        p.x1 = (R)c.x1; p.y1 = (R)c.y1; p.x2 = (R)c.x2; p.y2 = (R)c.y2; p.area = (R)c.area;
-        key = key64((double)iou_corners<R>(g, p, EPS));
-      }
+      int a;
+      const u64 key = slot_key<TP, R>(P, g, tile, lane, nullptr, a);
       const bool listed = key > thr_key;   // phase-2 candidate; one counter update per warp
       const u32 lm = __ballot_sync(SSDG_FULL, listed);
       if (lm) {
@@ -367,17 +334,23 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
       }
       // every lane keeps its own best (key, then lowest prior): one arg-max across the warp per ROW.  The running
       // row maximum only prunes: a lower bound of it (the key's high word, one REDUX) is all pass 2 needs.
-      if (valid && (key > best_key || (key == best_key && a < best_a))) { best_key = key; best_a = a; }
+      if (a >= 0 && a < P.A && (key > best_key || (key == best_key && a < best_a))) { best_key = key; best_a = a; }
       const u32 mhi = __reduce_max_sync(SSDG_FULL, (u32)(key >> 32));
       if (mhi > rowhi) {
         rowhi = mhi;
         rowlo = fmaxf(f_down(unkey64((u64)mhi << 32)), 0.f);
       }
     };
-    auto tile_ub = [&](const TileStat& ts) {
-      float iub, dlb;
-      iou_bound(gb, galo, ts, iub, dlb);
-      return (ts.safe && dlb > 0.f) ? __fdividef(iub, dlb) * 1.0002f : CUDART_INF_F;   // always > 0
+    // visit(l) for every lane l whose bound ub (< 0: nothing pending) still reaches min(thresh, running maximum),
+    // lowest lane first; the bound is consumed
+    auto drain = [&](float& ub, auto&& visit) {
+      for (;;) {
+        const u32 m = __ballot_sync(SSDG_FULL, ub >= 0.f && !(ub < fminf(thr_lo, rowlo)));
+        if (!m) break;
+        const int l = __ffs(m) - 1;
+        if (lane == l) ub = -1.f;
+        visit(l);
+      }
     };
     if (kHier) {
       // Two levels.  A ground-truth box can reach min(thresh, its row maximum) only in a handful of the ~300 tiles, and
@@ -390,9 +363,9 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
 #pragma unroll
       for (int q = 0; q < kSuperRegs; ++q) {
         const int sp = q * 32 + lane;
-        sub[q] = -1.f;                          // < 0: nothing pending
+        sub[q] = -1.f;
         if (sp < nsuper) {
-          sub[q] = tile_ub(P.supers[sp]);
+          sub[q] = tile_ub(gb, galo, P.supers[sp]);
           if (sub[q] > smax) { smax = sub[q]; sbest = sp; }
         }
       }
@@ -404,7 +377,7 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
       int stile;
       {
         const int tile = sbest * kSuper + (lane & (kSuper - 1));
-        const float ub = (lane < kSuper && tile < ntiles) ? tile_ub(tiles[tile]) : -1.f;
+        const float ub = (lane < kSuper && tile < ntiles) ? tile_ub(gb, galo, tiles[tile]) : -1.f;
         const u32 m = __reduce_max_sync(SSDG_FULL, key32(ub));
         stile = (int)__reduce_min_sync(SSDG_FULL, key32(ub) == m ? (u32)tile : 0x7fffffffu);
       }
@@ -413,59 +386,36 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
 #pragma unroll
       for (int q = 0; q < kSuperRegs; ++q) {
         if (q * 32 >= nsuper) break;
-        for (;;) {
-          const bool reach = sub[q] >= 0.f && !(sub[q] < fminf(thr_lo, rowlo));
-          const u32 m = __ballot_sync(SSDG_FULL, reach);
-          if (!m) break;
-          const int l = __ffs(m) - 1;
-          if (lane == l) sub[q] = -1.f;
-          const int tile = (q * 32 + l) * kSuper + (lane & (kSuper - 1));
-          float ub = (lane < kSuper && tile < ntiles && tile != stile) ? tile_ub(tiles[tile]) : -1.f;
-          for (;;) {
-            const bool r2 = ub >= 0.f && !(ub < fminf(thr_lo, rowlo));
-            const u32 m2 = __ballot_sync(SSDG_FULL, r2);
-            if (!m2) break;
-            const int l2 = __ffs(m2) - 1;
-            if (lane == l2) ub = -1.f;
-            evaluate((q * 32 + l) * kSuper + l2);
-          }
-        }
+        drain(sub[q], [&](int l) {
+          const int base = (q * 32 + l) * kSuper, tile = base + (lane & (kSuper - 1));
+          float ub = (lane < kSuper && tile < ntiles && tile != stile) ? tile_ub(gb, galo, tiles[tile]) : -1.f;
+          drain(ub, [&](int l2) { evaluate(base + l2); });
+        });
       }
     } else {
-    // pass 1: bound every tile; the highest bound seeds the running maximum
-    float sub = -1.f;
-    int stile = 0x7fffffff;
+      // pass 1: bound every tile; the highest bound seeds the running maximum
+      float sub = -1.f;
+      int stile = 0x7fffffff;
 #pragma unroll 4
-    for (int tb = 0; tb < ntiles; tb += 32) {
-      const int tile = tb + lane;
-      if (tile < ntiles) {
-        const float ub = tile_ub(tiles[tile]);
-        if (ub > sub) { sub = ub; stile = tile; }
+      for (int tb = 0; tb < ntiles; tb += 32) {
+        const int tile = tb + lane;
+        if (tile < ntiles) {
+          const float ub = tile_ub(gb, galo, tiles[tile]);
+          if (ub > sub) { sub = ub; stile = tile; }
+        }
       }
-    }
-    {
-      const u32 m = __reduce_max_sync(SSDG_FULL, key32(sub));
-      stile = (int)__reduce_min_sync(SSDG_FULL, key32(sub) == m ? (u32)stile : 0x7fffffffu);
-    }
-    __syncwarp();
-    evaluate(stile);
-    // pass 2: every other tile whose bound still reaches min(thresh, running maximum)
-    for (int tb = 0; tb < ntiles; tb += 32) {
-      const int tile = tb + lane;
-      bool pending = tile < ntiles && tile != stile;
-      TileStat ts;
-      ts.x1 = ts.y1 = ts.x2 = ts.y2 = ts.wmax = ts.hmax = ts.amin = ts.cx1 = ts.cy1 = ts.cx2 = ts.cy2 = 0.f; ts.safe = 1u;
-      if (pending) ts = tiles[tile];
-      for (;;) {
-        const float bound = fminf(thr_lo, rowlo);
-        const bool reach = pending && may_reach(gb, galo, ts, bound);
-        const u32 m = __ballot_sync(SSDG_FULL, reach);
-        if (!m) break;
-        const int l = __ffs(m) - 1;
-        if (lane == l) pending = false;
-        evaluate(tb + l);
+      {
+        const u32 m = __reduce_max_sync(SSDG_FULL, key32(sub));
+        stile = (int)__reduce_min_sync(SSDG_FULL, key32(sub) == m ? (u32)stile : 0x7fffffffu);
       }
-    }
+      __syncwarp();
+      evaluate(stile);
+      // pass 2: every other tile whose bound still reaches min(thresh, running maximum)
+      for (int tb = 0; tb < ntiles; tb += 32) {
+        const int tile = tb + lane;
+        float ub = (tile < ntiles && tile != stile) ? tile_ub(gb, galo, tiles[tile]) : -1.f;
+        drain(ub, [&](int l) { evaluate(tb + l); });
+      }
     }
     warp_argmax_u64(best_key, best_a);
     if (lane == 0) {
@@ -476,7 +426,9 @@ __global__ void __launch_bounds__(kSearchThreads, kSearchCtasPerSm) search_kerne
   }
 }
 
-enum { C_IMG = 0, C_NCAND, C_NRS, C_DONE, C_ROUND, C_DEGEN, C_MINELIM, C_NEXTROW, C_RLO, C_RA, C_RKEY_LO, C_RKEY_HI, C_GENERIC, C_HEAD, C_NLIVE };
+enum { C_IMG = 0, C_NRS, C_DONE, C_ROUND, C_DEGEN, C_MINELIM, C_RLO, C_RA, C_RKEY_LO, C_RKEY_HI, C_GENERIC, C_HEAD, C_NLIVE };
+// C_RKEY_LO / C_RKEY_HI are read as one u64; MatchSmem::ctl is 16-byte aligned
+static_assert(C_RKEY_LO % 2 == 0, "C_RKEY_LO must be 8-byte aligned");
 
 template <typename TG, typename TP>
 __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(MatchParams P) {
@@ -502,11 +454,6 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
     for (int i = tid; i < ntiles; i += kMatchThreads) S.tiles_s[i] = P.tiles[i];
   for (int a = tid; a < A; a += kMatchThreads) { colkey[a] = 0ull; colt[a] = 0x7fffffff; }
 
-  auto load_prior = [&](int a, Corners<R>& p, TP& dx, TP& dy, TP& dw, TP& dh) {
-    Vec4<TP>::load(P.priors, a, dx, dy, dw, dh);
-    Corners<TP> c = corners_of<TP>(dx, dy, dw, dh);
-    p.x1 = (R)c.x1; p.y1 = (R)c.y1; p.x2 = (R)c.x2; p.y2 = (R)c.y2; p.area = (R)c.area;
-  };
   auto load_gt = [&](int t) {
     Corners<R> g;
     g.x1 = S.gx1[t]; g.y1 = S.gy1[t]; g.x2 = S.gx2[t]; g.y2 = S.gy2[t]; g.area = S.ga[t];
@@ -515,7 +462,7 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
   auto bit_test = [&](const u32* bm, int a) { return (bm[a >> 5] >> (a & 31)) & 1u; };
 
   // The index must belong to THESE priors (in-place edits such as ssdg_priors_clip, or a recycled address, would
-  // silently pair with stale tiles): one CTA re-derives the content checksum and raises status bit 3 on mismatch.
+  // silently pair with stale tiles): one CTA re-derives the content checksum and raises ST_STALE_INDEX on mismatch.
   if (P.index_sum != 0ull && blockIdx.x == 0) {
     const u64* w = reinterpret_cast<const u64*>(P.priors);
     u64 acc = 0ull;
@@ -527,7 +474,7 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
     __syncthreads();
     if (lane == 0) atomicAdd(reinterpret_cast<unsigned long long*>(cs), (unsigned long long)acc);
     __syncthreads();
-    if (tid == 0 && *cs != P.index_sum) atomicOr(&P.ws_head[1], 8u);
+    if (tid == 0 && *cs != P.index_sum) atomicOr(&P.ws_head[H_STATUS], ST_STALE_INDEX);
     __syncthreads();
   }
 
@@ -545,7 +492,7 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
 #ifdef SSDG_MATCH_TIMING
     if (tid == 0) tk0 = clock64();
 #endif
-    if (tid == 0) S.ctl[C_IMG] = (int)atomicAdd(&P.ws_head[0], 1u);
+    if (tid == 0) S.ctl[C_IMG] = (int)atomicAdd(&P.ws_head[H_NEXT_IMG], 1u);
     __syncthreads();
     const int img = S.ctl[C_IMG];
     if (img >= P.B) break;
@@ -553,30 +500,24 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
     int T = P.gt_off[img + 1] - g0;
     if (T < 0) T = 0;
     bool bad = false;
-    if (T > P.max_gt) { if (tid == 0) atomicOr(&P.ws_head[1], 1u); bad = true; }
-    if (T > A) { if (tid == 0) atomicOr(&P.ws_head[1], 2u); bad = true; }
+    if (T > P.max_gt) { if (tid == 0) atomicOr(&P.ws_head[H_STATUS], ST_TOO_MANY_GT); bad = true; }
+    if (T > A) { if (tid == 0) atomicOr(&P.ws_head[H_STATUS], ST_MORE_GT_THAN_PRIORS); bad = true; }
     if (bad) T = 0;  // outputs for the image are still fully written (all unmatched)
     const size_t obase = (size_t)img * A;
     const Cand* cand = P.ws_cand + (size_t)img * kCandCap;
 
     // ---- per-image setup -------------------------------------------------------------------
     for (int t = tid; t < T; t += kMatchThreads) {
-      TG cx, cy, w, h;
-      Vec4<TG>::load(P.gt_boxes, g0 + t, cx, cy, w, h);
-      Corners<TG> c = corners_of<TG>(cx, cy, w, h);
-      R x1 = (R)c.x1, y1 = (R)c.y1, x2 = (R)c.x2, y2 = (R)c.y2, ar = (R)c.area;
-      S.gx1[t] = x1; S.gy1[t] = y1; S.gx2[t] = x2; S.gy2[t] = y2; S.ga[t] = ar;
-      const bool ok = finite4((double)x1, (double)y1, (double)x2, (double)y2) && isfinite((double)ar);
-      S.cbox[t] = make_float4(f_down((double)x1), f_down((double)y1), f_up((double)x2), f_up((double)y2));
-      S.galo[t] = ok ? f_down((double)ar) : CUDART_NAN_F;
+      const Corners<R> g = gt_row<TG, R>(P.gt_boxes, g0 + t, S.cbox[t], S.galo[t]);
+      S.gx1[t] = g.x1; S.gy1[t] = g.y1; S.gx2[t] = g.x2; S.gy2[t] = g.y2; S.ga[t] = g.area;
       S.rowkey[t] = P.ws_rowkey[(size_t)img * P.tm + t];     // the search kernel's result for this row
       S.rowcol[t] = P.ws_rowcol[(size_t)img * P.tm + t];
       S.dead[t] = 0;
     }
     for (int w = tid; w < P.elim_words; w += kMatchThreads) { elim[w] = 0u; touch[w] = 0u; }
     if (tid == 0) {
-      S.ctl[C_NCAND] = 0; S.ctl[C_NRS] = 0; S.ctl[C_DONE] = 0; S.ctl[C_ROUND] = 0; S.ctl[C_DEGEN] = 0;
-      S.ctl[C_MINELIM] = 0x7fffffff; S.ctl[C_NEXTROW] = 0; S.ctl[C_GENERIC] = 0; S.ctl[C_HEAD] = 0; S.ctl[C_NLIVE] = -1;
+      S.ctl[C_NRS] = 0; S.ctl[C_DONE] = 0; S.ctl[C_ROUND] = 0; S.ctl[C_DEGEN] = 0;
+      S.ctl[C_MINELIM] = 0x7fffffff; S.ctl[C_GENERIC] = 0; S.ctl[C_HEAD] = 0; S.ctl[C_NLIVE] = -1;
     }
     __syncthreads();
 
@@ -597,12 +538,7 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
         const int tile = tb + lane;
         bool pending = tile < ntiles;
         float ub = 0.f;
-        if (pending) {
-          const TileStat ts = tiles[tile];
-          float iub, dlb;
-          iou_bound(gb, galo, ts, iub, dlb);
-          ub = (ts.safe && dlb > 0.f) ? __fdividef(iub, dlb) * 1.0002f : CUDART_INF_F;
-        }
+        if (pending) ub = tile_ub(gb, galo, tiles[tile]);
         for (;;) {
           const float rowlo = __int_as_float(*reinterpret_cast<volatile int*>(&S.ctl[C_RLO]));
           const bool reach = pending && !(ub < fminf(thr_lo, rowlo));
@@ -611,23 +547,9 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
           const u32 mk = __reduce_max_sync(SSDG_FULL, reach ? key32(ub) : 0u);
           const int l = __ffs(__ballot_sync(SSDG_FULL, reach && key32(ub) == mk)) - 1;
           if (lane == l) pending = false;
-          const int slot = ((tb + l) << 5) + lane;
-          const int a = P.perm ? __ldg(P.perm + slot) : slot;
-          const bool valid = a >= 0 && a < A && !bit_test(elim, a);
-          u64 key = 0ull;
-          if (valid) {
-            Corners<R> p; TP dx, dy, dw, dh;
-            if (P.pprior) {
-              Vec4<TP>::load(P.pprior, slot, dx, dy, dw, dh);
-              Corners<TP> c = corners_of<TP>(dx, dy, dw, dh);
-              p.x1 = (R)c.x1; p.y1 = (R)c.y1; p.x2 = (R)c.x2; p.y2 = (R)c.y2; p.area = (R)c.area;
-            } else {
-              load_prior(a, p, dx, dy, dw, dh);
-            }
-            key = key64((double)iou_corners<R>(g, p, EPS));
-          }
-          u64 wk = key;
-          int wa = valid ? a : 0x7fffffff;
+          int a;
+          u64 wk = slot_key<TP, R>(P, g, tb + l, lane, elim, a);
+          int wa = wk ? a : 0x7fffffff;
           warp_argmax_u64(wk, wa);
           if (wk > my_key || (wk == my_key && wa < my_a)) { my_key = wk; my_a = wa; }
           if (lane == 0 && wk > 0ull) {
@@ -651,10 +573,9 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
     const int ncand = cand_overflow ? 0 : ncand_raw;
     if (cand_overflow) {
       // more pairs above the threshold than the list holds: exhaustive exact scan, one prior per thread
-      if (tid == 0) atomicOr(&P.ws_head[1], 4u);
+      if (tid == 0) atomicOr(&P.ws_head[H_STATUS], ST_RESCAN);
       for (int a = tid; a < A; a += kMatchThreads) {
-        Corners<R> p; TP dx, dy, dw, dh;
-        load_prior(a, p, dx, dy, dw, dh);
+        const Corners<R> p = load_corners<TP, R>(P.priors, a);
         u64 bk = 0ull;
         int bt = 0x7fffffff;
         for (int t = 0; t < T; ++t) {
@@ -829,37 +750,42 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
       if (tid == 0 && nrs > 0) atomicAdd((unsigned long long*)&P.ws_head[42], (unsigned long long)(clock64() - rs0));
 #endif
       __syncthreads();
-      if (tid == 0) { S.ctl[C_NRS] = 0; S.ctl[C_NEXTROW] = 0; }
+      if (tid == 0) S.ctl[C_NRS] = 0;
       __syncthreads();
       if (done) break;
     }
 
     TICK(3);
     // ---- output: every prior once, in prior order (phase 2), then the phase-1 pairs ---------------------
-    auto emit_prior = [&](int a, bool pos, const float4& un) {
+    // targets of prior a: matched to row t, or unmatched (t < 0) with encoding un (when P.unmatched)
+    auto write_targets = [&](int a, int t, const float4& un) {
       float bx = 0.f, by = 0.f, bw = 0.f, bh = 0.f;
-      int lab = 0, ct = -1;
-      if (pos) {
-        ct = colt[a];
+      int lab = 0;
+      if (t >= 0) {
         TG gx, gy, gw, gh;
-        Vec4<TG>::load(P.gt_boxes, g0 + ct, gx, gy, gw, gh);
+        Vec4<TG>::load(P.gt_boxes, g0 + t, gx, gy, gw, gh);
         bx = (float)gx; by = (float)gy; bw = (float)gw; bh = (float)gh;
-        lab = (int)__ldg(P.gt_cls + g0 + ct);
-        colkey[a] = 0ull; colt[a] = 0x7fffffff;     // leave the scratch clean for the next image
+        lab = (int)__ldg(P.gt_cls + g0 + t);
       }
       if (P.out_cls) P.out_cls[obase + a] = lab;
-      if (P.out_mask) P.out_mask[obase + a] = pos ? 1 : 0;
-      if (P.out_match) P.out_match[obase + a] = ct;
+      if (P.out_mask) P.out_mask[obase + a] = t >= 0 ? 1 : 0;
+      if (P.out_match) P.out_match[obase + a] = t;
       if (P.out_box) reinterpret_cast<float4*>(P.out_box)[obase + a] = make_float4(bx, by, bw, bh);
       if (P.out_loc) {
         float4 enc = un;
-        if (pos || !P.unmatched) {
+        if (t >= 0 || !P.unmatched) {
           TP dx, dy, dw, dh;
           Vec4<TP>::load(P.priors, a, dx, dy, dw, dh);
           enc = encode_row<TP>(bx, by, bw, bh, dx, dy, dw, dh);
         }
         reinterpret_cast<float4*>(P.out_loc)[obase + a] = enc;
       }
+    };
+    // phase 2: a positive takes its column's first-arg-max row and leaves the scratch clean for the next image
+    auto emit_prior = [&](int a, bool pos, const float4& un) {
+      int t = -1;
+      if (pos) { t = colt[a]; colkey[a] = 0ull; colt[a] = 0x7fffffff; }
+      write_targets(a, t, un);
     };
     {
       // Positives are ~3 % of the priors and their encoding is ~300 float64 instructions (two logarithms, four
@@ -901,19 +827,7 @@ __global__ void __launch_bounds__(kMatchThreads, kMatchCtasPerSm) match_kernel(M
       if (degen)
         for (int k2 = k + 1; k2 < T; ++k2)
           if (S.pair_a[k2] == a) { last = false; break; }
-      if (!last) continue;
-      TG gx, gy, gw, gh;
-      Vec4<TG>::load(P.gt_boxes, g0 + t, gx, gy, gw, gh);
-      const float bx = (float)gx, by = (float)gy, bw = (float)gw, bh = (float)gh;
-      if (P.out_cls) P.out_cls[obase + a] = (int)__ldg(P.gt_cls + g0 + t);
-      if (P.out_mask) P.out_mask[obase + a] = 1;
-      if (P.out_match) P.out_match[obase + a] = t;
-      if (P.out_box) reinterpret_cast<float4*>(P.out_box)[obase + a] = make_float4(bx, by, bw, bh);
-      if (P.out_loc) {
-        TP dx, dy, dw, dh;
-        Vec4<TP>::load(P.priors, a, dx, dy, dw, dh);
-        reinterpret_cast<float4*>(P.out_loc)[obase + a] = encode_row<TP>(bx, by, bw, bh, dx, dy, dw, dh);
-      }
+      if (last) write_targets(a, t, make_float4(0.f, 0.f, 0.f, 0.f));
     }
     TICK(4);
   }
@@ -935,14 +849,13 @@ static int launch_match(const MatchParams& P, int grid, size_t smem, cudaStream_
   prof_begin(SSDG_PROF_MATCH, st);
   {
     const bool hier = P.ntiles <= kTileSmemMax;
-    const size_t ssm = 0;
     auto skern = hier ? search_kernel<TG, TP, true> : search_kernel<TG, TP, false>;
     SSDG_CUDA_TRY(cudaFuncSetAttribute(skern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     long long sgrid = (long long)sm_count() * kSearchCtasPerSm;
     const long long want = ((long long)P.B * (P.max_gt > 0 ? P.max_gt : 1) + kSearchWarps - 1) / kSearchWarps;
     if (want < sgrid) sgrid = want;
     prof_begin(SSDG_PROF_SEARCH, st);
-    skern<<<(unsigned)sgrid, kSearchThreads, ssm, st>>>(P);
+    skern<<<(unsigned)sgrid, kSearchThreads, 0, st>>>(P);
     prof_end(SSDG_PROF_SEARCH, st);
     SSDG_LAUNCH_CHECK();
   }
@@ -1166,7 +1079,7 @@ extern "C" int ssdg_match_encode(const void* gt_boxes, int32_t gt_dtype, const f
   P.out_cls = out_cls; P.out_box = out_box; P.out_loc = out_loc; P.out_mask = out_mask; P.out_match = out_match;
   P.elim_words = (n_priors + 31) / 32;
   P.ws_head = ws.head; P.ws_ncand = ws.ncand; P.ws_rowkey = ws.rowkey; P.ws_rowcol = ws.rowcol; P.ws_cand = ws.cand; P.ws_colkey = ws.colkey; P.ws_colt = ws.colt; P.ws_bits = ws.bits;
-  P.tiles = ws.tiles; P.supers = ws.supers; P.perm = nullptr; P.unmatched = nullptr; P.pprior = nullptr; P.ntiles = (n_priors + 31) / 32;
+  P.tiles = ws.tiles; P.supers = ws.supers; P.perm = nullptr; P.unmatched = nullptr; P.pprior = priors; P.ntiles = (n_priors + 31) / 32;
   P.index_sum = 0ull;
   P.prior_words = (long long)n_priors * 4 * (prior_dtype == SSDG_F64 ? 8 : 4) / 8;
   if (prior_index) {

@@ -21,6 +21,8 @@ from ssdgeom.utils import bbox              # noqa: E402
 from ssdgeom.models import ssd_model as M   # noqa: E402
 
 RTOL = 1e-5
+# status bits that flag an image the matcher could not assign, or a stale prior index
+MATCH_ERRORS = ops.MATCH_STATUS_TOO_MANY_GT | ops.MATCH_STATUS_MORE_GT_THAN_PRIORS | ops.MATCH_STATUS_STALE_INDEX
 
 
 def sha(*arrays):
@@ -57,7 +59,7 @@ def _check_large_prior_path(priors, out):
     # more than kTileSmemMax (csrc/match.cu) tiles of 32 priors: the single-level row search, and match_kernel
     # reads the tile statistics from global memory
     assert priors.shape[0] > 32 * 1024
-    assert ops.match_status(out) & 4 == 0     # every pair fit the pair list: no exhaustive rescan
+    assert ops.match_status(out) & ops.MATCH_STATUS_RESCAN == 0     # every pair fit the pair list: no exhaustive rescan
 
 
 # ---- A1 ----------------------------------------------------------------------------------------------
@@ -199,7 +201,7 @@ def test_assign_config1_golden(golden_dir, priors300):
     boxes, cls, offsets = _config1_inputs()
     assert sha(boxes, cls, offsets, priors300) == str(g["input_sha"])
     out = ops.match_encode(boxes, cls, offsets, priors300, 8, 100, 0.5, want=("cls", "box", "loc", "mask", "match"))
-    assert ops.match_status(out) & 11 == 0
+    assert ops.match_status(out) & MATCH_ERRORS == 0
     o_cls, o_box, o_loc = out["cls"].to_host(), out["box"].to_host(), out["loc"].to_host()
     o_mask = out["mask"].to_host().astype(bool)
     for i in range(8):
@@ -241,27 +243,45 @@ def test_assign_random_bit_exact(table, batch, max_t, mode, seed, priors300, pri
 
 @pytest.mark.parametrize("table,batch,max_t,mode", [("ssd300", 12, 100, "max"), ("ssd300", 16, 100, "coco"),
                                                    ("ssd512", 3, 100, "max"), ("ssd512", 2, 500, "max"),
-                                                   ("large", 3, 100, "max")])
+                                                   ("large", 3, 100, "max"), ("ssd300", 2, 100, "wide")])
 def test_assign_with_prior_index(table, batch, max_t, mode, priors300, priors512, priors_large):
     """The shape-sorted prior index is an acceleration structure only: identical outputs with and
-    without it, and equal to the oracle."""
+    without it, and equal to the oracle.  "wide": max_t boxes of 0.5-0.9 per side in every image, matched at
+    threshold 0.01, so the pairs above the threshold overflow the pair list and the matcher rescans every prior."""
     priors = {"ssd300": priors300, "ssd512": priors512, "large": priors_large}[table]
-    boxes, cls, off = synth.make_gt(41, batch, max_t, mode)
+    thresh = 0.5
+    if mode == "wide":
+        rng = np.random.default_rng(41)
+        n = batch * max_t
+        boxes = np.concatenate([rng.uniform(0.25, 0.75, (n, 2)), rng.uniform(0.5, 0.9, (n, 2))], 1).astype(np.float32)
+        cls = rng.integers(0, 80, n).astype(np.float32)
+        off = (np.arange(batch + 1) * max_t).astype(np.int32)
+        thresh = 0.01
+    else:
+        boxes, cls, off = synth.make_gt(41, batch, max_t, mode)
     want = ("cls", "box", "loc", "mask", "match")
-    plain = ops.match_encode(boxes, cls, off, priors, batch, int(np.diff(off).max()), 0.5, want=want)
+    plain = ops.match_encode(boxes, cls, off, priors, batch, int(np.diff(off).max()), thresh, want=want)
     if table == "large":
         _check_large_prior_path(priors, plain)
     d_pri = D.to_device(priors)
     idx = ops.prior_index(d_pri)
     assert ops.prior_index(d_pri) is idx                      # cached on the array
-    fast = ops.match_encode(boxes, cls, off, d_pri, batch, int(np.diff(off).max()), 0.5, want=want)
+    fast = ops.match_encode(boxes, cls, off, d_pri, batch, int(np.diff(off).max()), thresh, want=want)
     if table == "large":
         _check_large_prior_path(priors, fast)
+    if mode == "wide":
+        assert ops.match_status(plain) & ops.MATCH_STATUS_RESCAN and ops.match_status(fast) & ops.MATCH_STATUS_RESCAN
     for k in want:
         assert np.array_equal(plain[k].to_host(), fast[k].to_host()), k
     for i in (0, batch - 1):
-        w = O.match_bbox(cls[off[i]:off[i + 1]], boxes[off[i]:off[i + 1]], priors, 0.5, sweeps=False)
-        assert np.array_equal(fast["cls"].to_host()[i], w[0]) and np.array_equal(fast["mask"].to_host()[i].astype(bool), w[2])
+        w_cls, w_box, w_mask, pairs = O.match_bbox(cls[off[i]:off[i + 1]], boxes[off[i]:off[i + 1]], priors, thresh,
+                                                   sweeps=False, return_pairs=True)
+        w_match = np.full(priors.shape[0], -1, np.int32)
+        for t, a in pairs:
+            w_match[a] = t
+        assert np.array_equal(fast["cls"].to_host()[i], w_cls) and np.array_equal(fast["mask"].to_host()[i].astype(bool), w_mask)
+        assert np.array_equal(fast["box"].to_host()[i], w_box) and np.array_equal(fast["match"].to_host()[i], w_match)
+        close(fast["loc"].to_host()[i], O.apply_anchor_box(w_box, priors).astype(np.float32))
     # irregular priors (many distinct shapes -> single class, spatial blocking only) and float32 priors
     rng = np.random.default_rng(3)
     odd = np.concatenate([rng.uniform(0, 1, (1500, 2)), rng.uniform(0.03, 0.6, (1500, 2))], 1)
@@ -279,14 +299,15 @@ def test_assign_with_prior_index(table, batch, max_t, mode, priors300, priors512
 
 def test_assign_edge_cases(priors300):
     pri = priors300[::7].copy()
-    # duplicates, GT outside the image, tiny GT, T == 1, ragged offsets incl. an empty image
+    # duplicates, GT outside the image, tiny GT, T == 1, ragged offsets incl. an empty image, and a huge finite GT
+    # (area above 2^126: the search's float bound must not round it to 0 and skip the tile holding the arg-max)
     boxes = np.array([[0.5, 0.5, 0.3, 0.3], [0.5, 0.5, 0.3, 0.3], [3.0, 3.0, 0.1, 0.1], [0.2, 0.7, 1e-4, 1e-4],
-                      [0.31, 0.62, 0.25, 0.4]], dtype=np.float32)
-    cls = np.array([1, 2, 3, 4, 5], dtype=np.float32)
-    off = np.array([0, 4, 4, 5], dtype=np.int32)
-    out = ops.match_encode(boxes, cls, off, pri, 3, 4, 0.5, want=("cls", "box", "mask"))
+                      [0.31, 0.62, 0.25, 0.4], [0.5, 0.5, 1e19, 1e19]], dtype=np.float32)
+    cls = np.array([1, 2, 3, 4, 5, 6], dtype=np.float32)
+    off = np.array([0, 4, 4, 5, 6], dtype=np.int32)
+    out = ops.match_encode(boxes, cls, off, pri, 4, 4, 0.5, want=("cls", "box", "mask"))
     o_cls, o_box, o_mask = out["cls"].to_host(), out["box"].to_host(), out["mask"].to_host().astype(bool)
-    for i in (0, 2):
+    for i in (0, 2, 3):
         s, e = off[i], off[i + 1]
         for sweeps in (True, False):
             w = O.match_bbox(cls[s:e], boxes[s:e], pri, 0.5, sweeps=sweeps)
@@ -309,7 +330,7 @@ def test_assign_full_size_properties(priors300):
     out = ops.match_encode(boxes, cls, off, priors300, batch, 100, 0.5, want=("cls", "box", "loc", "mask", "match"))
     o_match, o_mask = out["match"].to_host(), out["mask"].to_host()
     o_box, o_cls = out["box"].to_host(), out["cls"].to_host()
-    assert ops.match_status(out) & 11 == 0
+    assert ops.match_status(out) & MATCH_ERRORS == 0
     # forced assignment: every ground truth owns at least one prior; mask <=> match >= 0
     assert np.array_equal(o_mask.astype(bool), o_match >= 0)
     for i in range(batch):

@@ -153,7 +153,8 @@ def test_hotpath_refuses_batches_it_cannot_match(priors300):
     # a correctly sized pipeline reports a clean status through download()
     hp = HotPath(synth.SSD300, batch=b, max_gt=12, total_gt=boxes.shape[0])
     hp.step_host(boxes, cls, off, pc, pb, *out)
-    assert int(hp._status_host.array[1]) & 11 == 0 and out[0][7] == 0
+    errors = ops.MATCH_STATUS_TOO_MANY_GT | ops.MATCH_STATUS_MORE_GT_THAN_PRIORS | ops.MATCH_STATUS_STALE_INDEX
+    assert int(hp._status_host.array[1]) & errors == 0 and out[0][7] == 0
 
 
 def test_prior_index_content_check_and_destroy():
