@@ -22,6 +22,7 @@
 //                  iterating "kept(i) <=> no kept j < i suppresses i" to its fixed point.
 #include <math_constants.h>
 #include <algorithm>
+#include <cstring>
 #include <type_traits>
 #include "common.cuh"
 
@@ -473,6 +474,8 @@ struct NmsParams {
   int B;
   int fast_ok;         // 0 < iou_thresh < 1e6: the division-free pre-test exists
   float q, tq0, inv_l; // thr/(1+thr); shrink factor of the slab intervals; 1 / log2 of the size-class ratio
+  u32 key_base;        // score word of the filter's threshold: every listed key's score word lies above it
+  float key_scale;     // 256 / (score word of 1.0 - key_base): rank-sort buckets over the scores (thresh, 1]
 };
 
 // The NMS kernel is instruction-cache sensitive (12 CTAs per SM in different phases): its block-stride loops
@@ -483,22 +486,32 @@ struct NmsParams {
 //   * the list is the concatenation of the runs the filter CTAs left in its slots; the counts of up to four runs
 //     are fetched together (one memory latency in front of the keys);
 //   * exact top-k: a list longer than the sort width goes through an 8-bit radix select of the composite key; then a
-//     BUCKETED RANK SORT -- 256 buckets monotone in the key, scaled to the list's own [min, max] score word (prior
-//     word when every score is equal); rank = keys in higher buckets + larger keys in the own bucket.  Exact for
-//     any input (clustered scores only lengthen a count loop);
+//     BUCKETED RANK SORT -- 256 buckets monotone in the key, fixed over the score words (threshold, 1] so that the
+//     key load builds the histogram (no range pass); only when every key lands in one bucket (equal or tightly
+//     clustered scores) are the buckets rebuilt over the keys' own [min, max] score word (prior word when every
+//     score is equal); rank = keys in higher buckets + larger keys in the own bucket.  Exact for any input
+//     (clustered scores only lengthen a count loop).  The thread that places a key at rank r < top_k also prepares
+//     box r and registers it in the join tables below, so the box load overlaps the count loop;
 //   * suppression bits by an INTERVAL JOIN instead of all pairs.  iou(i, j) > t means inter > q (a_i + a_j),
 //     q = t / (1 + t); the y overlap is at most min(h_i, h_j), so the x overlap exceeds q (w_i + w_j): the x
 //     extents of i and j, each SHRUNK by q times its width at both ends, still meet (same in y).  Every box gets
-//     the interval [a, b] of the 32 slabs per axis its shrunk extents touch; two intervals meet <=> a_j <= b_i and
+//     the interval [a, b] of the 32 slabs per axis its shrunk extents touch -- slabs fixed over [0, 1], the ends
+//     clamped (a monotone map: clamping only merges slabs); two intervals meet <=> a_j <= b_i and
 //     b_j >= a_i.  Per axis two cumulative bitset tables over the boxes, LE[s] = {j : a_j <= s}, GE[s] = {j : b_j >= s}
 //     (each box registered at its two end slabs, then a running OR along the slabs), give the x partners of box i as
 //     LE[b_i] & GE[a_i]: two loads per axis whatever the width.  SIZE CLASSES prune further: iou > t needs
 //     inter > t' E_i and inter <= w_j h_i, so the widths -- and the heights -- of a pair differ by less than 1/t';
-//     with classes of that ratio a pair's classes differ by at most one, and two more tables (class
-//     neighbourhoods) join the AND.  Survivors get the branch-free float test inter >= 0.9999 q (a_i + a_j), then
-//     the formula itself in IEEE float32 (utils/bbox.py:13-25).  The bounds are stated in the formula's areas w*h;
-//     they carry over to the corner extents unless some box's extents do not reproduce its area to 0.1 % -- then
-//     nothing is shrunk and all boxes share one class.  Thresholds <= 0 or huge use all pairs with the formula;
+//     with classes of that ratio (log2 of the width against the fixed reference 1, clamped) a pair's classes differ
+//     by at most one, and two more tables (class neighbourhoods) join the AND.  Survivors get the branch-free float
+//     test inter >= 0.9999 q (a_i + a_j), then the formula itself in IEEE float32 (utils/bbox.py:13-25).
+//     The bounds are stated in the formula's areas w*h and carry over to the corner extents W, H of a box whose
+//     extents reproduce its area to 0.1 % (exact box).  A box j that does not (inexact) is registered UNSHRUNK and in
+//     EVERY size class, and as a row it takes all registered boxes as its size partners.  That stays conservative
+//     for any partner i: the size classes no longer prune the pair, and in x the unshrunk extent of j meets i's
+//     extent shrunk by tq W_i at both ends (tq <= 0.98 q < 1/2) in at least min(ex - tq W_i, (1 - 2 tq) W_i), ex the
+//     x overlap of the two boxes; ex >= inter / H_i > q (a_i + a_j) / H_i >= q a_i / H_i >= 0.999 q W_i for an exact
+//     i (a_j > 0 for a registered box), so both terms are positive (same in y).  Two inexact boxes are both unshrunk
+//     and meet whenever inter > 0.  Thresholds <= 0 or huge use all pairs with the formula;
 //   * the join runs per group of 32 rows in two passes (candidate words as straight-line code when the word count
 //     is a template constant, then the pair tests), the groups dealt to the warps in pairs (last + first, ...):
 //     group g costs g + 1 words, so every warp gets the same number of word steps;
@@ -506,32 +519,34 @@ struct NmsParams {
 //     iterating the fixed point of kept(i) <=> no kept j < i suppresses i -- identical to the sequential greedy by
 //     induction on i, no CTA-wide barrier per round.  The suppression matrix is the lower triangle only,
 //     [group][word][row] (conflict-free);
-//   * thresholds, shrink factor and class scale come from the host; slab and bucket scales are approximate
-//     reciprocals (any positive scale keeps those maps monotone, which is all the join and the sort need).
+//   * thresholds, shrink factor, class scale and bucket scale come from the host; the slab scale is a constant
+//     (any positive scale keeps those maps monotone, which is all the join and the sort need).
 template <int kW>   // kW: words of 32 rows (top_k rounded up / 32) as a constant, 0 = any
 __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int sortn = P.sortn, mcap = (P.top_k + 31) & ~31, W = mcap >> 5, RL = (4 * W) | 1;
   const int RS = (2 * W) | 1;
-  const int tabn = (max(512, kSlabs * RL) + kSizeCls * RS + 3) & ~3;   // words, whole uint4s
+  const int tabn = (kSlabs * RL + kSizeCls * RS + 3) & ~3;   // words, whole uint4s
   const int supn = 16 * W * (W + 1);
+  // Layout: nms_smem_bytes.  The sort scratch (tmp, hist, bstart) and the join's triangle (sup, unres) share one
+  // region: the rank loop fills crn / area / qlo / slidx and the tables while it still reads the sort scratch.
   u64* keys = reinterpret_cast<u64*>(smem_raw);                 // [sortn]
-  float4* crn = reinterpret_cast<float4*>(keys + sortn);        // [mcap] x1,y1,x2,y2 (sort scratch: sortn keys)
-  u32* hist = reinterpret_cast<u32*>(crn + mcap);               // [256] sort / select histogram
-  u32* bstart = hist + 256;                                     // [256] rank sort: first slot of each bucket
-  u32* tab = hist;                                              // [kSlabs][RL] interval tables of the join (after the sort)
-  u32* stab = tab + max(512, kSlabs * RL);                      // [kSizeCls][RS] width / height class neighbourhoods
+  float4* crn = reinterpret_cast<float4*>(keys + sortn);        // [mcap] x1,y1,x2,y2
+  u32* tab = reinterpret_cast<u32*>(crn + mcap);                // [kSlabs][RL] interval tables of the join
+  u32* stab = tab + kSlabs * RL;                                // [kSizeCls][RS] width / height class neighbourhoods
   float* qlo = reinterpret_cast<float*>(tab + tabn);            // [mcap] q*area*0.9999
   float* area = qlo + mcap;                                     // [mcap]
   u32* slidx = reinterpret_cast<u32*>(area + mcap);             // [mcap] slab intervals and size classes of the box
+  u64* tmp = reinterpret_cast<u64*>(slidx + mcap);              // [sortn] rank sort: keys grouped by bucket
+  u32* hist = reinterpret_cast<u32*>(tmp + sortn);              // [256] sort / select histogram
+  u32* bstart = hist + 256;                                     // [256] rank sort: first slot of each bucket
   u32* sup = slidx + mcap;                                      // lower triangle, [group g][word w <= g][row of the group]
   u32* unres = sup + supn;                                      // [mcap] the open rows, listed
-  float* dom = reinterpret_cast<float*>(unres + mcap);          // [4*kNmsWarps] per-warp extents of the boxes
-  u32* mm = reinterpret_cast<u32*>(dom + 4 * kNmsWarps);        // [4*kNmsWarps] per-warp min/max of the score and prior words
-  u32* keptw = mm + 4 * kNmsWarps;                              // [W]
+  u32* keptw = slidx + mcap + max(2 * sortn + 512, supn + mcap);   // [W]
   u32* remw = keptw + W;                                        // [W]
   u32* openw = remw + W;                                        // [W] rows with at least one suppressor
+  u32* wpre = openw + W;                                        // [W + 1] kept boxes before word w
   __shared__ u64 sel_prefix;
   __shared__ int sel_k, sel_fill;
 
@@ -571,21 +586,33 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     return base;
   };
 
-  // Lists up to the sort width (all but pathological ones) go straight into the sort buffer; a longer one keeps its
-  // first sortn keys there only until the select below refills the buffer.
-  u32 hmin = ~0u, hmax = 0u, lmin = ~0u, lmax = 0u;   // range of the score and prior words of the keys
+  // Sort histogram and join tables start at zero (neither shares memory with anything the key load writes).
+  NMS_LOOP
+  for (int i = tid; i < (tabn >> 2) + 64; i += kNmsThreads)
+    reinterpret_cast<uint4*>(i < (tabn >> 2) ? tab : hist - tabn)[i] = make_uint4(0u, 0u, 0u, 0u);
+  if (tid < W) { remw[tid] = 0u; openw[tid] = 0u; }
+  __syncthreads();
+  // Rank-sort buckets (head of the kernel): first fixed over the score words above the threshold's.
+  bool byscore = true;
+  u32 kbase = P.key_base;
+  float kscale = P.key_scale;
+  auto bucket = [&](u64 v) {   // the clamp, the conversions, the product and the truncation are all monotone
+    const u32 x = byscore ? (u32)(v >> 32) : (u32)v;
+    return min(255, (int)((float)(max(x, kbase) - kbase) * kscale));
+  };
+  // Lists up to the sort width (all but pathological ones) go straight into the sort buffer and its histogram; a
+  // longer one keeps its first sortn keys there only until the select below refills the buffer.
   int n = for_keys([&](u64 v, int i) {
-    if (i < sortn) keys[i] = v;
-    hmin = min(hmin, (u32)(v >> 32)); hmax = max(hmax, (u32)(v >> 32));
-    lmin = min(lmin, (u32)v); lmax = max(lmax, (u32)v);
+    if (i < sortn) {
+      keys[i] = v;
+      atomicAdd(&hist[bucket(v)], 1u);
+    }
   });
   const bool selected = n > P.sortn;   // more candidates than the sort takes: radix select first
+  __syncthreads();
   if (selected) {
-    hmin = ~0u; hmax = 0u; lmin = ~0u; lmax = 0u;   // taken again from the selected keys
-    __syncthreads();
     // Radix select of the top_k-th largest composite key (keys are unique), 8 bits per pass.
     if (tid == 0) { sel_prefix = 0ull; sel_k = P.top_k; sel_fill = 0; }
-    __syncthreads();
     for (int shift = 56; shift >= 0; shift -= 8) {
       NMS_LOOP
       for (int i = tid; i < 256; i += kNmsThreads) hist[i] = 0u;
@@ -618,169 +645,129 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     __syncthreads();
     n = min(sel_fill, sortn);
   }
-  // Rank sort, descending (keys are unique), see the head of the kernel.
-  {
-    u64* tmp = reinterpret_cast<u64*>(crn);   // [n] keys grouped by bucket; crn is filled after the sort
-    NMS_LOOP
-    for (int i = tid; i < 256; i += kNmsThreads) hist[i] = 0u;
-    if (selected) {   // the keys came out of the select: scan them
+  // The histogram is rebuilt for the keys the select left, and once more, over the keys' own range, when every key
+  // sits in one bucket (all scores equal, or within one bucket's width: the count loop would be quadratic).
+  for (bool redo = selected, ranged = false;;) {
+    if (redo) {
       NMS_LOOP
-      for (int i = tid; i < n; i += kNmsThreads) {
-        const u64 v = keys[i];
-        hmin = min(hmin, (u32)(v >> 32)); hmax = max(hmax, (u32)(v >> 32));
-        lmin = min(lmin, (u32)v); lmax = max(lmax, (u32)v);
-      }
+      for (int i = tid; i < 256; i += kNmsThreads) hist[i] = 0u;
+      __syncthreads();
+      NMS_LOOP
+      for (int i = tid; i < n; i += kNmsThreads) atomicAdd(&hist[bucket(keys[i])], 1u);
+      __syncthreads();
     }
-    hmin = __reduce_min_sync(SSDG_FULL, hmin); hmax = __reduce_max_sync(SSDG_FULL, hmax);
-    lmin = __reduce_min_sync(SSDG_FULL, lmin); lmax = __reduce_max_sync(SSDG_FULL, lmax);
-    if (lane == 0) reinterpret_cast<uint4*>(mm)[warp] = make_uint4(hmin, hmax, lmin, lmax);
-    __syncthreads();
-    {
-      const uint4 p0 = reinterpret_cast<const uint4*>(mm)[0];
-      hmin = p0.x; hmax = p0.y; lmin = p0.z; lmax = p0.w;
-#pragma unroll
-      for (int w = 1; w < kNmsWarps; ++w) {
-        const uint4 pw = reinterpret_cast<const uint4*>(mm)[w];
-        hmin = min(hmin, pw.x); hmax = max(hmax, pw.y); lmin = min(lmin, pw.z); lmax = max(lmax, pw.w);
-      }
-    }
-    const bool byscore = hmax > hmin;
-    const u32 kbase = byscore ? hmin : lmin;
-    const float kscale = __fdividef(256.f, (float)((byscore ? hmax : lmax) - kbase) + 1.f) * 0.999f;   // any monotone map sorts
-    auto bucket = [&](u64 v) {   // conversions, the product and the truncation are all monotone
-      const u32 x = (byscore ? (u32)(v >> 32) : (u32)v) - kbase;
-      return min(255, (int)((float)x * kscale));
-    };
-    NMS_LOOP
-    for (int i = tid; i < n; i += kNmsThreads) atomicAdd(&hist[bucket(keys[i])], 1u);
-    __syncthreads();
-    if (warp == 0) {   // start[b] = number of keys in buckets above b; lane l owns buckets 255-8l .. 248-8l
-      u32 c[8], tot = 0u;
-#pragma unroll
-      for (int r = 0; r < 8; ++r) { c[r] = hist[255 - 8 * lane - r]; tot += c[r]; }
-      u32 incl = tot;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const u32 v = __shfl_up_sync(SSDG_FULL, incl, o);
-        if (lane >= o) incl += v;
-      }
-      u32 run = incl - tot;
-#pragma unroll
-      for (int r = 0; r < 8; ++r) { bstart[255 - 8 * lane - r] = run; hist[255 - 8 * lane - r] = run; run += c[r]; }
-    }
-    __syncthreads();
+    if (ranged || n < 2 || (int)hist[bucket(keys[0])] < n) break;
+    u32 hmin = ~0u, hmax = 0u, lmin = ~0u, lmax = 0u;   // range of the score and prior words of the keys
     NMS_LOOP
     for (int i = tid; i < n; i += kNmsThreads) {
       const u64 v = keys[i];
-      tmp[atomicAdd(&hist[bucket(v)], 1u)] = v;   // hist[b] ends as the end of bucket b
+      hmin = min(hmin, (u32)(v >> 32)); hmax = max(hmax, (u32)(v >> 32));
+      lmin = min(lmin, (u32)v); lmax = max(lmax, (u32)v);
     }
+    hmin = __reduce_min_sync(SSDG_FULL, hmin); hmax = __reduce_max_sync(SSDG_FULL, hmax);
+    lmin = __reduce_min_sync(SSDG_FULL, lmin); lmax = __reduce_max_sync(SSDG_FULL, lmax);
+    uint4* mm = reinterpret_cast<uint4*>(bstart);   // [kNmsWarps] per-warp ranges (bstart is filled after this)
+    if (lane == 0) mm[warp] = make_uint4(hmin, hmax, lmin, lmax);
     __syncthreads();
-    NMS_LOOP
-    for (int i = tid; i < n; i += kNmsThreads) {
-      const u64 v = tmp[i];
-      const int bk = bucket(v);
-      const int s0 = (int)bstart[bk], s1 = (int)hist[bk];
-      int r = s0;
-#pragma unroll 1
-      for (int t = s0; t < s1; ++t) r += tmp[t] > v;
-      keys[r] = v;
+#pragma unroll
+    for (int w = 0; w < kNmsWarps; ++w) {
+      const uint4 pw = mm[w];
+      hmin = min(hmin, pw.x); hmax = max(hmax, pw.y); lmin = min(lmin, pw.z); lmax = max(lmax, pw.w);
     }
-    __syncthreads();
+    byscore = hmax > hmin;
+    kbase = byscore ? hmin : lmin;
+    kscale = __fdividef(256.f, (float)((byscore ? hmax : lmax) - kbase) + 1.f) * 0.999f;
+    redo = ranged = true;
   }
+  if (warp == 0) {   // start[b] = number of keys in buckets above b; lane l owns buckets 255-8l .. 248-8l
+    u32 c[8], tot = 0u;
+#pragma unroll
+    for (int r = 0; r < 8; ++r) { c[r] = hist[255 - 8 * lane - r]; tot += c[r]; }
+    u32 incl = tot;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const u32 v = __shfl_up_sync(SSDG_FULL, incl, o);
+      if (lane >= o) incl += v;
+    }
+    u32 run = incl - tot;
+#pragma unroll
+    for (int r = 0; r < 8; ++r) { bstart[255 - 8 * lane - r] = run; hist[255 - 8 * lane - r] = run; run += c[r]; }
+  }
+  __syncthreads();
+  NMS_LOOP
+  for (int i = tid; i < n; i += kNmsThreads) {
+    const u64 v = keys[i];
+    tmp[atomicAdd(&hist[bucket(v)], 1u)] = v;   // hist[b] ends as the end of bucket b
+  }
+  __syncthreads();
   const int m = min(n, P.top_k);
   const int mpad = (m + 31) & ~31;
   const int ngroups = mpad >> 5;
 
-  // Decoded boxes; corners in the formula's own float32 operations (utils/bbox.py:13-21).
-  // qa = q*(area + 0.5e-10):  iou > thr  <=>  inter > qa_i + qa_j  in exact arithmetic (positive denominator); boxes
-  // that can never overlap anything (w <= 0, h <= 0, non-finite, padding) get qa = +inf so the fast test rejects
-  // them exactly like the formula does (their intersection is 0).  The same pass collects what the join needs: the
-  // extents of all sane boxes (slab domain) and whether every box's corner extents reproduce its area to 0.1 %.
+  // Rank, then -- for the top_k ranks -- the box and its registration in the join tables (head of the kernel).
+  // Corners in the formula's own float32 operations (utils/bbox.py:13-21).  qa = q*(area + 0.5e-10):  iou > thr  <=>
+  // inter > qa_i + qa_j  in exact arithmetic (positive denominator); boxes that can never overlap anything (w <= 0,
+  // h <= 0, non-finite) get qa = +inf and no registration, so the fast test rejects them exactly like the formula
+  // does (their intersection is 0).  Rows m .. mpad are left unprepared: no test uses them.
   const float thr = P.iou_thresh;
   const bool fast_ok = P.fast_ok != 0;
   const float q = P.q;
-  int inexact = 0;
-  float x1 = CUDART_INF_F, y1 = CUDART_INF_F, x2 = -CUDART_INF_F, y2 = -CUDART_INF_F;   // extents of the sane boxes
   NMS_LOOP
-  for (int i = tid; i < mpad; i += kNmsThreads) {
-    float4 cr = make_float4(0.f, 0.f, 0.f, 0.f);
-    float ar = 0.f, qa = CUDART_INF_F;
-    if (i < m) {
-      const int a = (int)(~(u32)keys[i]);
-      const float4 bx = __ldg(reinterpret_cast<const float4*>(P.boxes) + (size_t)b * P.A + a);
-      const float hw = __fmul_rn(bx.z, 0.5f), hh = __fmul_rn(bx.w, 0.5f);
-      cr = make_float4(__fsub_rn(bx.x, hw), __fsub_rn(bx.y, hh), __fadd_rn(bx.x, hw), __fadd_rn(bx.y, hh));
-      ar = __fmul_rn(bx.z, bx.w);
-      const bool sane = bx.z > 0.f && bx.w > 0.f && isfinite(cr.x) && isfinite(cr.y) && isfinite(cr.z) &&
-                        isfinite(cr.w) && isfinite(ar);
-      if (sane) {
-        qa = q * (ar + 0.5e-10f);
-        const float pr = (cr.z - cr.x) * (cr.w - cr.y);
-        inexact |= !(ar >= 0.999f * pr && ar <= 1.001f * pr);
-        x1 = fminf(x1, cr.x); y1 = fminf(y1, cr.y); x2 = fmaxf(x2, cr.z); y2 = fmaxf(y2, cr.w);
-      }
-    }
-    crn[i] = cr;
-    area[i] = ar;
-    qlo[i] = qa * 0.9999f;
-  }
-  {
-    const u32 k1 = __reduce_min_sync(SSDG_FULL, key32(x1)), k2 = __reduce_min_sync(SSDG_FULL, key32(y1));
-    const u32 k3 = __reduce_max_sync(SSDG_FULL, key32(x2)), k4 = __reduce_max_sync(SSDG_FULL, key32(y2));
-    if (lane == 0) reinterpret_cast<float4*>(dom)[warp] = make_float4(unkey32(k1), unkey32(k2), unkey32(k3), unkey32(k4));
-  }
-  NMS_LOOP
-  for (int i = tid; i < W; i += kNmsThreads) { remw[i] = 0u; openw[i] = 0u; }
-  // the sort is done with hist / bstart: the join tables take their place
-  NMS_LOOP
-  for (int i = tid; i < (tabn >> 2); i += kNmsThreads) reinterpret_cast<uint4*>(tab)[i] = make_uint4(0u, 0u, 0u, 0u);
-  inexact = __syncthreads_or(inexact);
-
-  if (fast_ok) {
-    // Slab join + size classes (derivation at the head of the kernel).
-    float dx0, dy0, dsx, dsy, lwx, lwy;
-    {
-      float4 e = reinterpret_cast<const float4*>(dom)[0];
-#pragma unroll
-      for (int w = 1; w < kNmsWarps; ++w) {
-        const float4 f = reinterpret_cast<const float4*>(dom)[w];
-        e.x = fminf(e.x, f.x); e.y = fminf(e.y, f.y); e.z = fmaxf(e.z, f.z); e.w = fmaxf(e.w, f.w);
-      }
-      dx0 = e.x; dy0 = e.y;
-      // any positive scale keeps the slab map monotone; 0.999 keeps the largest coordinate inside the last slab
-      dsx = (e.z > e.x) ? __fdividef((float)kSlabs * 0.999f, e.z - e.x) : 0.f;
-      dsy = (e.w > e.y) ? __fdividef((float)kSlabs * 0.999f, e.w - e.y) : 0.f;
-      lwx = (e.z > e.x) ? __log2f(e.z - e.x) : 0.f;
-      lwy = (e.w > e.y) ? __log2f(e.w - e.y) : 0.f;
-    }
-    auto slab = [&](float v, float o, float sc) {   // monotone in v (the conversion saturates, NaN -> 0)
-      return min(max(__float2int_rd((v - o) * sc), 0), kSlabs - 1);
-    };
-    const float tq = inexact ? 0.f : P.tq0;
-    const float inv_l = inexact ? 0.f : P.inv_l;
-    auto size_cls = [&](float ext, float lref) {   // monotone in ext, clamped (clamping only merges classes)
-      return min(max(__float2int_rd((lref - __log2f(ext)) * inv_l), 0), kSizeCls - 1);
-    };
-    NMS_LOOP
-    for (int i = tid; i < m; i += kNmsThreads) {
-      if (!isfinite(qlo[i])) { slidx[i] = 0u; continue; }
-      const float4 c = crn[i];
-      const u32 bit = 1u << (i & 31);
-      const int wi = i >> 5;
+  for (int i = tid; i < n; i += kNmsThreads) {
+    const u64 v = tmp[i];
+    const float4 bx = __ldg(reinterpret_cast<const float4*>(P.boxes) + (size_t)b * P.A + (int)(~(u32)v));
+    const int bk = bucket(v);
+    const int s0 = (int)bstart[bk], s1 = (int)hist[bk];
+    int r = s0;
+#pragma unroll 1
+    for (int t = s0; t < s1; ++t) r += tmp[t] > v;
+    if (r >= m) continue;
+    keys[r] = v;
+    const float hw = __fmul_rn(bx.z, 0.5f), hh = __fmul_rn(bx.w, 0.5f);
+    const float4 c = make_float4(__fsub_rn(bx.x, hw), __fsub_rn(bx.y, hh), __fadd_rn(bx.x, hw), __fadd_rn(bx.y, hh));
+    const float ar = __fmul_rn(bx.z, bx.w);
+    crn[r] = c;
+    area[r] = ar;
+    float qa = CUDART_INF_F;
+    u32 sl = 0u;
+    if (bx.z > 0.f && bx.w > 0.f && isfinite(c.x) && isfinite(c.y) && isfinite(c.z) && isfinite(c.w) && isfinite(ar)) {
+      qa = q * (ar + 0.5e-10f);
+      const float pr = (c.z - c.x) * (c.w - c.y);
+      const bool exact = ar >= 0.999f * pr && ar <= 1.001f * pr;   // see the head of the kernel for an inexact box
+      const float tq = exact ? P.tq0 : 0.f;
+      auto slab = [&](float u) {   // monotone in u (the conversion saturates, NaN -> 0)
+        return min(max(__float2int_rd(u * (float)kSlabs), 0), kSlabs - 1);
+      };
+      auto size_cls = [&](float ext) {   // monotone in ext, clamped (clamping only merges classes)
+        return exact ? min(max(__float2int_rd(-__log2f(ext) * P.inv_l), 0), kSizeCls - 1) : kSizeCls - 1;
+      };
       const float sx = tq * (c.z - c.x) - 1e-6f * (fabsf(c.x) + fabsf(c.z));
       const float sy = tq * (c.w - c.y) - 1e-6f * (fabsf(c.y) + fabsf(c.w));
-      const int ax = slab(c.x + sx, dx0, dsx), bx = max(slab(c.z - sx, dx0, dsx), ax);
-      const int ay = slab(c.y + sy, dy0, dsy), by = max(slab(c.w - sy, dy0, dsy), ay);
-      const int cw = inv_l > 0.f ? size_cls(c.z - c.x, lwx) : 0, ch = inv_l > 0.f ? size_cls(c.w - c.y, lwy) : 0;
-      slidx[i] = (u32)ax | ((u32)bx << 5) | ((u32)ay << 10) | ((u32)by << 15) | ((u32)cw << 20) | ((u32)ch << 24) | 0x80000000u;
+      const int ax = slab(c.x + sx), bx_ = max(slab(c.z - sx), ax);
+      const int ay = slab(c.y + sy), by = max(slab(c.w - sy), ay);
+      const int cw = size_cls(c.z - c.x), ch = size_cls(c.w - c.y);
+      sl = (u32)ax | ((u32)bx_ << 5) | ((u32)ay << 10) | ((u32)by << 15) | ((u32)cw << 20) | ((u32)ch << 24) |
+           (exact ? 0u : 0x40000000u) | 0x80000000u;
+      const u32 bit = 1u << (r & 31);
+      const int wi = r >> 5;
       atomicOr(&tab[ax * RL + wi], bit);
-      atomicOr(&tab[bx * RL + W + wi], bit);
+      atomicOr(&tab[bx_ * RL + W + wi], bit);
       atomicOr(&tab[ay * RL + 2 * W + wi], bit);
       atomicOr(&tab[by * RL + 3 * W + wi], bit);
-      atomicOr(&stab[cw * RS + wi], bit);
-      atomicOr(&stab[ch * RS + W + wi], bit);
+#pragma unroll 1
+      for (int k = exact ? 0 : kSizeCls - 1; k >= 0; --k) {   // an inexact box goes into every class
+        atomicOr(&stab[(cw - k) * RS + wi], bit);
+        atomicOr(&stab[(ch - k) * RS + W + wi], bit);
+      }
     }
-    __syncthreads();
+    qlo[r] = qa * 0.9999f;
+    slidx[r] = sl;
+  }
+  __syncthreads();
+
+  if (fast_ok) {
+    // Slab join + size classes (derivation at the head of the kernel): running ORs along the slabs, class
+    // neighbourhoods.
     NMS_LOOP
     for (int col = tid; col < 6 * W; col += kNmsThreads) {
       if (col < 4 * W) {
@@ -820,8 +807,10 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
       const u32* gex = tab + (si & 31u) * RL + W;                // GEx[a_i]
       const u32* ley = tab + ((si >> 15) & 31u) * RL + 2 * W;    // LEy[b_i]
       const u32* gey = tab + ((si >> 10) & 31u) * RL + 3 * W;    // GEy[a_i]
-      const u32* szw = stab + ((si >> 20) & 15u) * RS;           // width classes next to the row's
-      const u32* szh = stab + ((si >> 24) & 15u) * RS + W;       // height classes
+      // width / height classes next to the row's; an inexact row (bit 30) takes every size: LEx / LEy again
+      const bool inx = (si & 0x40000000u) != 0u;
+      const u32* szw = inx ? lex : stab + ((si >> 20) & 15u) * RS;
+      const u32* szh = inx ? ley : stab + ((si >> 24) & 15u) * RS + W;
       u32* myrow = sup + 16 * gi * (gi + 1) + lane;              // slot of word w: myrow[32 w]
       u32 any = 0u;
       if (kW > 0) {
@@ -916,7 +905,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
 
   // Closed rows are kept at once.  The open ones: fixed point of  kept(i) <=> no kept j < i with sup(i, j);
   // removed(i) <=> some kept j < i with sup(i, j), by one warp (a handful of rows per list: no CTA-wide barrier per
-  // round); then hist[w] = kept boxes before word w for the output.
+  // round); then wpre[w] = kept boxes before word w for the output.
   if (warp == 0) {
     const u32 ow = lane < W ? openw[lane] : 0u;
     const u32 lm = m >= 32 * (lane + 1) ? ~0u : (m > 32 * lane ? (1u << (m - 32 * lane)) - 1u : 0u);
@@ -966,13 +955,13 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
       const int v = __shfl_up_sync(SSDG_FULL, incl, o);
       if (lane >= o) incl += v;
     }
-    if (lane < W) hist[lane] = (u32)(incl - c);   // W <= 32 (shared memory limits sortn to 1024)
-    if (lane == 31) hist[W] = (u32)incl;
+    if (lane < W) wpre[lane] = (u32)(incl - c);   // W <= 32 (shared memory limits sortn to 1024)
+    if (lane == 31) wpre[W] = (u32)incl;
   }
   __syncthreads();
   int* ok = P.out_kept + list * (size_t)P.top_k;
   float* os = P.out_score ? P.out_score + list * (size_t)P.top_k : nullptr;
-  const int total = (int)hist[W];
+  const int total = (int)wpre[W];
   for (int i = total + tid; i < P.top_k; i += kNmsThreads) {
     ok[i] = -1;
     if (os) os[i] = 0.f;
@@ -981,7 +970,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
   for (int i = tid; i < m; i += kNmsThreads) {
     const u32 kw = keptw[i >> 5], bit = 1u << (i & 31);
     if (kw & bit) {
-      const int rank = (int)hist[i >> 5] + __popc(kw & (bit - 1u));
+      const int rank = (int)wpre[i >> 5] + __popc(kw & (bit - 1u));
       ok[rank] = (int)(~(u32)keys[i]);
       if (os) os[rank] = unkey32((u32)(keys[i] >> 32));
     }
@@ -1026,11 +1015,12 @@ static int next_pow2(int v) {
   while (p < v) p <<= 1;
   return p;
 }
-static size_t nms_smem_bytes(int sortn, int top_k) {
+static size_t nms_smem_bytes(int sortn, int top_k) {   // the layout at the head of nms_kernel
   const int mcap = (top_k + 31) & ~31, W = mcap / 32, RL = (4 * W) | 1;
-  const size_t tab = (size_t)kSlabs * RL > 512 ? (size_t)kSlabs * RL : 512;   // hist + bstart, then the join tables
-  return (size_t)sortn * 8 + (size_t)mcap * (16 + 4 + 4 + 4) + (size_t)16 * W * (W + 1) * 4 + 3 * W * 4 +
-         (size_t)mcap * 4 + 9 * kNmsWarps * 4 + tab * 4 + (size_t)kSizeCls * ((2 * W) | 1) * 4 + 16 + 128;
+  const size_t tabn = ((size_t)kSlabs * RL + (size_t)kSizeCls * ((2 * W) | 1) + 3) & ~(size_t)3;
+  const size_t sort = (size_t)2 * sortn + 512, join = (size_t)16 * W * (W + 1) + mcap;   // words of the shared region
+  return (size_t)sortn * 8 + (size_t)mcap * (16 + 4 + 4 + 4) + tabn * 4 + std::max(sort, join) * 4 +
+         (size_t)(4 * W + 1) * 4 + 16 + 128;
 }
 
 struct DetectWs {
@@ -1080,8 +1070,17 @@ static int run_filter(DetectParams& P, DetectMode mode, int prior_dtype, cudaStr
   return SSDG_OK;
 }
 
-static int run_nms(const DetectWs& ws, const float* boxes, long long batch, int A, int C, int top_k, float iou_thresh,
-                   int* out_kept, int* out_count, float* out_score, cudaStream_t st) {
+// key32 of the device code (common.cuh) on the host
+static u32 host_key32(float v) {
+  if (v != v) return ~0u;
+  if (v == 0.0f) v = 0.0f;
+  u32 b;
+  std::memcpy(&b, &v, 4);
+  return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
+}
+
+static int run_nms(const DetectWs& ws, const float* boxes, long long batch, int A, int C, int top_k, float score_thresh,
+                   float iou_thresh, int* out_kept, int* out_count, float* out_score, cudaStream_t st) {
   FilterGeom g;
   if (!filter_geom(batch, A, C, &g)) return SSDG_ERR_LIMIT;
   NmsParams Q;
@@ -1098,6 +1097,9 @@ static int run_nms(const DetectWs& ws, const float* boxes, long long batch, int 
     const float tp = 0.99f * iou_thresh / (1.f + 0.001f * iou_thresh);
     Q.inv_l = (Q.fast_ok && tp < 0.98f) ? -1.f / log2f(tp) : 0.f;
   }
+  // The filter lists only scores > score_thresh; softmax scores are <= 1 (larger ones share the last bucket).
+  Q.key_base = host_key32(score_thresh);
+  Q.key_scale = 256.f / (float)std::max<long long>((long long)host_key32(1.f) - (long long)Q.key_base, 256);
   const size_t smem = nms_smem_bytes(Q.sortn, top_k);
   if ((int)smem > max_smem_optin()) return SSDG_ERR_LIMIT;
   auto go = [&](auto kern) -> int {
@@ -1414,7 +1416,8 @@ static int detect_run(DetectMode mode, int stages, const float* scores, const fl
     if (rc) return rc;
   }
   if (stages & kDetectNms)
-    return run_nms(ws, P.boxes, batch, n_priors, n_classes, top_k, iou_thresh, out_kept, out_count, out_kept_score, st);
+    return run_nms(ws, P.boxes, batch, n_priors, n_classes, top_k, score_thresh, iou_thresh, out_kept, out_count,
+                   out_kept_score, st);
   return SSDG_OK;
 }
 
