@@ -481,6 +481,32 @@ struct NmsParams {
 // The NMS kernel is instruction-cache sensitive (12 CTAs per SM in different phases): its block-stride loops
 // stay rolled (3280 -> 2240 SASS instructions, 7% faster).
 #define NMS_LOOP _Pragma("unroll 1")
+
+// Phase attribution (build with SSDG_EXTRA_NVCC_FLAGS=-DSSDG_NMS_TIMING; profiles/nms_phase_timing.py): thread 0 of
+// every CTA reads clock64 after the barrier that ends each phase, the two join passes are clocked per warp, and the
+// counts each phase scales with are summed in shared memory; one flush per CTA into g_nms_timing, read (and zeroed)
+// by ssdg_nms_timing.  The default build contains none of it.
+enum NmsTiming {
+  NT_LOAD, NT_SELECT, NT_SCATTER, NT_RANK, NT_OR, NT_JOIN, NT_RESOLVE, NT_OUTPUT,   // CTA cycles per phase
+  NT_PASS_A, NT_PASS_B,                 // warp cycles of the two join passes (summed over the warps)
+  NT_LISTS, NT_KEYS, NT_SELECTED, NT_ROWS,   // lists, keys loaded, lists through the select, rows kept for the join
+  NT_COUNT_STEPS, NT_COUNT_TRIPS,       // count loop: steps summed over threads; trips of the warps (max over lanes)
+  NT_A_WORDS,                           // pass A: column words ANDed (per row group)
+  NT_B_PAIRS, NT_B_TRIPS, NT_B_WORDS,   // pass B: candidate pairs; trips of the warps; (row, word)s with candidates
+  NT_SUPPRESS, NT_OPEN, NT_ROUNDS,      // suppressing pairs; open rows; resolution rounds
+  NT_RANK_COUNT, NT_RANK_BOX,           // rank loop, warp cycles: key + count loop; box wait + preparation + registration
+  NT_SLOTS = 32
+};
+#ifdef SSDG_NMS_TIMING
+__device__ unsigned long long g_nms_timing[NT_SLOTS];
+#define NMS_TICK(slot) do { if (tid == 0) { const long long n_ = clock64(); atomicAdd(&nt_acc[slot], (unsigned long long)(n_ - nt_t0)); nt_t0 = n_; } } while (0)
+#define NMS_COUNT(slot, v) atomicAdd(&nt_acc[slot], (unsigned long long)(v))
+#define NMS_TIMING_ONLY(...) __VA_ARGS__
+#else
+#define NMS_TICK(slot) do { } while (0)
+#define NMS_COUNT(slot, v) do { } while (0)
+#define NMS_TIMING_ONLY(...)
+#endif
 // Structure (128 threads per list, ~17.8 KB shared memory, <= 40 registers => 12 CTAs per SM; the kernel is
 // issue- and barrier-bound, profiles/r20_*, r25_*):
 //   * the list is the concatenation of the runs the filter CTAs left in its slots; the counts of up to four runs
@@ -513,8 +539,9 @@ struct NmsParams {
 //     i (a_j > 0 for a registered box), so both terms are positive (same in y).  Two inexact boxes are both unshrunk
 //     and meet whenever inter > 0.  Thresholds <= 0 or huge use all pairs with the formula;
 //   * the join runs per group of 32 rows in two passes (candidate words as straight-line code when the word count
-//     is a template constant, then the pair tests), the groups dealt to the warps in pairs (last + first, ...):
-//     group g costs g + 1 words, so every warp gets the same number of word steps;
+//     is a template constant, then the pair tests, each lane walking its row's candidates through all its words),
+//     the groups dealt to the warps in pairs (last + first, ...): group g costs g + 1 words, so every warp gets the
+//     same number of word steps;
 //   * rows without a suppressor are kept at once; the others (a handful) are listed and resolved by ONE warp
 //     iterating the fixed point of kept(i) <=> no kept j < i suppresses i -- identical to the sequential greedy by
 //     induction on i, no CTA-wide barrier per round.  The suppression matrix is the lower triangle only,
@@ -552,6 +579,11 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
 
   const int b = (int)(blockIdx.z * 65535u + blockIdx.y);        // grid (class, image mod 65535, image / 65535)
   if (b >= P.B) return;
+#ifdef SSDG_NMS_TIMING
+  __shared__ unsigned long long nt_acc[NT_SLOTS];
+  long long nt_t0 = clock64();
+  if (tid < NT_SLOTS) nt_acc[tid] = 0ull;
+#endif
   const size_t list = (size_t)b * P.n_fg + blockIdx.x;
   // The list is the concatenation of the runs the filter CTAs left in its slots (prior space, DetectParams).
   // f(key, index in the list) for every key, block-strided; returns the length.  Everything is derived inside (the
@@ -610,6 +642,8 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
   });
   const bool selected = n > P.sortn;   // more candidates than the sort takes: radix select first
   __syncthreads();
+  NMS_TICK(NT_LOAD);
+  if (tid == 0) { NMS_COUNT(NT_LISTS, 1); NMS_COUNT(NT_KEYS, n); NMS_COUNT(NT_SELECTED, selected); }
   if (selected) {
     // Radix select of the top_k-th largest composite key (keys are unique), 8 bits per pass.
     if (tid == 0) { sel_prefix = 0ull; sel_k = P.top_k; sel_fill = 0; }
@@ -679,6 +713,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     kscale = __fdividef(256.f, (float)((byscore ? hmax : lmax) - kbase) + 1.f) * 0.999f;
     redo = ranged = true;
   }
+  NMS_TICK(NT_SELECT);
   if (warp == 0) {   // start[b] = number of keys in buckets above b; lane l owns buckets 255-8l .. 248-8l
     u32 c[8], tot = 0u;
 #pragma unroll
@@ -700,6 +735,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     tmp[atomicAdd(&hist[bucket(v)], 1u)] = v;   // hist[b] ends as the end of bucket b
   }
   __syncthreads();
+  NMS_TICK(NT_SCATTER);
   const int m = min(n, P.top_k);
   const int mpad = (m + 31) & ~31;
   const int ngroups = mpad >> 5;
@@ -714,6 +750,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
   const float q = P.q;
   NMS_LOOP
   for (int i = tid; i < n; i += kNmsThreads) {
+    NMS_TIMING_ONLY(const long long nt_r0 = clock64();)
     const u64 v = tmp[i];
     const float4 bx = __ldg(reinterpret_cast<const float4*>(P.boxes) + (size_t)b * P.A + (int)(~(u32)v));
     const int bk = bucket(v);
@@ -721,6 +758,12 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     int r = s0;
 #pragma unroll 1
     for (int t = s0; t < s1; ++t) r += tmp[t] > v;
+    NMS_TIMING_ONLY({   // (__activemask: the lanes still in the loop, not necessarily converged -- these per-warp
+                        // trips, and the rank cycles below, are approximate)
+      const u32 am = __activemask(), tr = __reduce_max_sync(am, (u32)(s1 - s0)), st = __reduce_add_sync(am, (u32)(s1 - s0));
+      if (lane == __ffs(am) - 1) { NMS_COUNT(NT_COUNT_TRIPS, tr); NMS_COUNT(NT_COUNT_STEPS, st); }
+    })
+    NMS_TIMING_ONLY(const long long nt_r1 = clock64();)
     if (r >= m) continue;
     keys[r] = v;
     const float hw = __fmul_rn(bx.z, 0.5f), hh = __fmul_rn(bx.w, 0.5f);
@@ -762,40 +805,57 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     }
     qlo[r] = qa * 0.9999f;
     slidx[r] = sl;
+    NMS_TIMING_ONLY({
+      const long long nt_r2 = clock64();
+      const u32 am = __activemask();
+      const u32 c = __reduce_max_sync(am, (u32)(nt_r1 - nt_r0)), p = __reduce_max_sync(am, (u32)(nt_r2 - nt_r1));
+      if (lane == __ffs(am) - 1) { NMS_COUNT(NT_RANK_COUNT, c); NMS_COUNT(NT_RANK_BOX, p); }
+    })
   }
   __syncthreads();
+  NMS_TICK(NT_RANK);
+  if (tid == 0) NMS_COUNT(NT_ROWS, m);
 
   if (fast_ok) {
     // Slab join + size classes (derivation at the head of the kernel): running ORs along the slabs, class
     // neighbourhoods.
     NMS_LOOP
     for (int col = tid; col < 6 * W; col += kNmsThreads) {
+      // (the words of a column are loaded into registers before any is stored: a load after a store to the same
+      // column would wait for it, one shared-memory round trip per slab)
       if (col < 4 * W) {
         const bool up = ((col / W) & 1) == 0;   // LE: ascending running OR, GE: descending
+        const int step = up ? RL : -RL;
+        u32* p = tab + col + (up ? 0 : (kSlabs - 1) * RL);
         u32 acc = 0u;
-#pragma unroll 8
-        for (int k = 0; k < kSlabs; ++k) {
-          const int sl = up ? k : kSlabs - 1 - k;
-          acc |= tab[sl * RL + col];
-          tab[sl * RL + col] = acc;
+#pragma unroll 1
+        for (int k = 0; k < kSlabs; k += 8, p += 8 * step) {
+          u32 v[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) v[e] = p[e * step];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) { acc |= v[e]; p[e * step] = acc; }
         }
       } else {
         u32* sc = stab + (col - 4 * W);
         u32 prev = 0u, cur = sc[0];
-#pragma unroll 4
-        for (int k = 0; k < kSizeCls; ++k) {
-          const u32 nxt = k + 1 < kSizeCls ? sc[(k + 1) * RS] : 0u;
-          sc[k * RS] = prev | cur | nxt;
-          prev = cur; cur = nxt;
+#pragma unroll 1
+        for (int k = 0; k < kSizeCls; k += 8) {
+          u32 v[8];
+#pragma unroll
+          for (int e = 0; e < 8; ++e) v[e] = k + e + 1 < kSizeCls ? sc[(k + e + 1) * RS] : 0u;
+#pragma unroll
+          for (int e = 0; e < 8; ++e) { sc[(k + e) * RS] = prev | cur | v[e]; prev = cur; cur = v[e]; }
         }
       }
     }
     __syncthreads();
+    NMS_TICK(NT_OR);
     // The join proper, per group of 32 rows (lane = row), in two passes over the column words w <= g:
     //   A  candidate words = AND of the six table words -- straight-line code when the word count is a template
     //      constant (immediate offsets, no address arithmetic), parked in the row's slots of the triangle;
-    //   B  the candidates of each word get the cheap float test (1e-4 margin), survivors the formula itself -- IEEE
-    //      float32, no contraction (utils/bbox.py:13-25); the word is rewritten with the real suppressions.
+    //   B  every candidate gets the cheap float test (1e-4 margin), survivors the formula itself -- IEEE float32, no
+    //      contraction (utils/bbox.py:13-25); each word is rewritten with the real suppressions.
     // Rows that end without a suppressor stay closed (kept at once); the others are opened for the resolution.
     const u32 ltmask = (1u << lane) - 1u;
     auto join_group = [&](int gi) {
@@ -812,7 +872,8 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
       const u32* szw = inx ? lex : stab + ((si >> 20) & 15u) * RS;
       const u32* szh = inx ? ley : stab + ((si >> 24) & 15u) * RS + W;
       u32* myrow = sup + 16 * gi * (gi + 1) + lane;              // slot of word w: myrow[32 w]
-      u32 any = 0u;
+      NMS_TIMING_ONLY(long long nt_w0 = clock64(); u32 nt_pairs = 0u;)
+      u32 wm = 0u;   // the row's words that hold candidates
       if (kW > 0) {
 #pragma unroll
         for (int w = 0; w < kW; ++w) {
@@ -820,7 +881,8 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
             u32 cand = lex[w] & gex[w] & ley[w] & gey[w] & szw[w] & szh[w] & smask;
             if (w == gi) cand &= ltmask;
             myrow[w << 5] = cand;
-            any |= cand;
+            if (cand) wm |= 1u << w;
+            NMS_TIMING_ONLY(nt_pairs += __popc(cand);)
           }
         }
       } else {
@@ -829,38 +891,64 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
           u32 cand = lex[w] & gex[w] & ley[w] & gey[w] & szw[w] & szh[w] & smask;
           if (w == gi) cand &= ltmask;
           myrow[w << 5] = cand;
-          any |= cand;
+          if (cand) wm |= 1u << w;
+          NMS_TIMING_ONLY(nt_pairs += __popc(cand);)
         }
       }
-      if (!__any_sync(SSDG_FULL, any != 0u)) return;
+      NMS_TIMING_ONLY({
+        __syncwarp();
+        const long long n_ = clock64();
+        const u32 tr = __reduce_max_sync(SSDG_FULL, nt_pairs), np = __reduce_add_sync(SSDG_FULL, nt_pairs);
+        const u32 nw = __reduce_add_sync(SSDG_FULL, (u32)__popc(wm));
+        if (lane == 0) {
+          NMS_COUNT(NT_PASS_A, n_ - nt_w0); NMS_COUNT(NT_A_WORDS, gi + 1);
+          NMS_COUNT(NT_B_TRIPS, tr); NMS_COUNT(NT_B_PAIRS, np); NMS_COUNT(NT_B_WORDS, nw);
+        }
+        nt_w0 = n_;
+      })
+      if (!__any_sync(SSDG_FULL, wm != 0u)) return;
       const float4 bi = live ? crn[i] : make_float4(0.f, 0.f, 0.f, 0.f);
       const float qi_lo = live ? qlo[i] : 0.f;
       const float ai = live ? area[i] : 0.f;
-      any = 0u;
+      NMS_TIMING_ONLY(u32 nt_sup = 0u;)
+      // Each lane walks the candidates of its own row through all its words, one pair per trip: the warp runs the
+      // largest candidate count of its rows, not the sum over the words of each word's largest count, and casts no
+      // vote per word.  A word is rewritten with its real suppressions after its last candidate.
+      u32 any = 0u, cand = 0u, bits = 0u;
+      int w = 0;
 #pragma unroll 1
-      for (int w = 0; w <= gi; ++w) {
-        u32 cand = myrow[w << 5];
-        if (!__any_sync(SSDG_FULL, cand != 0u)) continue;
-        u32 bits = 0u;
-        while (cand) {
-          const int jj = __ffs(cand) - 1;
-          cand &= cand - 1;
-          const int j = (w << 5) + jj;
-          const float4 bj = crn[j];
-          const float lox = fmaxf(bi.x, bj.x), hix = fminf(bi.z, bj.z), loy = fmaxf(bi.y, bj.y), hiy = fminf(bi.w, bj.w);
-          const float fx = hix - lox, fy = hiy - loy;
-          if (!(fx > 0.f && fx * fy >= qi_lo + qlo[j])) continue;
+      while (wm | cand) {
+        if (cand == 0u) {
+          w = __ffs(wm) - 1;
+          wm &= wm - 1u;
+          cand = myrow[w << 5];
+        }
+        const int jj = __ffs(cand) - 1;
+        cand &= cand - 1u;
+        const int j = (w << 5) + jj;
+        const float4 bj = crn[j];
+        const float lox = fmaxf(bi.x, bj.x), hix = fminf(bi.z, bj.z), loy = fmaxf(bi.y, bj.y), hiy = fminf(bi.w, bj.w);
+        const float fx = hix - lox, fy = hiy - loy;
+        if (fx > 0.f && fx * fy >= qi_lo + qlo[j]) {
           const float ex = fmaxf(0.f, __fsub_rn(hix, lox));
           const float ey = fmaxf(0.f, __fsub_rn(hiy, loy));
           const float inter = __fmul_rn(ex, ey);
           const float den = __fadd_rn(__fsub_rn(__fadd_rn(area[j], ai), inter), 1e-10f);
           if (__fdiv_rn(inter, den) > thr) bits |= 1u << jj;
         }
-        myrow[w << 5] = bits;
-        any |= bits;
+        if (cand == 0u) {
+          myrow[w << 5] = bits;
+          any |= bits;
+          NMS_TIMING_ONLY(nt_sup += __popc(bits);)
+          bits = 0u;
+        }
       }
       const u32 open_rows = __ballot_sync(SSDG_FULL, any != 0u);
       if (lane == 0) openw[gi] = open_rows;
+      NMS_TIMING_ONLY({
+        nt_sup = __reduce_add_sync(SSDG_FULL, nt_sup);
+        if (lane == 0) { NMS_COUNT(NT_PASS_B, clock64() - nt_w0); NMS_COUNT(NT_SUPPRESS, nt_sup); }
+      })
     };
     // group g costs g + 1 words: dealt in pairs (last + first, ...) every warp gets the same number of word steps
     for (int k = warp; 2 * k < ngroups; k += kNmsWarps) {
@@ -902,6 +990,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
       openw[g] = m >= 32 * (g + 1) ? ~0u : (m > 32 * g ? (1u << (m - 32 * g)) - 1u : 0u);
   }
   __syncthreads();
+  NMS_TICK(NT_JOIN);
 
   // Closed rows are kept at once.  The open ones: fixed point of  kept(i) <=> no kept j < i with sup(i, j);
   // removed(i) <=> some kept j < i with sup(i, j), by one warp (a handful of rows per list: no CTA-wide barrier per
@@ -927,7 +1016,9 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
       }
     }
     __syncwarp();
+    if (lane == 0) NMS_COUNT(NT_OPEN, nu);
     for (;;) {
+      if (lane == 0) NMS_COUNT(NT_ROUNDS, 1);
       bool unknown = false;
       for (int k = lane; k < nu; k += 32) {
         const int i = (int)unres[k], gi = i >> 5;
@@ -959,6 +1050,7 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     if (lane == 31) wpre[W] = (u32)incl;
   }
   __syncthreads();
+  NMS_TICK(NT_RESOLVE);
   int* ok = P.out_kept + list * (size_t)P.top_k;
   float* os = P.out_score ? P.out_score + list * (size_t)P.top_k : nullptr;
   const int total = (int)wpre[W];
@@ -976,6 +1068,12 @@ __global__ void __launch_bounds__(kNmsThreads, 12) nms_kernel(NmsParams P) {
     }
   }
   if (tid == 0) P.out_count[list] = total;
+#ifdef SSDG_NMS_TIMING
+  __syncthreads();
+  NMS_TICK(NT_OUTPUT);
+  __syncthreads();
+  if (tid < NT_SLOTS && nt_acc[tid]) atomicAdd(&g_nms_timing[tid], nt_acc[tid]);
+#endif
 }
 
 // Launch geometry of the filter pass, a pure function of the shape (both stages and the workspace size derive it).
@@ -1078,6 +1176,18 @@ static u32 host_key32(float v) {
   std::memcpy(&b, &v, 4);
   return (b & 0x80000000u) ? ~b : (b | 0x80000000u);
 }
+
+#ifdef SSDG_NMS_TIMING
+// Copies the phase attribution of the nms_kernel launches since the last call (NmsTiming slots) and zeroes it.
+extern "C" SSDG_API int ssdg_nms_timing(unsigned long long* out, int32_t n) {
+  if (!out || n <= 0 || n > NT_SLOTS) return SSDG_ERR_ARG;
+  SSDG_CUDA_TRY(cudaDeviceSynchronize());
+  SSDG_CUDA_TRY(cudaMemcpyFromSymbol(out, g_nms_timing, (size_t)n * 8));
+  static const unsigned long long zero[NT_SLOTS] = {};
+  SSDG_CUDA_TRY(cudaMemcpyToSymbol(g_nms_timing, zero, sizeof(zero)));
+  return SSDG_OK;
+}
+#endif
 
 static int run_nms(const DetectWs& ws, const float* boxes, long long batch, int A, int C, int top_k, float score_thresh,
                    float iou_thresh, int* out_kept, int* out_count, float* out_score, cudaStream_t st) {
